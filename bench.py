@@ -54,7 +54,15 @@ def parse():
     ap.add_argument("--no-resample", action="store_true", help="skip the config-C5 resampling leg")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-legs", action="store_true", help="skip the C1 / C2 / C3 legs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (rank 0): the "
+                         "per-frame results of the device-resident step and a seeded sample of the clouds of the e2e step")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
 
 
 def peaks():
@@ -207,6 +215,35 @@ def family_bytes(st, cfg, S, P, icp_iters=()):
     return b
 
 
+DUMP_ROWS = 1 << 21      # cloud rows --dump-outputs writes at most: 2 Mi rows x (12 + 8) B = 40 MiB of the 64 MB allowed
+
+
+def result_arrays(res, S):
+    """The kp_frame_result array a pipeline call returns, field by field, as float64 arrays (frame first)."""
+    out = {k: np.array([getattr(r, k) for r in res], np.float64)
+           for k in ("n_fused", "n_voxel", "n_sor", "n_floor_inliers", "n_out", "status")}
+    out["icp_T"] = np.array([[list(r.icp_T[i]) for i in range(S - 1)] for r in res], np.float64).reshape(len(res), S - 1, 4, 4)
+    for k in ("icp_fitness", "icp_rmse", "icp_iters"):
+        out[k] = np.array([list(getattr(r, k))[:S - 1] for r in res], np.float64)
+    return out
+
+
+def cloud_sample(xyz, n_out, rows=DUMP_ROWS, seed=0):
+    """Final clouds xyz float32 [F, stride, 3], of which the first n_out[f] rows of frame f are valid: all valid rows when
+    there are at most `rows` of them, else a seeded uniform sample of `rows`, in (frame, row) order, with their indices."""
+    off = np.concatenate([[0], np.cumsum(np.asarray(n_out, np.int64))])
+    g = np.arange(off[-1]) if off[-1] <= rows else np.sort(np.random.default_rng(seed).choice(off[-1], rows, replace=False))
+    f = np.searchsorted(off, g, side="right") - 1
+    r = g - off[f]
+    return {"points": np.ascontiguousarray(xyz[f, r], np.float32), "points_index": np.stack([f, r], 1).astype(np.float32)}
+
+
+def write_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_pipeline_leg(ctx, cfg, depth, tab, T_fuse, T_icp, device, frames, steps):
     """frames/s of a pipeline configuration with depth resident in HBM (CUDA events on the ctx stream, L2 flushed)."""
     from kinectpy_b200.pipeline import FramePipeline
@@ -301,15 +338,16 @@ def main():
 
     def timed(fn, steps):
         """K steps, each bracketed by CUDA events on the ctx stream (a step call returns only after every batch
-        slot's streams are drained, so the event pair spans the whole step); L2 flushed between steps."""
-        total_ms = 0.0
+        slot's streams are drained, so the event pair spans the whole step); L2 flushed between steps.  Returns the
+        summed time and what the last step returned."""
+        total_ms, out = 0.0, None
         for _ in range(steps):
             ctx.flush_l2()
             ctx.sync()
             ctx.timer_start()
-            fn()
+            out = fn()
             total_ms += ctx.timer_stop()
-        return total_ms
+        return total_ms, out
 
     step_dev = lambda: pipe.run_raw(d_batch.ptr, True, B)
     for _ in range(max(args.warmup, 3)):
@@ -319,11 +357,12 @@ def main():
     sampler.start()
     l0 = pipe.launch_count()
     wall0 = time.perf_counter()
-    ms = timed(step_dev, args.steps)                    # the headline number carries no profiling events
+    ms, last = timed(step_dev, args.steps)              # the headline number carries no profiling events
     barrier()
     wall = time.perf_counter() - wall0
     launches = pipe.launch_count() - l0
     clocks = sampler.stop()
+    dump = result_arrays(last, S) if args.dump_outputs and rank == 0 else {}
 
     # ------------------------------------------------------------------ e2e: host buffers in, clouds out
     e2e = None
@@ -338,12 +377,17 @@ def main():
         for _ in range(2):
             res = step_e2e()
         barrier()
-        ms_e2e = timed(step_e2e, args.steps)
+        ms_e2e, res = timed(step_e2e, args.steps)
         barrier()
         d2h = sum(int(res[f].n_out) * 12 for f in range(B)) + B * C.sizeof(_cabi.FrameResult)
         e2e = {"ms": ms_e2e, "h2d": int(batch.nbytes), "d2h": int(d2h)}
+        if args.dump_outputs and rank == 0:
+            xyz = np.ctypeslib.as_array((C.c_float * (B * stride * 3)).from_address(hout.value)).reshape(B, stride, 3)
+            dump.update(cloud_sample(xyz, [res[f].n_out for f in range(B)]))
         lib.kp_host_free(hin)
         lib.kp_host_free(hout)
+    if dump:
+        write_outputs(args.dump_outputs, dump)
 
     # ------------------------------------------------------------------ reduce over ranks (max time) before the rank-0-only legs
     per_rank = None

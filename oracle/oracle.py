@@ -10,6 +10,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -22,10 +23,18 @@ F_DROP_ANY_ZERO = 2
 
 
 def build(force: bool = False) -> str:
-    """Compile the C restatement with gcc (no FMA contraction, OpenMP if available)."""
+    """Compile the C restatement with gcc (no FMA contraction, OpenMP if available).  In a tree that cannot be
+    written (a read-only checkout) the library goes to a temporary directory instead."""
+    global _SO
     src = os.path.join(_HERE, "kp_oracle.c")
     if force or not os.path.exists(_SO) or os.path.getmtime(_SO) < os.path.getmtime(src):
-        os.makedirs(os.path.dirname(_SO), exist_ok=True)
+        try:
+            os.makedirs(os.path.dirname(_SO), exist_ok=True)
+            writable = os.access(os.path.dirname(_SO), os.W_OK)
+        except OSError:
+            writable = False
+        if not writable:
+            _SO = os.path.join(tempfile.mkdtemp(prefix="kp_oracle_"), "libkp_oracle.so")
         base = ["-O2", "-ffp-contract=off", "-fPIC", "-shared", "-fvisibility=hidden", "-o", _SO, src, "-lm"]
         for cc in ("/usr/bin/gcc", "gcc", "cc"):
             for omp in (["-fopenmp"], []):

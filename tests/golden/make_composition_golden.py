@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Generate tests/golden/reference_compositions.npz by RUNNING THE REFERENCE'S OWN WRAPPERS
-(/root/reference, read-only) in this container.
+"""Generate tests/golden/reference_compositions.npz and reference_registrations.npz by RUNNING THE REFERENCE'S OWN
+WRAPPERS (a checkout of tiborcamargo/KinectPy, read-only).
 
 Open3D is absent here, so the reference's wrapper code is executed, unmodified, against an ``open3d`` stand-in
 whose geometry routines are the CPU oracle's (oracle/kp_oracle.c).  What this pins is everything the WRAPPERS
@@ -20,7 +20,7 @@ tests/test_golden.py then checks that the oracle's array-level compositions (``o
 ``oracle.remove_floor``, and the registration composition the frame pipeline uses) reproduce these outputs;
 the GPU tests compare the kernels with those compositions.
 
-Run:  python tests/golden/make_composition_golden.py     (needs /root/reference; the .npz is committed)
+Run:  python tests/golden/make_composition_golden.py <KinectPy checkout>     (the .npz files are committed)
 """
 import contextlib
 import copy
@@ -33,8 +33,8 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
 OUT = os.path.join(HERE, "reference_compositions.npz")
+OUT_REG = os.path.join(HERE, "reference_registrations.npz")      # glob_* / col_*: kept apart so each file stays under 1 MB
 sys.path.insert(0, ROOT)
 
 CALLS = []          # (routine, arguments) in the order the reference's wrappers made them
@@ -220,8 +220,9 @@ def scene(n, seed, mm=False):
 
 
 def main():
+    ref = sys.argv[1]          # a checkout of tiborcamargo/KinectPy
     PointCloud = install_oracle_backed_open3d()
-    sys.path.insert(0, REF)
+    sys.path.insert(0, ref)
     from preprocessing import filtering as ref_filtering
     from preprocessing import registration as ref_registration
     out = {}
@@ -253,14 +254,14 @@ def main():
     out["reg_master"], out["reg_sub"], out["reg_init"], out["reg_T"] = master, sub, init, np.asarray(T, np.float64)
     out["reg_calls"] = np.array(repr(CALLS))
     # the wrappers' own source text (fixture data, like floor_source / fuse_source below): tests/test_gpu_dropin.py executes
-    # it, unmodified, over kinectpy_b200.o3d on the GPU box, where /root/reference does not exist
+    # it, unmodified, over kinectpy_b200.o3d without a KinectPy checkout
     import inspect
     out["fo_source"] = np.array(inspect.getsource(ref_filtering.filter_outliers))
     out["reg_source"] = np.array("\n".join(inspect.getsource(f) for f in (ref_registration.preprocess_point_cloud, ref_registration.prepare_dataset,
                                                                           ref_registration.execute_point_to_plane_registration)))
 
     # ---- floor removal: the body of the script's loop, exec'd verbatim from the reference's file
-    src_lines = open(os.path.join(REF, "floor_removal.py")).read().splitlines()
+    src_lines = open(os.path.join(ref, "floor_removal.py")).read().splitlines()
     main_at = next(i for i, ln in enumerate(src_lines) if ln.startswith("if __name__"))
     first = next(i for i, ln in enumerate(src_lines) if i > main_at and "pcd_points = np.asarray(pcd.points)" in ln)
     last = next(i for i, ln in enumerate(src_lines) if i > main_at and "remove_statistical_outlier(" in ln)
@@ -279,7 +280,7 @@ def main():
     # ---- fusion: the body of DataProcessor's frame loop (preprocessing/data.py:41-61), exec'd verbatim
     from preprocessing import data as ref_data        # (only for its module-level imports to resolve as in the reference)
     del ref_data
-    src_lines = open(os.path.join(REF, "preprocessing", "data.py")).read().splitlines()
+    src_lines = open(os.path.join(ref, "preprocessing", "data.py")).read().splitlines()
     first = next(i for i, ln in enumerate(src_lines) if "registered_pcd_points, registered_pcd_colors = [], []" in ln)
     last = next(i for i, ln in enumerate(src_lines) if "registered_pcd = filter_outliers(registered_pcd)" in ln)
     body = "\n".join(ln[12:] if ln.startswith(" " * 12) else ln.strip() for ln in src_lines[first:last + 1])
@@ -330,7 +331,9 @@ def main():
     out["col_master"], out["col_sub"], out["col_colors"], out["col_T"] = cm, cs, ccol, np.asarray(Tc, np.float64)
     out["col_calls"] = np.array(repr(CALLS))
 
-    np.savez_compressed(OUT, **out)
+    reg = {k: out[k] for k in out if k.startswith(("glob_", "col_"))}
+    np.savez_compressed(OUT, **{k: v for k, v in out.items() if k not in reg})
+    np.savez_compressed(OUT_REG, **reg)
     for k in ("fo_calls", "fo_default_calls", "reg_calls", "floor_calls", "fuse_calls", "so_calls", "glob_calls", "col_calls"):
         print(k, out[k])
     print("wrote", OUT, {k: getattr(v, "shape", None) for k, v in out.items()})

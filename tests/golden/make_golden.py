@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Generate tests/golden/reference_own_arithmetic.npz by RUNNING THE REFERENCE'S OWN CODE
-(/root/reference, read-only) in this container.
+(a checkout of tiborcamargo/KinectPy, read-only).
 
 The reference's geometric heavy lifting is Open3D (absent here), but a few steps of the path are
 the reference's own numpy arithmetic.  Those are executed here, unmodified, with a minimal
@@ -13,7 +13,7 @@ select_by_index with Open3D's mask-walk order) -- no geometry is computed by the
 * ``preprocessing.filtering.kalman_filter``                         (preprocessing/filtering.py:98-129)
 * the floor-band split expression of the script body                (floor_removal.py:64-66, evaluated verbatim)
 
-Run:  python tests/golden/make_golden.py        (needs /root/reference; the .npz is committed)
+Run:  python tests/golden/make_golden.py <KinectPy checkout>        (the .npz is committed)
 """
 import contextlib
 import io
@@ -24,7 +24,6 @@ import types
 
 import numpy as np
 
-REF = "/root/reference"
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_own_arithmetic.npz")
 
 
@@ -60,8 +59,9 @@ def install_stubs():
 
 
 def main():
+    ref = sys.argv[1]          # a checkout of tiborcamargo/KinectPy
     StubPointCloud = install_stubs()
-    sys.path.insert(0, REF)
+    sys.path.insert(0, ref)
     import floor_removal as ref_floor
     from preprocessing import filtering as ref_filtering
     from preprocessing.data import DataProcessor

@@ -198,6 +198,30 @@ def test_bench_b200_arm_fails_loudly_without_a_gpu():
     assert "no CUDA device" in (r.stderr + r.stdout) and not any(ln.startswith("{") for ln in r.stdout.splitlines())
 
 
+def test_bench_dump_outputs_arrays():
+    """`bench.py --dump-outputs`: every field of the per-frame results as float64, and the final clouds as float32 -- all
+    valid rows when they fit, else the same seeded sample of (frame, row) pairs on every run -- within 64 MB."""
+    sys.path.insert(0, ROOT)
+    import bench
+    from kinectpy_b200 import _cabi
+    res = (_cabi.FrameResult * 2)()
+    res[1].n_out, res[1].icp_T[0][3], res[1].icp_iters[1] = 5, 0.25, 7
+    a = bench.result_arrays(res, 3)
+    assert a["icp_T"].shape == (2, 2, 4, 4) and a["icp_T"][1, 0, 0, 3] == 0.25 and a["icp_iters"][1, 1] == 7
+    assert a["n_out"].tolist() == [0, 5] and all(v.dtype == np.float64 for v in a.values())
+    xyz = np.random.default_rng(0).normal(size=(3, 10, 3)).astype(np.float32)
+    full = bench.cloud_sample(xyz, [4, 0, 10])
+    assert np.array_equal(full["points"], np.concatenate([xyz[0, :4], xyz[2]])) and full["points_index"].dtype == np.float32
+    s = bench.cloud_sample(xyz, [4, 0, 10], rows=6)
+    f, r = s["points_index"].astype(np.int64).T
+    assert len(f) == 6 and (r < np.array([4, 0, 10])[f]).all() and (np.diff(f * 10 + r) > 0).all()
+    assert np.array_equal(s["points"], xyz[f, r]) and np.array_equal(s["points"], bench.cloud_sample(xyz, [4, 0, 10], rows=6)["points"])
+    assert bench.DUMP_ROWS * (12 + 8) < 64e6
+    for bad in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "x"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + bad, capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and "error" in r.stderr
+
+
 def test_bench_gives_every_rank_the_same_workload():
     """Weak scaling needs the same per-GPU work on every rank: `bench.make_inputs` hands every rank the same distinct frames,
     rotated by rank (a first version gave rank r its own window of the synthetic sequence; the windows differed by up to

@@ -1,5 +1,5 @@
 """Golden vectors produced by running the REFERENCE'S OWN numpy arithmetic (tests/golden/make_golden.py,
-executed in the build container against /root/reference with a container-only open3d stand-in).
+run on a checkout of KinectPy with an open3d stand-in).
 CPU part: the oracle and the host-side mirrors against the fixtures.  GPU part: the kernels, through the
 reference-shaped Python surface, against the same fixtures."""
 import os
@@ -93,9 +93,10 @@ def test_gpu_floor_band_matches_reference():
 # Wrapper-level goldens: tests/golden/reference_compositions.npz was produced by the reference's OWN wrapper functions
 # (preprocessing/filtering.py, preprocessing/registration.py, the loop body of floor_removal.py) driving an `open3d`
 # stand-in computed by the oracle (tests/golden/make_composition_golden.py).  They pin what the wrappers decide:
-# call order, arguments and defaults, source / target roles, what is copied and returned.
-def _compositions():
-    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_compositions.npz"))
+# call order, arguments and defaults, source / target roles, what is copied and returned.  The global and coloured
+# registration cases are in tests/golden/reference_registrations.npz.
+def _compositions(name="reference_compositions.npz"):
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", name))
 
 
 def _oracle_backed():
@@ -192,7 +193,7 @@ def test_mirror_global_and_colored_registration_make_the_reference_calls(oracle,
     mod = _oracle_backed()
     PointCloud, registration, geometry = mod.oracle_backed_namespace()
     from kinectpy_b200.preprocessing import registration as our_registration
-    g = _compositions()
+    g = _compositions("reference_registrations.npz")
     ns = type("G", (), {})()
     for k, v in list(vars(registration).items()) + list(vars(geometry).items()):
         setattr(ns, k, v)

@@ -6,14 +6,11 @@ The reference's hot-path wrappers -- ``filter_outliers`` (preprocessing/filterin
 ``DataProcessor``'s frame loop (preprocessing/data.py:41-61) -- are executed UNMODIFIED with ``o3d`` bound to
 ``kinectpy_b200.o3d`` (the import swap of INTEGRATION.md) on the B200, and their results are compared with
 tests/golden/reference_compositions.npz, which the same source produced over the CPU oracle
-(tests/golden/make_composition_golden.py).  The source text comes from /root/reference when it exists (this
-container) and otherwise from the fixture, where the generator stored it verbatim (the GPU box has no /root/reference)."""
+(tests/golden/make_composition_golden.py).  The source text is the fixture's: the generator stored it verbatim."""
 import contextlib
 import copy
-import inspect
 import io
 import os
-import sys
 import types
 
 import numpy as np
@@ -22,7 +19,6 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = "/root/reference"
 
 
 @pytest.fixture(scope="module")
@@ -45,33 +41,9 @@ def cloud(o3d, pts, colors=None):
 
 def reference_functions(gold, names, key):
     """The reference's functions, compiled from its own source with `o3d` = the B200 shim."""
-    o3d = shim()
-    ns = {"o3d": o3d, "np": np, "copy": copy}
-    if os.path.isdir(REF):
-        # this container: import the reference modules themselves over the shim
-        saved = {k: sys.modules.get(k) for k in ("open3d", "tensorflow", "imghdr", "cv2", "preprocessing", "preprocessing.filtering", "preprocessing.registration")}
-        try:
-            mod = types.ModuleType("open3d")
-            mod.__dict__.update({k: getattr(o3d, k) for k in ("geometry", "utility", "pipelines", "io")})
-            sys.modules["open3d"] = mod
-            for n in ("tensorflow", "imghdr", "cv2"):
-                sys.modules.setdefault(n, types.ModuleType(n))
-            sys.path.insert(0, REF)
-            for n in ("preprocessing", "preprocessing.filtering", "preprocessing.registration"):
-                sys.modules.pop(n, None)
-            from preprocessing import filtering as rf, registration as rr
-            src = "\n".join(inspect.getsource(getattr(rf if hasattr(rf, n) else rr, n)) for n in names)
-        finally:
-            sys.path.remove(REF)
-            for k, v in saved.items():
-                if v is None:
-                    sys.modules.pop(k, None)
-                else:
-                    sys.modules[k] = v
-        assert src == str(gold[key]), "the fixture's copy of the reference source is stale: regenerate the goldens"
-    else:
-        src = str(gold[key])
-    exec(src, ns)
+    ns = {"o3d": shim(), "np": np, "copy": copy}
+    exec(str(gold[key]), ns)
+    assert all(n in ns for n in names)
     return ns
 
 
