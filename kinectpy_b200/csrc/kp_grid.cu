@@ -789,6 +789,36 @@ __constant__ signed char HQ_COLS[25][2] = {
 // smallest double-precision d2 a candidate outside bins 0..b can have
 __device__ __forceinline__ double hq_lower_edge(int b, float scale) { return ((double)b + 0.5) / (double)scale * (1.0 - 1e-6); }
 
+// Shared memory of a histogram-kernel CTA of T threads: per thread cap candidate entries (4-byte positions into the point
+// array) and then nb 16-bit bins, each strided by T (buf[slot * T], hist[bin * T]: any slot pattern is bank-conflict
+// free).  hq_smem(T, cap, 0) is where the bins start.
+__host__ __device__ constexpr size_t hq_smem(int T, int cap, int nb) { return (size_t)T * ((size_t)cap * sizeof(unsigned) + (size_t)nb * sizeof(unsigned short)); }
+
+// Orders buf[0..m) -- positions, counting-sorted by bin as collected -- by (fp32 d2, position); entries only move inside
+// their bin.  An entry stores no distance: its fp32 d2 is recomputed from the point (an L1 hit, the collection pass just
+// read it) exactly as the collection pass computed it.  The key of the last entry of the sorted prefix stays in registers,
+// so an entry already in place costs one gather; only a shift reads the entries it passes.
+template <int HQT>
+__device__ __forceinline__ void hq_sort_buf(unsigned *buf, int m, const float4 *pts, const float4 &me)
+{
+    unsigned dl = 0u, pl = 0u;   // (d2 bits, position) of buf[i - 1], the largest of the sorted prefix
+    for (int i = 0; i < m; ++i) {
+        const unsigned pos = buf[i * HQT];
+        const unsigned d = __float_as_uint(hq_d32(me.x, me.y, me.z, __ldg(pts + pos)));   // d2 >= 0: bits order as floats
+        if (i == 0 || dl < d || (dl == d && pl < pos)) { dl = d; pl = pos; continue; }
+        buf[i * HQT] = pl;
+        int j = i - 2;
+        while (j >= 0) {
+            const unsigned o = buf[j * HQT];
+            const unsigned od = __float_as_uint(hq_d32(me.x, me.y, me.z, __ldg(pts + o)));
+            if (od < d || (od == d && o < pos)) break;
+            buf[(j + 1) * HQT] = o;
+            --j;
+        }
+        buf[(j + 1) * HQT] = pos;
+    }
+}
+
 __device__ void kq_finish_normal(const KnnParams &p, int64_t row, int cnt, double *sm)
 {
     double nr[3] = {0.0, 0.0, 1.0};
@@ -807,9 +837,8 @@ template <int NB, int R, int HQT>
 __device__ __forceinline__ void hq_query(const KnnParams &p, const KpGridDev &g, const int64_t q, unsigned char *smem_raw)
 {
     const int tid = threadIdx.x;
-    // buf[slot * HQT], hist[bin * HQT]: any slot pattern is bank-conflict free
-    unsigned long long *buf = reinterpret_cast<unsigned long long *>(smem_raw) + tid;
-    unsigned short *hist = reinterpret_cast<unsigned short *>(smem_raw + (size_t)p.cap * HQT * sizeof(unsigned long long)) + tid;
+    unsigned *buf = reinterpret_cast<unsigned *>(smem_raw) + tid;
+    unsigned short *hist = reinterpret_cast<unsigned short *>(smem_raw + hq_smem(HQT, p.cap, 0)) + tid;
     const int k = p.k;
     const float4 me = __ldg(p.qpts + q);
     const int64_t row = __float_as_int(me.w);
@@ -865,7 +894,7 @@ __device__ __forceinline__ void hq_query(const KnnParams &p, const KpGridDev &g,
                 if (mm > u && (unsigned)bu <= (unsigned)b) {
                     const int slot = hist[bu * HQT];
                     hist[bu * HQT] = (unsigned short)(slot + 1);
-                    if (slot < m) buf[slot * HQT] = ((unsigned long long)__float_as_uint(dj[u]) << 32) | (unsigned)(t + u);
+                    if (slot < m) buf[slot * HQT] = (unsigned)(t + u);
                     ++nput;
                 }
             }
@@ -948,18 +977,7 @@ __device__ __forceinline__ void hq_query(const KnnParams &p, const KpGridDev &g,
     }
     // (a bin count that wrapped its 16 bits also ends here: > 65535 puts can never equal m <= cap)
     if (nput != m) { p.strag_flags[q] = 1; return; }
-    // ---- order by (fp32 d2, position): entries only move inside their bin
-    for (int i = 1; i < m; ++i) {
-        const unsigned long long key = buf[i * HQT];
-        int j = i - 1;
-        while (j >= 0) {
-            const unsigned long long o = buf[j * HQT];
-            if (o <= key) break;
-            buf[(j + 1) * HQT] = o;
-            --j;
-        }
-        buf[(j + 1) * HQT] = key;
-    }
+    hq_sort_buf<HQT>(buf, m, g.pts, me);
     // ---- exact evaluation in that order; the canonical (d2, index) order must be strictly ascending
     const bool capped = p.r2cap > 0;
     const bool normals = p.mode == KQ_MODE_NORMALS;
@@ -968,10 +986,10 @@ __device__ __forceinline__ void hq_query(const KnnParams &p, const KpGridDev &g,
     double sm[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
     int cnt = 0;
     bool bad = false, closed = false;
-    float4 cn = m > 0 ? __ldg(g.pts + (unsigned)buf[0]) : make_float4(0.f, 0.f, 0.f, 0.f);
+    float4 cn = m > 0 ? __ldg(g.pts + buf[0]) : make_float4(0.f, 0.f, 0.f, 0.f);
     for (int i = 0; i < m; ++i) {
         const float4 c = cn;
-        if (i + 1 < m) cn = __ldg(g.pts + (unsigned)buf[(i + 1) * HQT]);     // next gather in flight during this evaluation
+        if (i + 1 < m) cn = __ldg(g.pts + buf[(i + 1) * HQT]);     // next gather in flight during this evaluation
         const double d = kp_d2(qx, qy, qz, (double)c.x, (double)c.y, (double)c.z);
         const int id = __float_as_int(c.w);
         if (!hq_before(pd, pi, d, id)) bad = true;
@@ -1053,8 +1071,8 @@ template <int NB, int HQT>
 __device__ __forceinline__ void vq_query(const KnnParams &p, const KpVbiDev &v, const int64_t q, unsigned char *smem_raw)
 {
     const int tid = threadIdx.x;
-    unsigned long long *buf = reinterpret_cast<unsigned long long *>(smem_raw) + tid;
-    unsigned short *hist = reinterpret_cast<unsigned short *>(smem_raw + (size_t)p.cap * HQT * sizeof(unsigned long long)) + tid;
+    unsigned *buf = reinterpret_cast<unsigned *>(smem_raw) + tid;
+    unsigned short *hist = reinterpret_cast<unsigned short *>(smem_raw + hq_smem(HQT, p.cap, 0)) + tid;
     const int k = p.k;
     const float4 me = __ldg(v.pts + q);
     const int64_t row = __float_as_int(me.w);
@@ -1108,33 +1126,22 @@ __device__ __forceinline__ void vq_query(const KnnParams &p, const KpVbiDev &v, 
             if ((unsigned)bu <= (unsigned)b) {
                 const int slot = hist[bu * HQT];
                 hist[bu * HQT] = (unsigned short)(slot + 1);
-                if (slot < m) buf[slot * HQT] = ((unsigned long long)__float_as_uint(dj) << 32) | (unsigned)pos;
+                if (slot < m) buf[slot * HQT] = (unsigned)pos;
                 ++nput;
             }
         });
         if (nput != m) { p.strag_flags[q] = 1; return; }
-        // ---- order by (fp32 d2, position): entries only move inside their bin
-        for (int i = 1; i < m; ++i) {
-            const unsigned long long key = buf[i * HQT];
-            int j = i - 1;
-            while (j >= 0) {
-                const unsigned long long o = buf[j * HQT];
-                if (o <= key) break;
-                buf[(j + 1) * HQT] = o;
-                --j;
-            }
-            buf[(j + 1) * HQT] = key;
-        }
+        hq_sort_buf<HQT>(buf, m, v.pts, me);
         // ---- exact evaluation in that order; the canonical (d2, index) order must be strictly ascending
         double pd = -1.0; int pi = -1;
         double acc = 0.0;
         double sm[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
         int cnt = 0;
         bool bad = false, closed = false;
-        float4 cn = m > 0 ? __ldg(v.pts + (unsigned)buf[0]) : make_float4(0.f, 0.f, 0.f, 0.f);
+        float4 cn = m > 0 ? __ldg(v.pts + buf[0]) : make_float4(0.f, 0.f, 0.f, 0.f);
         for (int i = 0; i < m; ++i) {
             const float4 c = cn;
-            if (i + 1 < m) cn = __ldg(v.pts + (unsigned)buf[(i + 1) * HQT]);
+            if (i + 1 < m) cn = __ldg(v.pts + buf[(i + 1) * HQT]);
             const double d = kp_d2(qx, qy, qz, (double)c.x, (double)c.y, (double)c.z);
             const int id = __float_as_int(c.w);
             if (!hq_before(pd, pi, d, id)) bad = true;
@@ -1448,12 +1455,12 @@ int knn_launch_warp(kp_ctx *ctx, KnnParams &p, int64_t grid_queries)
 template <int NB, int R>
 int knn_launch_hist(kp_ctx *ctx, KnnParams &p)
 {
-    // the per-thread buffer (k + slack entries of 8 bytes) is what limits occupancy for large k: smaller CTAs pack the
-    // 227 KB of an SM more tightly
+    // the per-thread buffer (k + slack entries) is what limits occupancy for large k: smaller CTAs pack the 227 KB of an
+    // SM more tightly
     constexpr int T = NB <= 32 ? 128 : 64;
     static const int slack = getenv("KP_KNN_SLACK") ? atoi(getenv("KP_KNN_SLACK")) : 8;   // swept: 6 / 8 / 12
     p.cap = p.k + slack;
-    size_t smem = (size_t)T * ((size_t)p.cap * sizeof(unsigned long long) + (size_t)NB * sizeof(unsigned short));
+    const size_t smem = hq_smem(T, p.cap, NB);
     if (smem > 48 * 1024) KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_hist<NB, R, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     k_knn_hist<NB, R, T><<<kp_blocks(p.nq, T), T, smem, ctx->stream>>>(p);
     KP_LAUNCH_CHECK(ctx);
@@ -1715,9 +1722,9 @@ int kp_knn_batch_create(kp_ctx *ctx, const KpKnnSegDesc *segs, int nseg, int k, 
     const size_t smem_w = (size_t)KQ_WARPS * capw * (sizeof(double) + sizeof(int));
     if (smem_w > 200 * 1024) return kp_set_err(ctx, KP_E_ARG, "k = %d neighbours is too many for the per-warp buffer", k);
     if (smem_w > 48 * 1024) KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_b, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_w));
-    const size_t smem_m = (size_t)64 * ((size_t)out->cap_mid * 8 + 64 * 2);
+    const size_t smem_m = hq_smem(64, out->cap_mid, 64);
     if (smem_m > 48 * 1024) KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_mid_b, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_m));
-    const size_t smem_h = (size_t)(k <= 32 ? 128 : 64) * ((size_t)out->cap_hist * 8 + (size_t)(k <= 32 ? 32 : 64) * 2);
+    const size_t smem_h = k <= 32 ? hq_smem(128, out->cap_hist, 32) : hq_smem(64, out->cap_hist, 64);
     if (smem_h > 48 * 1024) {
         if (k <= 32) {
             KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_hist_b<32, 2, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h));
@@ -1746,7 +1753,7 @@ template <int NB, int R, int T>
 static int knn_level0_launch(kp_ctx *ctx, const KpKnnBatch &b, int64_t cap_rows, int per_sm, int level = 0)
 {
     const KnnParams *hp = (const KnnParams *)b.h_params + (size_t)level * b.nseg;
-    const size_t smem = (size_t)T * ((size_t)(level == 3 ? b.cap_mid : b.cap_hist) * 8 + NB * 2);
+    const size_t smem = hq_smem(T, level == 3 ? b.cap_mid : b.cap_hist, NB);
     int64_t gx = (cap_rows + T - 1) / T;
     if (gx > (int64_t)ctx->sm_count * per_sm) gx = (int64_t)ctx->sm_count * per_sm;
     for (int s0 = 0; s0 < b.nseg; s0 += KNN_ARG_SEGS) {
@@ -1774,13 +1781,13 @@ int kp_knn_batch_vbi(kp_ctx *ctx, const KpKnnBatch &b, int64_t cap_rows)
     KP_PROFB(ctx, "knn_vbi", 0.0);
     if (b.k <= 32) {
         constexpr int T = 128;
-        const size_t smem = (size_t)T * ((size_t)b.cap_hist * 8 + 32 * 2);
+        const size_t smem = hq_smem(T, b.cap_hist, 32);
         int64_t gx = (cap_rows + T - 1) / T;
         if (gx > (int64_t)ctx->sm_count * 24) gx = (int64_t)ctx->sm_count * 24;
         k_knn_vbi_b<32, T><<<dim3((unsigned)(gx > 0 ? gx : 1), (unsigned)b.nseg), T, smem, ctx->stream>>>(pp);
     } else {
         constexpr int T = 64;
-        const size_t smem = (size_t)T * ((size_t)b.cap_hist * 8 + 64 * 2);
+        const size_t smem = hq_smem(T, b.cap_hist, 64);
         int64_t gx = (cap_rows + T - 1) / T;
         if (gx > (int64_t)ctx->sm_count * 32) gx = (int64_t)ctx->sm_count * 32;
         k_knn_vbi_b<64, T><<<dim3((unsigned)(gx > 0 ? gx : 1), (unsigned)b.nseg), T, smem, ctx->stream>>>(pp);
