@@ -337,9 +337,10 @@ KP_EXPORT int kp_pipeline_run_host(kp_pipeline *p, const uint16_t *h_depth, int6
 KP_EXPORT int64_t kp_pipeline_launch_count(kp_pipeline *p);
 /* frames per launch (B) and batch slots in flight (W) the pipeline was built with */
 KP_EXPORT int kp_pipeline_frames_in_flight(kp_pipeline *p, int *batch, int *slots);
-/* diagnostics: the device-side counts of the first frame of the last batch on slot 0, h_counts[26] =
+/* diagnostics: the device-side counts of the first frame of the last batch on slot 0, h_counts[n], n >= 26 =
  * n_fused, n_voxel, n_sor, n_band, n_band_kept, n_merged, n_floor_sor, n_out, level-0 leftovers of the three
- * neighbour searches [3], level-1 leftovers [3], valid rows of the ICP inputs [6], their voxel counts [6] */
+ * neighbour searches [3], level-1 leftovers [3], valid rows of the ICP inputs [6], their voxel counts [6];
+ * with n >= 29 also the mid-level leftovers of the three searches [3] (entries 26-28) */
 KP_EXPORT int kp_pipeline_frame_counts(kp_pipeline *p, int64_t *h_counts, int n);
 KP_EXPORT int kp_pipeline_profile(kp_pipeline *p, int enable_or_read, int max_entries,
                                   const char **h_names, double *h_ms, int64_t *h_calls, double *h_bytes, int *h_n);

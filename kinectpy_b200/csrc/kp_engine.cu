@@ -151,12 +151,19 @@ __global__ void __launch_bounds__(256) k_e_voxel_keys(const __grid_constant__ Vo
     const float *xyz = a.xyz + 3 * seg * a.xyz_stride;
     uint32_t *keys = a.keys + seg * a.key_stride;
     // A thread owns FOUR CONSECUTIVE rows = 48 bytes = three 16-byte loads, and writes their keys as one 16-byte store; two
-    // such groups per trip, all six loads issued before the first division.  (Segment strides are multiples of 64 rows and
-    // the arenas 256-byte aligned, so every group is 16-byte aligned.)  The kernel is a stream of 12-byte rows in and 4-byte
-    // keys out: the three IEEE double divisions per row are latency, not throughput.
+    // such groups per trip, all six loads issued before the first division.  (Key strides are multiples of 64 rows and the
+    // arenas 256-byte aligned, so every key group is 16-byte aligned.)  The kernel is a stream of 12-byte rows in and
+    // 4-byte keys out: the three IEEE double divisions per row are latency, not throughput.
     constexpr int U = 2;
-    const int64_t groups = a.n / 4;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    if ((((uintptr_t)xyz) & 15u) != 0u) {
+        // The input clouds (fused S * P rows per frame, raw P rows per sensor) are not padded: when P is not a multiple
+        // of 4 a segment after the first starts off the 16-byte grid, and its rows are read one by one.
+        for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < a.n; i += stride)
+            keys[i] = vox_key(vp, xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2]);
+        return;
+    }
+    const int64_t groups = a.n / 4;
     const float4 *x4 = reinterpret_cast<const float4 *>(xyz);
     uint4 *k4 = reinterpret_cast<uint4 *>(keys);
     for (int64_t g0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; g0 < groups; g0 += U * stride) {
@@ -1915,7 +1922,7 @@ int kp_pipeline_frame_counts(kp_pipeline *p, int64_t *h_counts, int n)
 {
     // the device-side counts of the first frame of batch slot 0 after its last batch (diagnostics / byte accounting):
     // n_fused, n_voxel, n_sor, n_lo, n_rest, n_merged, n_fsor, n_out, level-0 leftovers [3], level-1 leftovers [3],
-    // valid rows of the S ICP inputs [6], their voxel counts [6]
+    // valid rows of the S ICP inputs [6], their voxel counts [6]; with n >= 29 also mid-level leftovers [3]
     if (!p || !h_counts || n < 26) return KP_E_ARG;
     cudaSetDevice(p->device);
     EngSlot &s = p->slots[0];
@@ -1928,6 +1935,8 @@ int kp_pipeline_frame_counts(kp_pipeline *p, int64_t *h_counts, int n)
     for (int i = 0; i < 8; ++i) h_counts[i] = v[i];
     for (int i = 0; i < 3; ++i) { h_counts[8 + i] = d.cnt_l0[i]; h_counts[11 + i] = d.cnt_l1[i]; }
     for (int i = 0; i < 6; ++i) { h_counts[14 + i] = i < p->cfg.S ? cl[i].nv : 0; h_counts[20 + i] = i < p->cfg.S ? cl[i].n : 0; }
+    if (n >= 29)
+        for (int i = 0; i < 3; ++i) h_counts[26 + i] = d.cnt_lm[i];
     return KP_OK;
 }
 

@@ -173,14 +173,15 @@ class FramePipeline:
 
     def frame_counts(self) -> dict:
         """Device-side counts of the first frame of the last batch on slot 0 (diagnostics, byte accounting)."""
-        v = (C.c_int64 * 26)()
-        rc = self.lib.kp_pipeline_frame_counts(self.handle, v, 26)
+        v = (C.c_int64 * 29)()
+        rc = self.lib.kp_pipeline_frame_counts(self.handle, v, 29)
         if rc != 0:
             self._raise(rc)
         S = self.cfg.n_sensors
         d = dict(zip(("n_fused", "n_voxel", "n_sor", "n_lo", "n_rest", "n_merged", "n_fsor", "n_out"), [int(x) for x in v[:8]]))
         d["n_inl"] = d["n_lo"] - d["n_rest"]
         d["leftovers_l0"], d["leftovers_l1"] = [int(x) for x in v[8:11]], [int(x) for x in v[11:14]]
+        d["leftovers_mid"] = [int(x) for x in v[26:29]]      # (the ICP target's search has no mid level: [2] is 0)
         d["nv_icp"], d["n_icp"] = [int(x) for x in v[14:14 + S]], [int(x) for x in v[20:20 + S]]
         return d
 

@@ -405,10 +405,25 @@ def remove_floor(pts, band=200, thr=30, ransac_n=30, iters=2000, nb_neighbors=50
     return merged[keep.astype(bool)], plane, inl
 
 
-def frame_pipeline(cfg, depth_f, tab, T_fuse, T_icp, want_icp=True, timings=None):
+def _sor_or_all(pts, k, ratio):
+    """SOR's kept rows; k = 0 switches the stage off (every row kept), as the engine's sor_k / floor_sor_k = 0 do."""
+    if k <= 0:
+        return pts
+    keep, _, _ = sor(pts, k, ratio)
+    return pts[keep.astype(bool)]
+
+
+def frame_pipeline(cfg, depth_f, tab, T_fuse, T_icp, want_icp=True, timings=None, stages=False):
     """One frame of BASELINE config C4 on the CPU: the composition the batched GPU driver implements
     (preprocessing/data.py:44-61 -> floor_removal.py:64-73 -> preprocessing/registration.py:65-86).
-    ``cfg`` is any object with the PipelineConfig field names.  ``timings`` (dict) collects seconds per stage."""
+    ``cfg`` is any object with the PipelineConfig field names.  ``timings`` (dict) collects seconds per stage.
+
+    Every frame gets a result, by the engine's rules where upstream would raise (DESIGN §6): an empty cloud runs
+    every stage as a no-op; fewer SOR survivors than ``ransac_n`` skip floor removal (the SOR output is the frame's
+    cloud); a band smaller than ``ransac_n`` has no plane and no inliers (the band and the upper part still go
+    through the floor SOR).  ``stages=True`` adds ``n_lo`` (band), ``n_rest`` (band outliers), ``n_merged``,
+    ``n_fsor`` and, per sensor, ``nv_icp`` (valid rows of the ICP input) and ``n_icp`` (its voxel count): the
+    numbers ``FramePipeline.frame_counts()`` reports (0 for a stage that does not run)."""
     import time as _t
     S, P = cfg.n_sensors, cfg.pixels
     tick = [_t.perf_counter()]
@@ -426,32 +441,43 @@ def frame_pipeline(cfg, depth_f, tab, T_fuse, T_icp, want_icp=True, timings=None
     v = voxel_downsample(fused, cfg.voxel_size)
     out["n_voxel"] = v["m"]
     lap("voxel")
-    keep, _, _ = sor(v["points"], cfg.sor_k, cfg.sor_ratio)
-    A = v["points"][keep.astype(bool)]
+    A = _sor_or_all(v["points"], cfg.sor_k, cfg.sor_ratio)
     out["n_sor"] = len(A)
     lap("sor")
-    if cfg.do_floor:
+    st = {"n_lo": 0, "n_rest": 0, "n_merged": 0, "n_fsor": 0}
+    out["n_floor_inliers"] = 0
+    out["points"] = A
+    if cfg.do_floor and len(A) > 0:
         low = band_mask(A, cfg.floor_band, 1).astype(bool)
         floor, upper = A[low], A[~low]
-        plane, inl, best, _ = ransac_plane(floor, cfg.ransac_thr, cfg.ransac_n, cfg.ransac_iters, seed=cfg.seed)
-        out["n_floor_inliers"] = int(inl.sum())
-        out["plane"] = plane
-        merged = np.concatenate([floor[~inl.astype(bool)], upper], 0)
+        if len(floor) >= cfg.ransac_n:
+            plane, inl, best, _ = ransac_plane(floor, cfg.ransac_thr, cfg.ransac_n, cfg.ransac_iters, seed=cfg.seed)
+            inl = inl.astype(bool)
+        else:                                   # no hypothesis can be drawn: no plane, nobody is an inlier
+            plane, inl = np.full(4, np.nan), np.zeros(len(floor), bool)
+        merged = np.concatenate([floor[~inl], upper], 0)
         lap("ransac")
-        keep2, _, _ = sor(merged, cfg.floor_sor_k, cfg.floor_sor_ratio)
-        out["points"] = merged[keep2.astype(bool)]
+        fin = _sor_or_all(merged, cfg.floor_sor_k, cfg.floor_sor_ratio)
         lap("floor_sor")
-    else:
-        out["n_floor_inliers"] = 0
-        out["points"] = A
+        st.update(n_lo=len(floor), n_rest=len(floor) - int(inl.sum()), n_merged=len(merged),
+                  n_fsor=len(fin) if cfg.floor_sor_k > 0 else 0)
+        if len(A) >= cfg.ransac_n:              # else the floor stage is skipped: the SOR output stays the frame's cloud
+            out["n_floor_inliers"] = int(inl.sum())
+            out["plane"] = plane
+            out["points"] = fin
     out["icp"] = []
+    st["nv_icp"], st["n_icp"] = [0] * S, [0] * S
     if want_icp and cfg.do_icp and S > 1:
         tgt = voxel_downsample(fused[:P], cfg.icp_voxel)["points"]
         nrm = estimate_normals(tgt, cfg.normals_radius, cfg.normals_max_nn)
         lap("icp_prep")
-        for s in range(1, S):
-            raw, _, _ = unproject(depth_f[None, s:s + 1], tab[s:s + 1], None, flags=cfg.unproject_flags, scale=cfg.scale)
+        for s in range(S):
+            raw, ok, _ = unproject(depth_f[None, s:s + 1], tab[s:s + 1], None, flags=cfg.unproject_flags, scale=cfg.scale)
             src = voxel_downsample(raw[0], cfg.icp_voxel)["points"]
-            out["icp"].append(icp_point_to_plane(src, tgt, nrm, cfg.icp_max_corr, init=T_icp[s], max_iter=cfg.icp_max_iter))
+            st["nv_icp"][s], st["n_icp"][s] = int(ok.sum()), len(src)
+            if s > 0:
+                out["icp"].append(icp_point_to_plane(src, tgt, nrm, cfg.icp_max_corr, init=T_icp[s], max_iter=cfg.icp_max_iter))
         lap("icp")
+    if stages:
+        out.update(st)
     return out
