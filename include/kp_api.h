@@ -309,6 +309,13 @@ typedef struct {
     int32_t normals_max_nn; double normals_radius;
     uint64_t seed;
     int32_t n_streams;      /* frames in flight = B frames per launch x W batch slots (no worker threads) */
+    /* human crop (preprocessing/data.py:165-178), fused cloud only: a pixel is kept iff its segmentation colour is
+     * non-black in all three channels and z16 <= median(z16) + crop_gate, z16 = the int16 z of `_depth.dat` (0 outside
+     * the table), median over all P pixels of the (frame, sensor), crop_gate in millimetres whatever `scale` is.
+     * The ICP inputs are not cropped. */
+    int32_t do_crop;        double crop_gate;
+    /* fixed-N output (kp_resample_batch on each frame's final cloud, stream = frame id): 0 = off, else 1..16384 */
+    int32_t resample_n;     int32_t resample_mode;   /* KP_RESAMPLE_RANDOM / KP_RESAMPLE_PREFIX */
 } kp_pipeline_cfg;
 typedef struct {
     int64_t n_fused, n_voxel, n_sor, n_floor_inliers, n_out;
@@ -334,13 +341,24 @@ KP_EXPORT int kp_pipeline_run(kp_pipeline *p, const uint16_t *depth, int depth_o
  * frame) by a device kernel: the row counts never visit the host before the copy. */
 KP_EXPORT int kp_pipeline_run_host(kp_pipeline *p, const uint16_t *h_depth, int64_t F, kp_frame_result *h_results,
                                    float *h_out_xyz, int64_t out_stride);
+/* the general form.  rgb uint8 [F][S][P][3] segmentation images in the same memory space as depth: required when
+ * the pipeline crops, refused otherwise (KP_E_ARG).  h_frame_ids int64 [F] nullable (default f): the sample stream of
+ * frame f's fixed-N slot, so that a frame gives the same slot whichever call or rank it runs in.  d_fixed nullable
+ * float32 [F][resample_n][3] device: frame f's slot = kp_resample_batch on its final cloud with seed cfg.seed and
+ * stream h_frame_ids[f]; PREFIX pads a short cloud with zeros; a RANDOM frame with fewer than resample_n points gets
+ * status KP_E_ARG and a zero slot (the other frames are unaffected), one whose candidate list overflows KP_E_RANGE.
+ * As for every frame status, the call returns it after every frame's record is written. */
+KP_EXPORT int kp_pipeline_run_ex(kp_pipeline *p, const uint16_t *depth, const uint8_t *rgb, int inputs_on_device, int64_t F,
+                                 const int64_t *h_frame_ids, kp_frame_result *h_results, float *d_out_xyz,
+                                 int64_t out_stride, float *d_fixed);
 KP_EXPORT int64_t kp_pipeline_launch_count(kp_pipeline *p);
 /* frames per launch (B) and batch slots in flight (W) the pipeline was built with */
 KP_EXPORT int kp_pipeline_frames_in_flight(kp_pipeline *p, int *batch, int *slots);
 /* diagnostics: the device-side counts of the first frame of the last batch on slot 0, h_counts[n], n >= 26 =
  * n_fused, n_voxel, n_sor, n_band, n_band_kept, n_merged, n_floor_sor, n_out, level-0 leftovers of the three
  * neighbour searches [3], level-1 leftovers [3], valid rows of the ICP inputs [6], their voxel counts [6];
- * with n >= 29 also the mid-level leftovers of the three searches [3] (entries 26-28) */
+ * with n >= 29 also the mid-level leftovers of the three searches [3] (entries 26-28); with n >= 35 also twice
+ * the crop median of each sensor [6] (entries 29-34; 0 without the crop) */
 KP_EXPORT int kp_pipeline_frame_counts(kp_pipeline *p, int64_t *h_counts, int n);
 KP_EXPORT int kp_pipeline_profile(kp_pipeline *p, int enable_or_read, int max_entries,
                                   const char **h_names, double *h_ms, int64_t *h_calls, double *h_bytes, int *h_n);

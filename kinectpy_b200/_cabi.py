@@ -40,6 +40,7 @@ class PipelineCfg(C.Structure):
         ("do_icp", C.c_int32), ("icp_voxel", C.c_double), ("icp_max_corr", C.c_double), ("icp_max_iter", C.c_int32),
         ("normals_max_nn", C.c_int32), ("normals_radius", C.c_double),
         ("seed", C.c_uint64), ("n_streams", C.c_int32),
+        ("do_crop", C.c_int32), ("crop_gate", C.c_double), ("resample_n", C.c_int32), ("resample_mode", C.c_int32),
     ]
 
 
@@ -115,6 +116,7 @@ SIGNATURES = {
     "kp_pipeline_frame_counts": (C.c_int, [_vp, _pi64, C.c_int]),
     "kp_pipeline_profile": (C.c_int, [_vp, C.c_int, C.c_int, C.POINTER(C.c_char_p), _pf64, _pi64, _pf64, C.POINTER(C.c_int)]),
     "kp_pipeline_run_host": (C.c_int, [_vp, _vp, _i64, C.POINTER(FrameResult), _vp, _i64]),
+    "kp_pipeline_run_ex": (C.c_int, [_vp, _vp, _vp, C.c_int, _i64, _vp, C.POINTER(FrameResult), _vp, _i64, _vp]),
 }
 
 _lib = None

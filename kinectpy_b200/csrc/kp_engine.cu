@@ -18,8 +18,19 @@
 #include "kp_batch.cuh"
 
 int kp_unproject_engine(kp_ctx *ctx, const uint16_t *d_depth, const float *d_xytab, const double *h_T, int B, int S, int64_t P,
-                        int flags, double scale, float *d_xyz, float *d_xyz_raw, int32_t *d_slots, int32_t *d_rows);
+                        int flags, double scale, float *d_xyz, float *d_xyz_raw, int32_t *d_slots, int32_t *d_rows,
+                        const uint8_t *d_rgb, const double *d_crop_med, double crop_gate);
 size_t kp_unproject_engine_slots(int B, int S, int64_t P);
+int kp_crop_median_engine(kp_ctx *ctx, const uint16_t *d_depth, const uint32_t *d_vbits, int B, int S, int64_t P, uint32_t *d_hist,
+                          double *d_med);
+size_t kp_crop_median_hist_elems();
+int kp_resample_engine(kp_ctx *ctx, const float *const *d_base, int64_t stride, const int32_t *d_n, int64_t n_step, int B, int64_t N, int mode,
+                       uint64_t seed, const int64_t *h_ids, int32_t *d_status, int64_t status_step, uint32_t *keys, uint32_t *hist,
+                       void *st, unsigned long long *list, float *d_out);
+size_t kp_resample_engine_hist_elems();
+size_t kp_resample_engine_state_bytes();
+int64_t kp_resample_engine_cap(int64_t N);
+bool kp_resample_engine_fits(int64_t N);
 
 namespace {
 constexpr int ENG_MAX_S = 6;
@@ -1031,6 +1042,14 @@ __global__ void __launch_bounds__(256) k_e_copy_out(const __grid_constant__ Fini
         for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < 3LL * n; e += (int64_t)gridDim.x * blockDim.x) dst[e] = src[e];
     }
 }
+// where each frame's final cloud starts (the fixed-N resample reads it from there)
+__global__ void k_e_final_src(const __grid_constant__ FinishArgs a, int B, const float **src_out)
+{
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= B) return;
+    int n;
+    finish_pick(a, f, src_out[f], n);
+}
 __global__ void k_e_check_stride(EngDyn *dyn, kp_frame_result *res, int B, int64_t out_stride)
 {
     const int f = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1054,6 +1073,13 @@ struct EngSlot {
     std::vector<void *> allocs;
     // K1
     uint16_t *d_depth = nullptr;                      // staging for host depth [B][S][P]
+    uint8_t *d_rgb = nullptr;                         // crop: staging for host segmentation images [B][S][P][3]
+    uint32_t *crop_hist = nullptr;                    // crop: median-pass histograms [B*S][...] (zero between calls)
+    double *crop_med = nullptr;                       // crop: median of every (frame, sensor) of the last batch [B][S]
+    uint32_t *rs_hist = nullptr;                      // fixed-N output: radix-select histograms [B][...] (zero between calls)
+    void *rs_st = nullptr;                            //   per-frame selection state
+    unsigned long long *rs_list = nullptr;            //   candidate lists [B][cap]
+    const float **fin_src = nullptr;                  //   first row of each frame's final cloud [B]
     int32_t *k1_slots = nullptr, *k1_rows = nullptr;
     float *fused = nullptr, *icp_in = nullptr;        // [B][NP][3]
     EngDyn *dyn = nullptr;
@@ -1111,6 +1137,7 @@ struct kp_pipeline {
     int knn_rad = 1;                  // level-0 block radius in cells (KP_KNN_RAD): 1 = 27 cells of the full edge, 2 = 125 cells of half the edge
     std::vector<EngSlot> slots;
     float *d_tab = nullptr;
+    uint32_t *d_vbits = nullptr;      // crop: [S][(P + 31) / 32] bit set = finite table entry (z16 = 0 elsewhere)
     std::vector<double> T_fuse, T_icp;
     kp_frame_result *h_res = nullptr;   // pinned staging of the result records
     int64_t h_res_cap = 0;
@@ -1496,6 +1523,20 @@ int slot_create(kp_pipeline *pl, EngSlot &s)
 #define SA(ptr, count) KP_TRY(slot_alloc(pl, s, (size_t)(count), &(ptr)))
 #define SAZ(ptr, count) KP_TRY(slot_alloc(pl, s, (size_t)(count), &(ptr), true))
     SAZ(s.d_depth, B * NP);
+    if (c.do_crop) {
+        SAZ(s.d_rgb, B * NP * 3);
+        SAZ(s.crop_hist, (size_t)B * S * kp_crop_median_hist_elems());
+        SAZ(s.crop_med, (size_t)B * S);
+    }
+    if (c.resample_n > 0) {
+        // (the selection's key array is s.keys: the graph is done with it when the resample runs)
+        SAZ(s.rs_hist, (size_t)B * kp_resample_engine_hist_elems());
+        uint8_t *st = nullptr;
+        SAZ(st, (size_t)B * kp_resample_engine_state_bytes());
+        s.rs_st = st;
+        SA(s.rs_list, (size_t)B * kp_resample_engine_cap(c.resample_n));
+        SA(s.fin_src, B);
+    }
     SA(s.k1_slots, kp_unproject_engine_slots(B, S, P));
     SAZ(s.k1_rows, (size_t)B * S * 2 * 8);
     SA(s.fused, B * NP * 3);
@@ -1696,11 +1737,28 @@ int slot_capture(kp_pipeline *pl, EngSlot &s)
     return KP_OK;
 }
 
-int run_impl(kp_pipeline *p, const uint16_t *depth, int depth_on_device, int64_t F, kp_frame_result *h_results, float *out_xyz,
-             int64_t out_stride)
+// K1 of a batch (outside the graph): with the crop, the median pass over the batch's depth first
+int enqueue_k1(kp_pipeline *p, EngSlot &s, const uint16_t *d_depth, const uint8_t *d_rgb, int nf)
+{
+    const kp_pipeline_cfg &c = p->cfg;
+    const int S = c.S;
+    if (c.do_crop) KP_TRY(kp_crop_median_engine(s.ctx, d_depth, p->d_vbits, nf, S, c.P, s.crop_hist, s.crop_med));
+    return kp_unproject_engine(s.ctx, d_depth, p->d_tab, p->T_fuse.data(), nf, S, c.P, c.unproject_flags, c.scale, s.fused,
+                               (c.do_icp && S > 1) ? s.icp_in : nullptr, s.k1_slots, s.k1_rows, c.do_crop ? d_rgb : nullptr,
+                               s.crop_med, c.crop_gate);
+}
+
+int run_impl(kp_pipeline *p, const uint16_t *depth, const uint8_t *rgb, int depth_on_device, int64_t F, const int64_t *h_frame_ids,
+             kp_frame_result *h_results, float *out_xyz, int64_t out_stride, float *d_fixed)
 {
     if (!p || !h_results || F < 0 || (F > 0 && !depth)) return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_run: bad argument");
     if (out_xyz && out_stride <= 0) { p->err = "kp_pipeline_run: out_stride must be > 0 when an output buffer is given"; return KP_E_ARG; }
+    if (F > 0 && !rgb != !p->cfg.do_crop) {
+        p->err = p->cfg.do_crop ? "kp_pipeline_run: this pipeline crops: it needs the segmentation images (rgb)"
+                                : "kp_pipeline_run: rgb given to a pipeline created without the crop";
+        return KP_E_ARG;
+    }
+    if (d_fixed && p->cfg.resample_n <= 0) { p->err = "kp_pipeline_run: fixed-N output requested from a pipeline with resample_n = 0"; return KP_E_ARG; }
     if (F == 0) return KP_OK;
     const kp_pipeline_cfg &c = p->cfg;
     const int B = p->B, S = c.S;
@@ -1721,14 +1779,18 @@ int run_impl(kp_pipeline *p, const uint16_t *depth, int depth_on_device, int64_t
         const int64_t f0 = i * B;
         const int nf = (int)(F - f0 < B ? F - f0 : B);
         const uint16_t *d_depth = depth + f0 * NP;
+        const uint8_t *d_rgb = rgb ? rgb + 3 * f0 * NP : nullptr;
         if (!depth_on_device) {
             PL_CUDA(p, cudaMemcpyAsync(s.d_depth, depth + f0 * NP, sizeof(uint16_t) * (size_t)nf * NP, cudaMemcpyHostToDevice, ctx->stream));
             d_depth = s.d_depth;
+            if (rgb) {
+                PL_CUDA(p, cudaMemcpyAsync(s.d_rgb, d_rgb, 3 * (size_t)nf * NP, cudaMemcpyHostToDevice, ctx->stream));
+                d_rgb = s.d_rgb;
+            }
         }
         // frames of a short last batch beyond nf: empty bounds rows -> empty clouds, every stage is a no-op for them
         if (nf < B) PL_CUDA(p, cudaMemsetAsync(s.k1_rows, 0, sizeof(int32_t) * (size_t)B * S * 2 * 8, ctx->stream));
-        int rc = kp_unproject_engine(ctx, d_depth, p->d_tab, p->T_fuse.data(), nf, S, c.P, c.unproject_flags, c.scale, s.fused,
-                                     (c.do_icp && S > 1) ? s.icp_in : nullptr, s.k1_slots, s.k1_rows);
+        int rc = enqueue_k1(p, s, d_depth, d_rgb, nf);
         if (rc != KP_OK) { p->err = ctx->err; return rc; }
         if (direct) {
             rc = enqueue_core(p, s, !p->profiling);
@@ -1744,6 +1806,19 @@ int run_impl(kp_pipeline *p, const uint16_t *depth, int depth_on_device, int64_t
             ctx->launches++;
             k_e_check_stride<<<kp_blocks(nf, 32), 32, 0, ctx->stream>>>(s.dyn, s.d_res, nf, out_stride);
             ctx->launches++;
+        }
+        if (d_fixed) {
+            // each frame's fixed-N slot from its final cloud, sample stream = its frame id; short / overflowing frames
+            // get their status in the result record (written by the graph's k_e_finish just before)
+            int64_t ids[16];
+            for (int b = 0; b < nf; ++b) ids[b] = h_frame_ids ? h_frame_ids[f0 + b] : f0 + b;
+            FinishArgs fa{s.dyn, s.d_res, S, c.sor_k > 0 ? s.Bb : s.A, s.E, s.Fin, p->NPr, c.do_floor, c.floor_sor_k > 0, nullptr, 0};
+            k_e_final_src<<<kp_blocks(nf, 32), 32, 0, ctx->stream>>>(fa, nf, s.fin_src);
+            ctx->launches++;
+            rc = kp_resample_engine(ctx, s.fin_src, p->NPr, &s.dyn->n_out, (int64_t)(sizeof(EngDyn) / 4), nf, c.resample_n, c.resample_mode,
+                                    c.seed, ids, &s.d_res->status, (int64_t)(sizeof(kp_frame_result) / 4), s.keys, s.rs_hist, s.rs_st,
+                                    s.rs_list, d_fixed + 3 * f0 * (int64_t)c.resample_n);
+            if (rc != KP_OK) { p->err = ctx->err; return rc; }
         }
         PL_CUDA(p, cudaMemcpyAsync(p->h_res + f0, s.d_res, sizeof(kp_frame_result) * (size_t)nf, cudaMemcpyDeviceToHost, ctx->stream));
     }
@@ -1763,7 +1838,8 @@ int run_impl(kp_pipeline *p, const uint16_t *depth, int depth_on_device, int64_t
         if (h_results[f].status != KP_OK) {
             char buf[160];
             snprintf(buf, sizeof buf, "frame %lld: status %d (%s)", (long long)f, h_results[f].status,
-                     h_results[f].status == KP_E_RANGE ? "out_stride smaller than the frame's final cloud, or voxel / grid range exceeded" : "error");
+                     h_results[f].status == KP_E_RANGE ? "out_stride smaller than the frame's final cloud, voxel / grid range exceeded, or resample candidate list overflow"
+                     : h_results[f].status == KP_E_ARG ? "fewer final points than resample_n (select_points_randomly)" : "error");
             p->err = buf;
             return h_results[f].status;
         }
@@ -1782,6 +1858,12 @@ int kp_pipeline_create(int device, const kp_pipeline_cfg *cfg, const float *h_xy
         return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: segment_plane needs 3 <= ransac_n <= %d, iterations >= 1, threshold > 0", RS_MAX_N);
     if (cfg->do_icp && cfg->S > 1 && (!(cfg->icp_voxel > 0.0) || !(cfg->icp_max_corr > 0.0) || cfg->normals_max_nn < 1 || !(cfg->normals_radius > 0.0)))
         return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: ICP needs icp_voxel, icp_max_corr, normals_radius > 0 and normals_max_nn >= 1");
+    if (cfg->do_crop && !(cfg->crop_gate >= 0.0))
+        return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: crop_gate must be >= 0 (millimetres)");
+    if (cfg->resample_n != 0 && (cfg->resample_n < 1 || cfg->resample_n > 16384 || !kp_resample_engine_fits(cfg->resample_n)))
+        return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: resample_n must be 0 (off) or 1..16384 (got %d)", cfg->resample_n);
+    if (cfg->resample_n != 0 && cfg->resample_mode != KP_RESAMPLE_RANDOM && cfg->resample_mode != KP_RESAMPLE_PREFIX)
+        return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: resample_mode must be KP_RESAMPLE_RANDOM or KP_RESAMPLE_PREFIX");
     *out = nullptr;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
@@ -1838,6 +1920,18 @@ int kp_pipeline_create(int device, const kp_pipeline_cfg *cfg, const float *h_xy
     };
     if (cudaMalloc((void **)&p->d_tab, sizeof(float) * 2 * NP) != cudaSuccess) { p->err = "table allocation failed"; return fail(KP_E_NOMEM); }
     if (cudaMemcpy(p->d_tab, h_xytab, sizeof(float) * 2 * NP, cudaMemcpyHostToDevice) != cudaSuccess) { p->err = "table copy failed"; return fail(KP_E_CUDA); }
+    if (cfg->do_crop) {
+        // the crop median counts a pixel outside the table as z = 0: which pixels those are, one bit each
+        const int64_t words = (cfg->P + 31) / 32;
+        std::vector<uint32_t> bits((size_t)S * words, 0u);
+        for (int s = 0; s < S; ++s)
+            for (int64_t i = 0; i < cfg->P; ++i) {
+                const float *t = h_xytab + 2 * ((size_t)s * cfg->P + i);
+                if (!(t[0] != t[0] || t[1] != t[1])) bits[(size_t)s * words + i / 32] |= 1u << (i % 32);
+            }
+        if (cudaMalloc((void **)&p->d_vbits, sizeof(uint32_t) * bits.size()) != cudaSuccess) { p->err = "table bitmap allocation failed"; return fail(KP_E_NOMEM); }
+        if (cudaMemcpy(p->d_vbits, bits.data(), sizeof(uint32_t) * bits.size(), cudaMemcpyHostToDevice) != cudaSuccess) { p->err = "table bitmap copy failed"; return fail(KP_E_CUDA); }
+    }
     p->slots.resize((size_t)W);
     for (auto &s : p->slots) {
         int rc = slot_create(p, s);
@@ -1846,8 +1940,7 @@ int kp_pipeline_create(int device, const kp_pipeline_cfg *cfg, const float *h_xy
     // One untimed pass over empty frames per slot: loads every kernel outside a capture and proves the launch
     // sequence on the degenerate input; then the sequence is captured as the slot's graph.
     for (auto &s : p->slots) {
-        int rc = kp_unproject_engine(s.ctx, s.d_depth, p->d_tab, p->T_fuse.data(), B, S, cfg->P, cfg->unproject_flags, cfg->scale, s.fused,
-                                     (cfg->do_icp && S > 1) ? s.icp_in : nullptr, s.k1_slots, s.k1_rows);
+        int rc = enqueue_k1(p, s, s.d_depth, s.d_rgb, B);
         if (rc == KP_OK) rc = enqueue_core(p, s, true);
         if (rc != KP_OK) { p->err = s.ctx->err.empty() ? s.aux->err : s.ctx->err; return fail(rc); }
         if (cudaStreamSynchronize(s.ctx->stream) != cudaSuccess || cudaStreamSynchronize(s.aux->stream) != cudaSuccess) {
@@ -1871,6 +1964,7 @@ int kp_pipeline_destroy(kp_pipeline *p)
     cudaSetDevice(p->device);
     for (auto &s : p->slots) slot_destroy(s);
     if (p->d_tab) cudaFree(p->d_tab);
+    if (p->d_vbits) cudaFree(p->d_vbits);
     if (p->h_res) cudaFreeHost(p->h_res);
     delete p;
     return KP_OK;
@@ -1881,7 +1975,13 @@ const char *kp_pipeline_last_error(kp_pipeline *p) { return p ? p->err.c_str() :
 int kp_pipeline_run(kp_pipeline *p, const uint16_t *depth, int depth_on_device, int64_t F, kp_frame_result *h_results,
                     float *d_out_xyz, int64_t out_stride)
 {
-    return run_impl(p, depth, depth_on_device, F, h_results, d_out_xyz, out_stride);
+    return run_impl(p, depth, nullptr, depth_on_device, F, nullptr, h_results, d_out_xyz, out_stride, nullptr);
+}
+
+int kp_pipeline_run_ex(kp_pipeline *p, const uint16_t *depth, const uint8_t *rgb, int inputs_on_device, int64_t F,
+                       const int64_t *h_frame_ids, kp_frame_result *h_results, float *d_out_xyz, int64_t out_stride, float *d_fixed)
+{
+    return run_impl(p, depth, rgb, inputs_on_device, F, h_frame_ids, h_results, d_out_xyz, out_stride, d_fixed);
 }
 
 int kp_pipeline_run_host(kp_pipeline *p, const uint16_t *h_depth, int64_t F, kp_frame_result *h_results, float *h_out_xyz,
@@ -1897,7 +1997,7 @@ int kp_pipeline_run_host(kp_pipeline *p, const uint16_t *h_depth, int64_t F, kp_
             return KP_E_ARG;
         }
     }
-    return run_impl(p, h_depth, 0, F, h_results, h_out_xyz, out_stride);
+    return run_impl(p, h_depth, nullptr, 0, F, nullptr, h_results, h_out_xyz, out_stride, nullptr);
 }
 
 int64_t kp_pipeline_launch_count(kp_pipeline *p)
@@ -1937,6 +2037,12 @@ int kp_pipeline_frame_counts(kp_pipeline *p, int64_t *h_counts, int n)
     for (int i = 0; i < 6; ++i) { h_counts[14 + i] = i < p->cfg.S ? cl[i].nv : 0; h_counts[20 + i] = i < p->cfg.S ? cl[i].n : 0; }
     if (n >= 29)
         for (int i = 0; i < 3; ++i) h_counts[26 + i] = d.cnt_lm[i];
+    if (n >= 35) {
+        // twice the crop median of each sensor (a multiple of 0.5: exact), 0 without the crop
+        double med[ENG_MAX_S] = {0.0};
+        if (p->cfg.do_crop && cudaMemcpy(med, s.crop_med, sizeof(double) * p->cfg.S, cudaMemcpyDeviceToHost) != cudaSuccess) return KP_E_CUDA;
+        for (int i = 0; i < 6; ++i) h_counts[29 + i] = i < p->cfg.S ? (int64_t)(2.0 * med[i]) : 0;
+    }
     return KP_OK;
 }
 

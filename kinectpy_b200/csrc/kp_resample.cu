@@ -15,8 +15,12 @@
 //            pass restricted to the keys that match the prefix found so far; no data moves
 //   collect  keys <= threshold appended (warp-aggregated atomics) as 64-bit (key << 32 | index)
 //   sort     one CTA per cloud: bitonic sort of those ~N entries in shared memory, gather of the first N
-// A cloud whose candidate list overflows (more than 2048 keys tie with the threshold: never for hashed
-// keys) or whose N exceeds the shared-memory sort falls back to a full stable radix sort of (key, index).
+// The clouds of a batch are either CSR rows of one array (kp_resample_batch) or the fixed-stride final clouds of the
+// frame engine with their row counts in device memory (RselClouds).  For CSR input, a cloud whose candidate list
+// overflows (more than 2048 keys tie with the threshold: never for hashed keys) or whose N exceeds the
+// shared-memory sort falls back to a full stable radix sort of (key, index); the engine has no host round trip, so
+// there a short cloud or an overflow is the frame's status and its slot is zero-filled.
+#include <string.h>
 #include <vector>
 #include "kp_common.cuh"
 
@@ -29,6 +33,29 @@ struct RselState {
     uint32_t nvalid;      // non-NaN points
     uint32_t count;       // entries appended by collect
 };
+
+constexpr int RSEL_MAX_IDS = 16;       // frame ids carried in the launch parameters (the engine's frames per launch)
+
+// where cloud b lives: CSR rows off[b] .. off[b+1] of the points, or n_dev[b * n_step] rows (a count the device
+// wrote) from base[b] (a pointer the device wrote) with keys at b * stride; sample stream first_stream + b, or ids[b];
+// status (nullable): int32 per cloud at b * status_step
+struct RselClouds {
+    const int64_t *off;
+    const float *const *base;
+    int64_t stride;
+    const int32_t *n_dev; int64_t n_step;
+    uint64_t first_stream;
+    int use_ids;
+    uint64_t ids[RSEL_MAX_IDS];
+    int32_t *status; int64_t status_step;
+};
+// o: first key of the cloud; pts: its first point
+__device__ __forceinline__ void rsel_cloud(const RselClouds &c, const float *xyz, int b, int64_t &o, int64_t &n, const float *&pts)
+{
+    if (c.off) { o = c.off[b]; n = c.off[b + 1] - o; pts = xyz + 3 * o; }
+    else { o = (int64_t)b * c.stride; n = c.n_dev[(int64_t)b * c.n_step]; pts = c.base[b]; }
+}
+__device__ __forceinline__ uint64_t rsel_stream(const RselClouds &c, int b) { return c.use_ids ? c.ids[b] : c.first_stream + (uint64_t)b; }
 
 __device__ __forceinline__ uint32_t resample_key(const float *xyz, int64_t i, uint64_t seed, uint64_t stream)
 {
@@ -50,17 +77,19 @@ __global__ void __launch_bounds__(256) k_resample_keys(const float *xyz, int64_t
 }
 
 // batched: keys of every cloud + per-cloud valid count + first-pass histogram (top 11 bits)
-__global__ void __launch_bounds__(256) k_rsel_keys(const float *xyz, const int64_t *off, uint64_t seed, uint64_t first_stream,
+__global__ void __launch_bounds__(256) k_rsel_keys(const float *xyz, const __grid_constant__ RselClouds c, uint64_t seed,
                                                    uint32_t *keys, uint32_t *hist, RselState *st)
 {
     __shared__ uint32_t sh[RSEL_BINS];
     const int b = blockIdx.y;
-    const int64_t o = off[b], n = off[b + 1] - o;
+    int64_t o, n;
+    const float *pts;
+    rsel_cloud(c, xyz, b, o, n, pts);
     for (int e = threadIdx.x; e < RSEL_BINS; e += 256) sh[e] = 0;
     __syncthreads();
     int valid = 0;
     for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (int64_t)gridDim.x * 256) {
-        const uint32_t key = resample_key(xyz + 3 * o, i, seed, first_stream + (uint64_t)b);
+        const uint32_t key = resample_key(pts, i, seed, rsel_stream(c, b));
         keys[o + i] = key;
         valid += key != 0xffffffffu;
         atomicAdd(&sh[key >> 21], 1u);
@@ -73,11 +102,14 @@ __global__ void __launch_bounds__(256) k_rsel_keys(const float *xyz, const int64
 }
 
 // histogram of the next digit over the keys that match the prefix (pass 1: bits 20..10, pass 2: bits 9..0)
-__global__ void __launch_bounds__(256) k_rsel_hist(const uint32_t *keys, const int64_t *off, int pass, uint32_t *hist, const RselState *st)
+__global__ void __launch_bounds__(256) k_rsel_hist(const uint32_t *keys, const __grid_constant__ RselClouds c, int pass, uint32_t *hist,
+                                                   const RselState *st)
 {
     __shared__ uint32_t sh[RSEL_BINS];
     const int b = blockIdx.y;
-    const int64_t o = off[b], n = off[b + 1] - o;
+    int64_t o, n;
+    const float *pts;
+    rsel_cloud(c, nullptr, b, o, n, pts);
     for (int e = threadIdx.x; e < RSEL_BINS; e += 256) sh[e] = 0;
     __syncthreads();
     const uint32_t prefix = st[b].prefix;
@@ -121,10 +153,13 @@ __global__ void __launch_bounds__(256) k_rsel_pick(uint32_t *hist, int pass, uin
 }
 
 // keys <= threshold -> list[b][cap] as (key << 32 | index), any order
-__global__ void __launch_bounds__(256) k_rsel_collect(const uint32_t *keys, const int64_t *off, RselState *st, unsigned long long *list, int cap)
+__global__ void __launch_bounds__(256) k_rsel_collect(const uint32_t *keys, const __grid_constant__ RselClouds c, RselState *st,
+                                                      unsigned long long *list, int cap)
 {
     const int b = blockIdx.y;
-    const int64_t o = off[b], n = off[b + 1] - o;
+    int64_t o, n;
+    const float *pts;
+    rsel_cloud(c, nullptr, b, o, n, pts);
     const uint32_t T = st[b].prefix;                    // after three picks: the full 32-bit threshold key
     const int lane = threadIdx.x & 31;
     for (int64_t i0 = (int64_t)blockIdx.x * 256 + (threadIdx.x & ~31); i0 < n; i0 += (int64_t)gridDim.x * 256) {
@@ -141,34 +176,70 @@ __global__ void __launch_bounds__(256) k_rsel_collect(const uint32_t *keys, cons
     }
 }
 
-// one CTA per cloud: bitonic sort of the candidate list in shared memory, then the first N rows are gathered
-__global__ void __launch_bounds__(1024) k_rsel_sort_gather(const float *xyz, const int64_t *off, const RselState *st,
+// one CTA per cloud: sort of the candidate list in shared memory, then the first N rows are gathered.  The sorting
+// network is the bitonic one whose merges all run ascending (each merge starts by comparing i with its mirror in the
+// block), so the entries past the list -- +inf in a power-of-two array -- never move and are never stored: the buffer
+// holds `cap` entries, not the next power of two.  A cloud with fewer than N valid points or an overflowing list
+// returns untouched (the host checks the state), or, with a status array, gets that status and a zero slot.
+__global__ void __launch_bounds__(1024) k_rsel_sort_gather(const float *xyz, const __grid_constant__ RselClouds c, const RselState *st,
                                                            const unsigned long long *list, int cap, int cap2, int64_t N,
                                                            float *out, int32_t *index_out)
 {
     extern __shared__ unsigned long long sm[];
     const int b = blockIdx.x;
     const uint32_t cnt = st[b].count;
-    if (st[b].nvalid < (uint32_t)N || cnt > (uint32_t)cap) return;        // error / fallback: the host looks at the state
-    for (int e = threadIdx.x; e < cap2; e += 1024) sm[e] = (uint32_t)e < cnt ? list[(size_t)b * cap + e] : ~0ull;
+    if (st[b].nvalid < (uint32_t)N || cnt > (uint32_t)cap) {
+        if (c.status) {
+            if (threadIdx.x == 0) {
+                int32_t *sp = c.status + (int64_t)b * c.status_step;
+                if (*sp == KP_OK) *sp = st[b].nvalid < (uint32_t)N ? KP_E_ARG : KP_E_RANGE;
+            }
+            for (int64_t e = threadIdx.x; e < 3 * N; e += 1024) out[3 * (size_t)b * (size_t)N + (size_t)e] = 0.0f;
+        }
+        return;
+    }
+    for (int e = threadIdx.x; e < cap; e += 1024) sm[e] = (uint32_t)e < cnt ? list[(size_t)b * cap + e] : ~0ull;
     __syncthreads();
     for (int size = 2; size <= cap2; size <<= 1)
         for (int stride = size >> 1; stride > 0; stride >>= 1) {
             for (int t = threadIdx.x; t < (cap2 >> 1); t += 1024) {
-                const int i = ((t / stride) * 2 * stride) + (t % stride), j = i + stride;
-                const bool up = (i & size) == 0;
-                const unsigned long long x = sm[i], y = sm[j];
-                if ((y < x) == up) { sm[i] = y; sm[j] = x; }
+                int i, j;
+                if (stride == (size >> 1)) {            // first step of a merge: i against its mirror in the block
+                    i = (t / stride) * size + (t % stride);
+                    j = (t / stride) * size + size - 1 - (t % stride);
+                } else {
+                    i = ((t / stride) * 2 * stride) + (t % stride);
+                    j = i + stride;
+                }
+                if (j < cap) {
+                    const unsigned long long x = sm[i], y = sm[j];
+                    if (y < x) { sm[i] = y; sm[j] = x; }
+                }
             }
             __syncthreads();
         }
-    const float *src = xyz + 3 * off[b];
+    int64_t o, n;
+    const float *src;
+    rsel_cloud(c, xyz, b, o, n, src);
     for (int64_t t = threadIdx.x; t < N; t += 1024) {
         const int64_t i = (int64_t)(uint32_t)sm[t];
-        float *o = out + 3 * ((size_t)b * (size_t)N + (size_t)t);
-        o[0] = src[3 * i]; o[1] = src[3 * i + 1]; o[2] = src[3 * i + 2];
+        float *dst = out + 3 * ((size_t)b * (size_t)N + (size_t)t);
+        dst[0] = src[3 * i]; dst[1] = src[3 * i + 1]; dst[2] = src[3 * i + 2];
         if (index_out) index_out[(size_t)b * (size_t)N + (size_t)t] = (int32_t)i;
     }
+}
+
+// PREFIX mode with device counts: slot b = the first min(n, N) rows of cloud b, then zeros
+__global__ void __launch_bounds__(256) k_rsel_prefix(const float *xyz, const __grid_constant__ RselClouds c, int64_t N, float *out)
+{
+    const int b = blockIdx.y;
+    int64_t o, n;
+    const float *src;
+    rsel_cloud(c, xyz, b, o, n, src);
+    const int64_t m3 = 3 * (n < N ? n : N);
+    float *dst = out + 3 * (size_t)b * (size_t)N;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < 3 * N; e += (int64_t)gridDim.x * blockDim.x)
+        dst[e] = e < m3 ? src[e] : 0.0f;
 }
 
 __global__ void __launch_bounds__(256) k_resample_gather(const float *xyz, const int32_t *order, int64_t N, float *out,
@@ -210,16 +281,63 @@ int resample_full_sort(kp_ctx *ctx, const float *d_xyz, int64_t n, int64_t N, ui
     return KP_OK;
 }
 
-// random mode for a batch of clouds (d_off: device copy of the CSR offsets)
+// list capacity of the candidate sort (N + the 2048 ties it tolerates) and the power of two its network spans
+void rsel_sizes(int64_t N, int &cap, int &cap2)
+{
+    cap = (int)N + 2048;
+    cap2 = 1024;
+    while (cap2 < cap) cap2 <<= 1;
+}
+constexpr size_t RSEL_SORT_SMEM = 160 * 1024;
+
+// the selection launches for B clouds: keys, three histogram + pick passes, collect, sort + gather.
+// keys: one uint32 per row, addressed like the points; hist [B][RSEL_BINS] zero on entry (the picks leave it zero);
+// st [B] zeroed here; list [B][cap].
+int rsel_launch(kp_ctx *ctx, const float *d_xyz, const RselClouds &c, int B, int64_t N, uint64_t seed, unsigned gx, double rows,
+                uint32_t *keys, uint32_t *hist, RselState *st, unsigned long long *list, float *d_out, int32_t *d_index_out)
+{
+    int cap, cap2;
+    rsel_sizes(N, cap, cap2);
+    KP_CUDA(ctx, cudaMemsetAsync(st, 0, sizeof(RselState) * (size_t)B, ctx->stream));
+    const dim3 grid(gx, (unsigned)B);
+    {
+        KP_PROFB(ctx, "resample_keys", rows * (4.0 + 4.0));
+        k_rsel_keys<<<grid, 256, 0, ctx->stream>>>(d_xyz, c, seed, keys, hist, st);
+        KP_LAUNCH_CHECK(ctx);
+    }
+    {
+        KP_PROFB(ctx, "resample_select", rows * (2.0 * 4.0 + 4.0) + (double)B * (double)N * 8.0);
+        for (int pass = 0; pass < 3; ++pass) {
+            if (pass > 0) {
+                k_rsel_hist<<<grid, 256, 0, ctx->stream>>>(keys, c, pass, hist, st);
+                KP_LAUNCH_CHECK(ctx);
+            }
+            k_rsel_pick<<<B, 256, 0, ctx->stream>>>(hist, pass, (uint32_t)N, st);
+            KP_LAUNCH_CHECK(ctx);
+        }
+        k_rsel_collect<<<grid, 256, 0, ctx->stream>>>(keys, c, st, list, cap);
+        KP_LAUNCH_CHECK(ctx);
+    }
+    {
+        KP_PROFB(ctx, "resample_gather", (double)B * (double)N * (8.0 + 12.0 + 12.0));
+        const size_t smem = (size_t)cap * sizeof(unsigned long long);
+        if (smem > 48 * 1024)
+            KP_CUDA(ctx, cudaFuncSetAttribute(k_rsel_sort_gather, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_rsel_sort_gather<<<B, 1024, smem, ctx->stream>>>(d_xyz, c, st, list, cap, cap2, N, d_out, d_index_out);
+        KP_LAUNCH_CHECK(ctx);
+    }
+    return KP_OK;
+}
+
+// random mode for a batch of clouds given by host CSR offsets
 int resample_select_batch(kp_ctx *ctx, const float *d_xyz, const int64_t *h_off, int B, int64_t N, uint64_t seed,
                           uint64_t first_stream, float *d_out, int32_t *d_index_out)
 {
     int64_t total = h_off[B] - h_off[0], maxn = 0;
     for (int b = 0; b < B; ++b) maxn = h_off[b + 1] - h_off[b] > maxn ? h_off[b + 1] - h_off[b] : maxn;
-    const int cap = (int)N + 2048;
-    int cap2 = 1024;
-    while (cap2 < cap) cap2 <<= 1;
-    const bool cta_sort = (size_t)cap2 * 8 <= 160 * 1024;
+    int cap, cap2;
+    rsel_sizes(N, cap, cap2);
+    const bool cta_sort = (size_t)cap * 8 <= RSEL_SORT_SMEM;
     if (!cta_sort || total <= 0) {
         for (int b = 0; b < B; ++b) {
             kp_ws_reset(ctx);
@@ -240,38 +358,14 @@ int resample_select_batch(kp_ctx *ctx, const float *d_xyz, const int64_t *h_off,
     // offsets relative to d_xyz (the caller's rows h_off[0].. are addressed through them directly)
     KP_CUDA(ctx, cudaMemcpyAsync(d_off, h_off, sizeof(int64_t) * ((size_t)B + 1), cudaMemcpyHostToDevice, ctx->stream));
     KP_CUDA(ctx, cudaMemsetAsync(hist, 0, sizeof(uint32_t) * (size_t)B * RSEL_BINS, ctx->stream));
-    KP_CUDA(ctx, cudaMemsetAsync(st, 0, sizeof(RselState) * (size_t)B, ctx->stream));
     uint32_t *keys_rel = keys - h_off[0];                     // keys[o + i] with o = absolute offset
     unsigned gx = (unsigned)((maxn + 2047) / 2048);
     if (gx < 1) gx = 1;
     if (gx > 1024) gx = 1024;
-    const dim3 grid(gx, (unsigned)B);
-    {
-        KP_PROFB(ctx, "resample_keys", (double)total * (4.0 + 4.0));
-        k_rsel_keys<<<grid, 256, 0, ctx->stream>>>(d_xyz, d_off, seed, first_stream, keys_rel, hist, st);
-        KP_LAUNCH_CHECK(ctx);
-    }
-    {
-        KP_PROFB(ctx, "resample_select", (double)total * (2.0 * 4.0 + 4.0) + (double)B * (double)N * 8.0);
-        for (int pass = 0; pass < 3; ++pass) {
-            if (pass > 0) {
-                k_rsel_hist<<<grid, 256, 0, ctx->stream>>>(keys_rel, d_off, pass, hist, st);
-                KP_LAUNCH_CHECK(ctx);
-            }
-            k_rsel_pick<<<B, 256, 0, ctx->stream>>>(hist, pass, (uint32_t)N, st);
-            KP_LAUNCH_CHECK(ctx);
-        }
-        k_rsel_collect<<<grid, 256, 0, ctx->stream>>>(keys_rel, d_off, st, list, cap);
-        KP_LAUNCH_CHECK(ctx);
-    }
-    {
-        KP_PROFB(ctx, "resample_gather", (double)B * (double)N * (8.0 + 12.0 + 12.0));
-        const size_t smem = (size_t)cap2 * sizeof(unsigned long long);
-        if (smem > 48 * 1024)
-            KP_CUDA(ctx, cudaFuncSetAttribute(k_rsel_sort_gather, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_rsel_sort_gather<<<B, 1024, smem, ctx->stream>>>(d_xyz, d_off, st, list, cap, cap2, N, d_out, d_index_out);
-        KP_LAUNCH_CHECK(ctx);
-    }
+    RselClouds c;
+    memset(&c, 0, sizeof c);
+    c.off = d_off; c.first_stream = first_stream;
+    KP_TRY(rsel_launch(ctx, d_xyz, c, B, N, seed, gx, (double)total, keys_rel, hist, st, list, d_out, d_index_out));
     // one read for the whole batch: valid counts (the ValueError of np.random.choice) and list overflows (fallback)
     std::vector<RselState> hs((size_t)B);
     KP_CUDA(ctx, cudaMemcpyAsync(hs.data(), st, sizeof(RselState) * (size_t)B, cudaMemcpyDeviceToHost, ctx->stream));
@@ -344,3 +438,39 @@ int kp_resample_batch(kp_ctx *ctx, const float *d_xyz, const int64_t *h_offsets,
 }
 
 }  // extern "C"
+
+// frame engine: fixed-N slot of every frame of a batch, without a host round trip.  Cloud b = d_n[b * n_step] rows
+// from d_base[b] (keys at b * stride), sample stream h_ids[b]; d_status (int32 at b * status_step) takes KP_E_ARG for a RANDOM
+// cloud with fewer than N points and KP_E_RANGE for an overflowing candidate list (a frame that already has a status
+// keeps it); such a slot is zero-filled.  Work buffers (allocated by the caller once): keys [B * stride], hist
+// [B][kp_resample_engine_hist_elems()] zero, st [B] (kp_resample_engine_state_bytes), list [B][kp_resample_engine_cap(N)].
+int kp_resample_engine(kp_ctx *ctx, const float *const *d_base, int64_t stride, const int32_t *d_n, int64_t n_step, int B, int64_t N, int mode,
+                       uint64_t seed, const int64_t *h_ids, int32_t *d_status, int64_t status_step, uint32_t *keys, uint32_t *hist,
+                       void *st, unsigned long long *list, float *d_out)
+{
+    if (B <= 0) return KP_OK;
+    if (B > RSEL_MAX_IDS) return kp_set_err(ctx, KP_E_ARG, "kp_resample_engine: at most %d clouds per launch", RSEL_MAX_IDS);
+    RselClouds c;
+    memset(&c, 0, sizeof c);
+    c.base = d_base; c.stride = stride; c.n_dev = d_n; c.n_step = n_step; c.use_ids = 1;
+    for (int b = 0; b < B; ++b) c.ids[b] = (uint64_t)h_ids[b];
+    c.status = d_status; c.status_step = status_step;
+    // the final clouds are a fraction of the stride: a few CTAs per SM, grid-stride over the rows
+    int64_t gx = ((int64_t)ctx->sm_count * 4 + B - 1) / B;
+    const int64_t gmax = (stride + 2047) / 2048;
+    if (gx > gmax) gx = gmax;
+    if (gx < 1) gx = 1;
+    if (mode == KP_RESAMPLE_PREFIX) {
+        KP_PROFB(ctx, "resample_prefix", (double)B * (double)N * (12.0 + 12.0));
+        k_rsel_prefix<<<dim3((unsigned)gx, (unsigned)B), 256, 0, ctx->stream>>>(nullptr, c, N, d_out);
+        KP_LAUNCH_CHECK(ctx);
+        return KP_OK;
+    }
+    return rsel_launch(ctx, nullptr, c, B, N, seed, (unsigned)gx, (double)B * (double)stride, keys, hist, (RselState *)st, list, d_out,
+                       nullptr);
+}
+size_t kp_resample_engine_hist_elems() { return RSEL_BINS; }
+size_t kp_resample_engine_state_bytes() { return sizeof(RselState); }
+int64_t kp_resample_engine_cap(int64_t N) { int cap, cap2; rsel_sizes(N, cap, cap2); return cap; }
+bool kp_resample_engine_fits(int64_t N) { return (size_t)kp_resample_engine_cap(N) * 8 <= RSEL_SORT_SMEM; }
+

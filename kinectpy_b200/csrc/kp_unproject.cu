@@ -25,6 +25,12 @@ struct UnprojParams {
                            // s >= 1 (the ICP sources, in their own sensor frame) and the transformed master for s = 0;
                            // its bounds go to slot set 1
     double T[UP_MAX_S][12];
+    // CROP variant (frame engine, human crop of preprocessing/data.py:165-178): uint8 [B][S][P][3] segmentation image
+    // and the (frame, sensor) median of the int16 z column [B][S]; kept after the fields above so that the other
+    // variants address their parameters exactly as before
+    const uint8_t *rgb;
+    const double *crop_med;
+    double crop_gate;
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -53,7 +59,9 @@ __device__ __forceinline__ void up_store_rows(float *stage, const float *vals, f
     __syncwarp();
 }
 
-template <bool INT16, bool DROP, bool HAS_T, bool BOUNDS, bool RAW = false>
+// CROP: a pixel reaches the fused cloud only if its segmentation colour is non-black in all three channels and its
+// int16 z (0 outside the table) is <= median + gate; the ICP inputs (xyz_raw) and their bounds set ignore the crop.
+template <bool INT16, bool DROP, bool HAS_T, bool BOUNDS, bool RAW = false, bool CROP = false>
 __global__ void __launch_bounds__(UP_THREADS, RAW ? 2 : 3) k_unproject(const __grid_constant__ UnprojParams p)
 {
     __shared__ __align__(128) float2 tab_s[UP_TILE];
@@ -128,6 +136,32 @@ __global__ void __launch_bounds__(UP_THREADS, RAW ? 2 : 3) k_unproject(const __g
         float rmn[3] = {INFINITY, INFINITY, INFINITY}, rmx[3] = {-INFINITY, -INFINITY, -INFINITY};
         int cnt = 0;
         unsigned okmask = 0;
+        // CROP: the master's ICP-input bounds (without the crop), the ICP-input count, the crop's pixel mask
+        float cmn[3] = {INFINITY, INFINITY, INFINITY}, cmx[3] = {-INFINITY, -INFINITY, -INFINITY};
+        int rcnt = 0;
+        unsigned cropmask = 0;
+        if (CROP) {
+            uint8_t c[UP_PPT * 3];
+            const uint8_t *src = p.rgb + 3 * row;
+            if (full && (row % 8 == 0) && ((((uintptr_t)p.rgb) & 7u) == 0u)) {
+                const uint2 *s8 = reinterpret_cast<const uint2 *>(src);
+#pragma unroll
+                for (int q = 0; q < 3; ++q) {
+                    const uint2 w = __ldg(s8 + q);
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) { c[8 * q + k] = (w.x >> (8 * k)) & 0xffu; c[8 * q + 4 + k] = (w.y >> (8 * k)) & 0xffu; }
+                }
+            } else {
+#pragma unroll
+                for (int j = 0; j < UP_PPT * 3; ++j) c[j] = (px0 + j / 3 < npx) ? src[j] : (uint8_t)0;
+            }
+            const double lim = __dadd_rn(p.crop_med[(int64_t)b * p.S + s], p.crop_gate);
+#pragma unroll
+            for (int j = 0; j < UP_PPT; ++j) {
+                const int16_t z16 = (isnan(tb[j].x) || isnan(tb[j].y)) ? (int16_t)0 : (int16_t)dz[j];
+                if (c[3 * j] != 0 && c[3 * j + 1] != 0 && c[3 * j + 2] != 0 && (double)z16 <= lim) cropmask |= 1u << j;
+            }
+        }
 #pragma unroll
         for (int j = 0; j < UP_PPT; ++j) {
             const float xt = tb[j].x, yt = tb[j].y;
@@ -162,6 +196,7 @@ __global__ void __launch_bounds__(UP_THREADS, RAW ? 2 : 3) k_unproject(const __g
                 if (ok) {
                     rmn[0] = fminf(rmn[0], rx); rmn[1] = fminf(rmn[1], ry); rmn[2] = fminf(rmn[2], rz);
                     rmx[0] = fmaxf(rmx[0], rx); rmx[1] = fmaxf(rmx[1], ry); rmx[2] = fmaxf(rmx[2], rz);
+                    if (CROP) ++rcnt;
                 }
             }
             if (HAS_T && ok) {
@@ -170,9 +205,20 @@ __global__ void __launch_bounds__(UP_THREADS, RAW ? 2 : 3) k_unproject(const __g
                 const double z2 = kp_affine(T[8], T[9], T[10], T[11], X, Y, Z);
                 X = x2; Y = y2; Z = z2;
             }
+            if (CROP && RAW && s == 0) {
+                // the master's ICP input is the transformed master without the crop
+                const float rx = ok ? (float)X : NAN, ry = ok ? (float)Y : NAN, rz = ok ? (float)Z : NAN;
+                raw[3 * j] = rx; raw[3 * j + 1] = ry; raw[3 * j + 2] = rz;
+                if (ok) {
+                    cmn[0] = fminf(cmn[0], rx); cmn[1] = fminf(cmn[1], ry); cmn[2] = fminf(cmn[2], rz);
+                    cmx[0] = fmaxf(cmx[0], rx); cmx[1] = fmaxf(cmx[1], ry); cmx[2] = fmaxf(cmx[2], rz);
+                    ++rcnt;
+                }
+            }
+            if (CROP) ok = ok && ((cropmask >> j) & 1u);      // the crop is for the fused cloud only
             float fx3 = ok ? (float)X : NAN, fy3 = ok ? (float)Y : NAN, fz3 = ok ? (float)Z : NAN;
             out[3 * j] = fx3; out[3 * j + 1] = fy3; out[3 * j + 2] = fz3;
-            if (RAW && s == 0) { raw[3 * j] = fx3; raw[3 * j + 1] = fy3; raw[3 * j + 2] = fz3; }
+            if (RAW && !CROP && s == 0) { raw[3 * j] = fx3; raw[3 * j + 1] = fy3; raw[3 * j + 2] = fz3; }
             if (ok) okmask |= 1u << j;
             if (BOUNDS && ok) {
                 ++cnt;
@@ -240,19 +286,21 @@ __global__ void __launch_bounds__(UP_THREADS, RAW ? 2 : 3) k_unproject(const __g
                 slot[1] = make_int4(enc[4], enc[5], enc[6], 0);
             }
             if (RAW) {
-                // set 1: bounds of what went to xyz_raw (the master's are those of set 0)
-                int renc[6] = {kp_f2ord(s ? rmn[0] : mn[0]), kp_f2ord(s ? rmn[1] : mn[1]), kp_f2ord(s ? rmn[2] : mn[2]),
-                               kp_f2ord(s ? rmx[0] : mx[0]), kp_f2ord(s ? rmx[1] : mx[1]), kp_f2ord(s ? rmx[2] : mx[2])};
+                // set 1: bounds of what went to xyz_raw (without the crop the master's are those of set 0)
+                int renc[6] = {kp_f2ord(s ? rmn[0] : (CROP ? cmn[0] : mn[0])), kp_f2ord(s ? rmn[1] : (CROP ? cmn[1] : mn[1])),
+                               kp_f2ord(s ? rmn[2] : (CROP ? cmn[2] : mn[2])), kp_f2ord(s ? rmx[0] : (CROP ? cmx[0] : mx[0])),
+                               kp_f2ord(s ? rmx[1] : (CROP ? cmx[1] : mx[1])), kp_f2ord(s ? rmx[2] : (CROP ? cmx[2] : mx[2]))};
 #pragma unroll
                 for (int c = 0; c < 3; ++c) {
                     renc[c] = __reduce_min_sync(KP_FULL, renc[c]);
                     renc[3 + c] = __reduce_max_sync(KP_FULL, renc[3 + c]);
                 }
+                if (CROP) rcnt = __reduce_add_sync(KP_FULL, rcnt);
                 if (lane == 0) {
                     int4 *slot = reinterpret_cast<int4 *>(p.bounds_enc) +
                                  2 * (((((int64_t)b * p.S + s) * NSETS + 1) * gridDim.x + blockIdx.x) * (UP_THREADS / 32) + (tid >> 5));
                     slot[0] = make_int4(renc[0], renc[1], renc[2], renc[3]);
-                    slot[1] = make_int4(renc[4], renc[5], enc[6], 0);
+                    slot[1] = make_int4(renc[4], renc[5], CROP ? rcnt : enc[6], 0);
                 }
             }
         }
@@ -383,6 +431,142 @@ __global__ void k_crop_mask(const uint8_t *rgb, const int16_t *xyz16, int64_t n,
     keep[i] = nonblack && depth_ok;
 }
 
+// ---- frame engine: the crop median of every (frame, sensor) of a batch, numpy.median over all P int16 z values
+// (zeros included; 0 outside the table).  Two-level radix select on key = (uint16)z16 ^ 0x8000 (signed order):
+// a histogram of the high byte over all pixels, then one of the low byte over the pixels whose high byte is that
+// of one of the two middle ranks.  Histograms: [B*S][CM_BINS] uint32, zero on entry, cleared again by the pick.
+constexpr int CM_THREADS = 256;
+constexpr int CM_BINS = 256 + 2 * 256;          // level 1 | level 2 of rank lo | level 2 of rank hi
+
+struct CropMedParams {
+    const uint16_t *depth;      // [B][S][P]
+    const uint32_t *vbits;      // [S][words]: bit i of sensor s = table entry i is finite
+    int S; int64_t P, words;
+    uint32_t *hist;             // [B*S][CM_BINS]
+    double *med;                // [B*S]
+};
+
+__device__ __forceinline__ void cm_ranks(int64_t P, uint32_t r[2])
+{
+    r[1] = (uint32_t)(P / 2);
+    r[0] = (P % 2) ? r[1] : r[1] - 1;
+}
+
+// the bin of `h` (256 counts, one per thread) that holds rank r[q], and the count before it; every thread gets both
+__device__ void cm_find(const uint32_t *h, const uint32_t r[2], uint32_t *sh_scan /*[CM_THREADS / 32]*/, int bin[2], uint32_t before[2])
+{
+    __shared__ int s_bin[2];
+    __shared__ uint32_t s_before[2];
+    const int t = threadIdx.x, lane = t & 31, w = t >> 5;
+    const uint32_t c = h[t];
+    uint32_t inc = c;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const uint32_t v = __shfl_up_sync(KP_FULL, inc, d);
+        if (lane >= d) inc += v;
+    }
+    if (lane == 31) sh_scan[w] = inc;
+    __syncthreads();
+    uint32_t base = 0;
+    for (int i = 0; i < w; ++i) base += sh_scan[i];
+    const uint32_t lo = base + inc - c;           // exclusive prefix of bin t
+#pragma unroll
+    for (int q = 0; q < 2; ++q)
+        if (lo <= r[q] && r[q] < lo + c) { s_bin[q] = t; s_before[q] = lo; }
+    __syncthreads();
+    for (int q = 0; q < 2; ++q) { bin[q] = s_bin[q]; before[q] = s_before[q]; }
+    __syncthreads();
+}
+
+template <int LEVEL>
+__global__ void __launch_bounds__(CM_THREADS) k_crop_hist(const __grid_constant__ CropMedParams p)
+{
+    constexpr int NB = LEVEL == 0 ? 256 : 512;
+    constexpr int NW = CM_THREADS / 32;
+    __shared__ uint32_t h[NW][NB];                 // one histogram per warp: the depths of a frame cluster in a few bins
+    __shared__ uint32_t scan[NW];
+    const int bs = blockIdx.y, s = bs % p.S;
+    const int w = threadIdx.x >> 5;
+    for (int e = threadIdx.x; e < NW * NB; e += CM_THREADS) (&h[0][0])[e] = 0;
+    int pre[2] = {-1, -1};
+    if (LEVEL == 1) {
+        uint32_t r[2], before[2];
+        cm_ranks(p.P, r);
+        cm_find(p.hist + (size_t)bs * CM_BINS, r, scan, pre, before);
+        if (pre[1] == pre[0]) pre[1] = -1;        // both ranks in one bin: the rank-lo histogram serves both
+    }
+    __syncthreads();
+    const uint16_t *d = p.depth + (size_t)bs * p.P;
+    const uint32_t *vb = p.vbits + (size_t)s * p.words;
+    const int64_t ngroups = (p.P + 7) / 8;
+    const bool vec = (p.P % 8 == 0) && ((((uintptr_t)p.depth) & 15u) == 0u);
+    for (int64_t g = (int64_t)blockIdx.x * CM_THREADS + threadIdx.x; g < ngroups; g += (int64_t)gridDim.x * CM_THREADS) {
+        const int64_t i0 = 8 * g;
+        uint16_t z[8];
+        if (vec) {
+            const uint4 v = __ldg(reinterpret_cast<const uint4 *>(d + i0));
+            z[0] = v.x & 0xffff; z[1] = v.x >> 16; z[2] = v.y & 0xffff; z[3] = v.y >> 16;
+            z[4] = v.z & 0xffff; z[5] = v.z >> 16; z[6] = v.w & 0xffff; z[7] = v.w >> 16;
+        } else {
+#pragma unroll
+            for (int j = 0; j < 8; ++j) z[j] = i0 + j < p.P ? d[i0 + j] : (uint16_t)0;
+        }
+        const uint32_t bits = (uint32_t)(vb[i0 >> 5] >> (i0 & 31)) & 0xffu;    // i0 % 8 == 0: 8 bits of one word
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            if (i0 + j >= p.P) break;
+            const uint32_t key = (((bits >> j) & 1u) ? (uint32_t)z[j] : 0u) ^ 0x8000u;
+            if (LEVEL == 0) {
+                atomicAdd(&h[w][key >> 8], 1u);
+            } else {
+                const int hi = (int)(key >> 8);
+                if (hi == pre[0]) atomicAdd(&h[w][key & 0xffu], 1u);
+                else if (hi == pre[1]) atomicAdd(&h[w][256 + (key & 0xffu)], 1u);
+            }
+        }
+    }
+    __syncthreads();
+    uint32_t *gh = p.hist + (size_t)bs * CM_BINS + (LEVEL == 0 ? 0 : 256);
+    for (int e = threadIdx.x; e < NB; e += CM_THREADS) {
+        uint32_t v = 0;
+#pragma unroll
+        for (int k = 0; k < NW; ++k) v += h[k][e];
+        if (v) atomicAdd(gh + e, v);
+    }
+}
+
+// one CTA per (frame, sensor): the two middle values from the histograms -> median; clears the histograms
+__global__ void __launch_bounds__(CM_THREADS) k_crop_median(const __grid_constant__ CropMedParams p)
+{
+    __shared__ uint32_t scan[CM_THREADS / 32];
+    __shared__ uint32_t h2[2][256];
+    const int bs = blockIdx.x, t = threadIdx.x;
+    uint32_t *gh = p.hist + (size_t)bs * CM_BINS;
+    uint32_t r[2], before[2];
+    int pre[2], lo[2];
+    cm_ranks(p.P, r);
+    cm_find(gh, r, scan, pre, before);
+    h2[0][t] = gh[256 + t];
+    h2[1][t] = gh[512 + t];
+    __syncthreads();
+    for (int e = t; e < CM_BINS; e += CM_THREADS) gh[e] = 0;
+    // rank q inside its high-byte bin; rank hi has its own low-byte histogram only when its bin differs from rank lo's
+    const uint32_t rr[2] = {r[0] - before[0], r[1] - before[1]};
+    uint32_t unused[2];
+    cm_find(h2[0], rr, scan, lo, unused);
+    if (pre[1] != pre[0]) {
+        const uint32_t r1[2] = {rr[1], rr[1]};
+        int l1[2];
+        cm_find(h2[1], r1, scan, l1, unused);
+        lo[1] = l1[1];
+    }
+    if (t == 0) {
+        const double v0 = (double)(int16_t)(uint16_t)((((uint32_t)pre[0] << 8) | (uint32_t)lo[0]) ^ 0x8000u);
+        const double v1 = (double)(int16_t)(uint16_t)((((uint32_t)pre[1] << 8) | (uint32_t)lo[1]) ^ 0x8000u);
+        p.med[bs] = (v0 + v1) * 0.5;
+    }
+}
+
 static void fill_T12(const double *h_T16, double *T12)
 {
     for (int r = 0; r < 3; ++r)
@@ -433,19 +617,22 @@ int kp_unproject_device(kp_ctx *ctx, const uint16_t *d_depth, const float *d_xyt
 // (s = 0: the transformed master, s >= 1: the sub cloud in its own frame) + bounds rows [B][S][2][8] (set 0: fused
 // coordinates of sensor s, set 1: what went to the ICP input).  d_slots: [B*S*2*tiles*8 warps][8] int32 scratch.
 int kp_unproject_engine(kp_ctx *ctx, const uint16_t *d_depth, const float *d_xytab, const double *h_T, int B, int S, int64_t P,
-                        int flags, double scale, float *d_xyz, float *d_xyz_raw, int32_t *d_slots, int32_t *d_rows)
+                        int flags, double scale, float *d_xyz, float *d_xyz_raw, int32_t *d_slots, int32_t *d_rows,
+                        const uint8_t *d_rgb, const double *d_crop_med, double crop_gate)
 {
     if (B <= 0 || S <= 0 || P <= 0) return KP_OK;
     if (S > UP_MAX_S) return kp_set_err(ctx, KP_E_ARG, "frame engine: at most %d sensors (got %d)", UP_MAX_S, S);
-    KP_PROFB(ctx, "unproject_transform", (double)B * S * P * (2.0 + 12.0 + 12.0) + (double)S * P * 8.0);
+    KP_PROFB(ctx, "unproject_transform", (double)B * S * P * (2.0 + 12.0 + 12.0 + (d_rgb ? 3.0 : 0.0)) + (double)S * P * 8.0);
     UnprojParams p;
     p.depth = d_depth; p.tab = (const float2 *)d_xytab; p.B = B; p.S = S; p.P = P; p.flags = flags;
     p.has_T = 1; p.scale = scale; p.xyz = d_xyz; p.valid = nullptr; p.xyz16 = nullptr; p.xyz_raw = d_xyz_raw;
     p.bounds_enc = d_slots;
+    p.rgb = d_rgb; p.crop_med = d_crop_med; p.crop_gate = crop_gate;
     for (int s = 0; s < UP_MAX_S; ++s) fill_T12(h_T && s < S ? h_T + 16 * s : nullptr, p.T[s]);
     const int64_t ntiles = kp_blocks(P, UP_TILE);
     dim3 grid((unsigned)ntiles, (unsigned)S);
-    const int variant = ((flags & KP_UNPROJECT_INT16) ? 1 : 0) | ((flags & KP_UNPROJECT_DROP_ANY_ZERO) ? 2 : 0) | (d_xyz_raw ? 4 : 0);
+    const int variant = ((flags & KP_UNPROJECT_INT16) ? 1 : 0) | ((flags & KP_UNPROJECT_DROP_ANY_ZERO) ? 2 : 0) | (d_xyz_raw ? 4 : 0) |
+                        (d_rgb ? 8 : 0);
     switch (variant) {
     case 0: k_unproject<false, false, true, true, false><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
     case 1: k_unproject<true, false, true, true, false><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
@@ -454,7 +641,15 @@ int kp_unproject_engine(kp_ctx *ctx, const uint16_t *d_depth, const float *d_xyt
     case 4: k_unproject<false, false, true, true, true><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
     case 5: k_unproject<true, false, true, true, true><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
     case 6: k_unproject<false, true, true, true, true><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
-    default: k_unproject<true, true, true, true, true><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
+    case 7: k_unproject<true, true, true, true, true><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
+    case 8: k_unproject<false, false, true, true, false, true><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
+    case 9: k_unproject<true, false, true, true, false, true><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
+    case 10: k_unproject<false, true, true, true, false, true><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
+    case 11: k_unproject<true, true, true, true, false, true><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
+    case 12: k_unproject<false, false, true, true, true, true><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
+    case 13: k_unproject<true, false, true, true, true, true><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
+    case 14: k_unproject<false, true, true, true, true, true><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
+    default: k_unproject<true, true, true, true, true, true><<<grid, UP_THREADS, 0, ctx->stream>>>(p); break;
     }
     KP_LAUNCH_CHECK(ctx);
     // rows [B][S][sets][8]: one set without the ICP inputs, two with
@@ -466,6 +661,30 @@ size_t kp_unproject_engine_slots(int B, int S, int64_t P)
 {
     return (size_t)B * S * 2 * kp_blocks(P, UP_TILE) * (UP_THREADS / 32) * 8;
 }
+
+// frame engine: crop medians d_med [B][S] of the batch's depth (d_vbits [S][(P + 31) / 32]: finite table entries;
+// d_hist [B*S][kp_crop_median_hist_elems()] zero on entry and on return)
+int kp_crop_median_engine(kp_ctx *ctx, const uint16_t *d_depth, const uint32_t *d_vbits, int B, int S, int64_t P, uint32_t *d_hist,
+                          double *d_med)
+{
+    if (B <= 0 || S <= 0 || P <= 0) return KP_OK;
+    KP_PROFB(ctx, "crop_median", (double)B * S * P * (2.0 + 2.0) + 2.0 * (double)S * P / 8.0);
+    CropMedParams p{d_depth, d_vbits, S, P, (P + 31) / 32, d_hist, d_med};
+    // about four CTAs per SM over the batch, each streaming whole 16-byte groups of 8 pixels
+    int64_t gx = ((int64_t)ctx->sm_count * 4 + (int64_t)B * S - 1) / ((int64_t)B * S);
+    const int64_t gmax = kp_blocks((P + 7) / 8, CM_THREADS);
+    if (gx > gmax) gx = gmax;
+    if (gx < 1) gx = 1;
+    const dim3 grid((unsigned)gx, (unsigned)(B * S));
+    k_crop_hist<0><<<grid, CM_THREADS, 0, ctx->stream>>>(p);
+    KP_LAUNCH_CHECK(ctx);
+    k_crop_hist<1><<<grid, CM_THREADS, 0, ctx->stream>>>(p);
+    KP_LAUNCH_CHECK(ctx);
+    k_crop_median<<<B * S, CM_THREADS, 0, ctx->stream>>>(p);
+    KP_LAUNCH_CHECK(ctx);
+    return KP_OK;
+}
+size_t kp_crop_median_hist_elems() { return CM_BINS; }
 
 extern "C" {
 

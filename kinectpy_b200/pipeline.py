@@ -46,6 +46,12 @@ class PipelineConfig:
     normals_radius: float = 0.02
     seed: int = 1234
     n_streams: int = 4
+    # human crop of the fused cloud (preprocessing/data.py:165-178): segmentation non-black and z <= median + gate (mm)
+    do_crop: bool = False
+    crop_gate: float = 750.0
+    # fixed-N output per frame (the PointNet input): 0 = off, else N in 1..16384
+    resample_n: int = 0
+    resample_mode: int = _cabi.RESAMPLE_RANDOM
 
     def to_c(self) -> PipelineCfg:
         c = PipelineCfg()
@@ -57,6 +63,8 @@ class PipelineConfig:
         c.do_icp, c.icp_voxel, c.icp_max_corr, c.icp_max_iter = int(self.do_icp), self.icp_voxel, self.icp_max_corr, self.icp_max_iter
         c.normals_max_nn, c.normals_radius = self.normals_max_nn, self.normals_radius
         c.seed, c.n_streams = self.seed, self.n_streams
+        c.do_crop, c.crop_gate = int(self.do_crop), self.crop_gate
+        c.resample_n, c.resample_mode = self.resample_n, self.resample_mode
         return c
 
 
@@ -72,6 +80,8 @@ class FrameOutput:
     icp_rmse: np.ndarray
     icp_iters: np.ndarray
     points: Optional[np.ndarray] = None
+    fixed: Optional[np.ndarray] = None     # [N,3] fixed-N slot (want_fixed); zeros for a frame with status != 0
+    status: int = 0
 
 
 class FramePipeline:
@@ -107,23 +117,37 @@ class FramePipeline:
     def _raise(self, rc):
         raise KinectPyB200Error(rc, (self.lib.kp_pipeline_last_error(self.handle) or b"").decode())
 
-    def upload(self, depth: np.ndarray) -> _cabi.DeviceArray:
-        """depth uint16[F,S,P] -> device buffer for the HBM-resident leg."""
+    def upload(self, depth: np.ndarray, rgb: Optional[np.ndarray] = None):
+        """depth uint16[F,S,P] -> device buffer for the HBM-resident leg; with ``rgb`` (uint8[F,S,P,3] segmentation
+        images) -> (depth buffer, rgb buffer)."""
         d = self._ctx.to_device(depth, np.uint16)
+        if rgb is None:
+            self._ctx.sync()
+            return d
+        r = self._ctx.to_device(rgb, np.uint8)
         self._ctx.sync()
-        return d
+        return d, r
 
-    def run(self, depth, n_frames: Optional[int] = None, want_points: bool = False, out_stride: Optional[int] = None):
-        """depth: numpy uint16[F,S,P] (host: H2D inside the call) or a DeviceArray from ``upload``."""
+    def run(self, depth, rgb=None, n_frames: Optional[int] = None, want_points: bool = False, out_stride: Optional[int] = None,
+            want_fixed: bool = False, frame_ids=None, check: bool = True):
+        """depth: numpy uint16[F,S,P] (host: H2D inside the call) or a DeviceArray from ``upload``; rgb: the segmentation
+        images uint8[F,S,P,3] in the same memory space (required exactly when the pipeline crops).  ``want_fixed``: each
+        frame's fixed-N slot in ``FrameOutput.fixed`` (needs ``resample_n``); ``frame_ids`` int64[F] (default 0..F-1):
+        its sample stream.  ``check=False`` returns the outputs of a call whose frames carry a status instead of raising
+        (``FrameOutput.status``)."""
         S, P = self.cfg.n_sensors, self.cfg.pixels
         on_dev = isinstance(depth, _cabi.DeviceArray)
         if on_dev:
             F = int(depth.shape[0]) if n_frames is None else int(n_frames)
             ptr = depth.ptr
+            rptr = rgb.ptr if rgb is not None else None
         else:
             depth = np.ascontiguousarray(depth, dtype=np.uint16).reshape(-1, S, P)
             F = depth.shape[0] if n_frames is None else int(n_frames)
             ptr = depth.ctypes.data
+            if rgb is not None:
+                rgb = np.ascontiguousarray(rgb, dtype=np.uint8).reshape(-1, S, P, 3)
+            rptr = rgb.ctypes.data if rgb is not None else None
         res = (FrameResult * F)()
         out = None
         stride = 0
@@ -131,19 +155,33 @@ class FramePipeline:
             stride = int(out_stride or S * P)
             out = self._ctx.empty((F, stride, 3), np.float32)
             self._ctx.sync()
-        rc = self.lib.kp_pipeline_run(self.handle, ptr, 1 if on_dev else 0, F, res, out.ptr if out is not None else None, stride)
-        if rc != 0:
+        fixed = None
+        if want_fixed:
+            fixed = self._ctx.empty((F, max(int(self.cfg.resample_n), 1), 3), np.float32)
+            self._ctx.sync()
+        ids = None
+        if frame_ids is not None:
+            ids = np.ascontiguousarray(frame_ids, dtype=np.int64).reshape(-1)
+            if ids.size != F:
+                raise ValueError("frame_ids must hold one id per frame")
+        rc = self.lib.kp_pipeline_run_ex(self.handle, ptr, rptr, 1 if on_dev else 0, F, ids.ctypes.data if ids is not None else None,
+                                         res, out.ptr if out is not None else None, stride, fixed.ptr if fixed is not None else None)
+        if rc != 0 and (check or all(res[f].status == 0 for f in range(F))):      # (a call-level error has no frame status)
             self._raise(rc)
         outs: List[FrameOutput] = []
         host = out.to_host() if out is not None else None
+        hfixed = fixed.to_host() if fixed is not None else None
         for f in range(F):
             r = res[f]
             T = np.array([list(r.icp_T[i]) for i in range(max(S - 1, 0))], dtype=np.float64).reshape(-1, 4, 4)
             fo = FrameOutput(r.n_fused, r.n_voxel, r.n_sor, r.n_floor_inliers, r.n_out, T,
                              np.array(list(r.icp_fitness)[:S - 1]), np.array(list(r.icp_rmse)[:S - 1]),
                              np.array(list(r.icp_iters)[:S - 1]))
+            fo.status = int(r.status)
             if host is not None:
                 fo.points = host[f, :r.n_out].copy()
+            if hfixed is not None:
+                fo.fixed = hfixed[f].copy()
             outs.append(fo)
         self._last_raw = res
         return outs
@@ -173,8 +211,8 @@ class FramePipeline:
 
     def frame_counts(self) -> dict:
         """Device-side counts of the first frame of the last batch on slot 0 (diagnostics, byte accounting)."""
-        v = (C.c_int64 * 29)()
-        rc = self.lib.kp_pipeline_frame_counts(self.handle, v, 29)
+        v = (C.c_int64 * 35)()
+        rc = self.lib.kp_pipeline_frame_counts(self.handle, v, 35)
         if rc != 0:
             self._raise(rc)
         S = self.cfg.n_sensors
@@ -183,6 +221,7 @@ class FramePipeline:
         d["leftovers_l0"], d["leftovers_l1"] = [int(x) for x in v[8:11]], [int(x) for x in v[11:14]]
         d["leftovers_mid"] = [int(x) for x in v[26:29]]      # (the ICP target's search has no mid level: [2] is 0)
         d["nv_icp"], d["n_icp"] = [int(x) for x in v[14:14 + S]], [int(x) for x in v[20:20 + S]]
+        d["crop_median"] = [int(x) / 2.0 for x in v[29:29 + S]]     # (0.0 without the crop)
         return d
 
     def launch_count(self) -> int:

@@ -148,10 +148,9 @@ def _person(frame: int):
     ]
 
 
-def render_depth(mode: SensorMode, T_sensor: np.ndarray, frame: int, sensor: int, seed: int = 1234,
-                 noise: bool = True, table: np.ndarray | None = None) -> np.ndarray:
-    """One depth image uint16[H*W] in millimetres (Z along the optical axis; 0 = no return)."""
-    tab = xy_table(mode) if table is None else table
+def _raycast(T_sensor: np.ndarray, frame: int, tab: np.ndarray):
+    """First hit along every pixel's ray: distance t (metres along the unnormalised ray, so t * 1000 is Z in mm),
+    whether it is one of the person's ellipsoids, and the table's FOV mask."""
     ok = ~np.isnan(tab[:, 0])
     d_s = np.stack([tab[:, 0].astype(np.float64), tab[:, 1].astype(np.float64), np.ones(tab.shape[0])], axis=-1)
     d_s[~ok] = (0.0, 0.0, 1.0)
@@ -161,6 +160,7 @@ def render_depth(mode: SensorMode, T_sensor: np.ndarray, frame: int, sensor: int
     with np.errstate(divide="ignore", invalid="ignore"):
         tx = np.where(d > 0, (ROOM_HI - o) / d, np.where(d < 0, (ROOM_LO - o) / d, np.inf))
     t = tx.min(axis=1)
+    person = np.zeros(tab.shape[0], dtype=bool)
     for c, r in _person(frame):
         c = np.asarray(c)
         r = np.asarray(r)
@@ -172,7 +172,17 @@ def render_depth(mode: SensorMode, T_sensor: np.ndarray, frame: int, sensor: int
         disc = qb * qb - 4.0 * qa * qc
         hit = disc >= 0
         te = np.where(hit, (-qb - np.sqrt(np.where(hit, disc, 0.0))) / (2.0 * qa), np.inf)
-        t = np.where((te > 0) & (te < t), te, t)
+        closer = (te > 0) & (te < t)
+        t = np.where(closer, te, t)
+        person |= closer
+    return t, person & ok, ok
+
+
+def render_depth(mode: SensorMode, T_sensor: np.ndarray, frame: int, sensor: int, seed: int = 1234,
+                 noise: bool = True, table: np.ndarray | None = None) -> np.ndarray:
+    """One depth image uint16[H*W] in millimetres (Z along the optical axis; 0 = no return)."""
+    tab = xy_table(mode) if table is None else table
+    t, _, ok = _raycast(T_sensor, frame, tab)
     z_mm = t * 1000.0
     pix = np.arange(tab.shape[0], dtype=np.uint64)
     key_a = np.uint64(frame) * np.uint64(16) + np.uint64(sensor)
@@ -191,6 +201,41 @@ def render_depth(mode: SensorMode, T_sensor: np.ndarray, frame: int, sensor: int
     z = np.rint(z_mm)
     z = np.where(ok & ~drop & (z > 0) & (z < 65535), z, 0.0)
     return z.astype(np.uint16)
+
+
+FAR_WALL_M = 4.0     # a wall pixel at least this far away can be part of the false-positive patch
+
+
+def render_segmentation(mode: SensorMode, T_sensor: np.ndarray, frame: int, sensor: int, seed: int = 1234,
+                        table: np.ndarray | None = None) -> np.ndarray:
+    """The segmentation image that goes with ``render_depth``: uint8[H*W, 3], non-black where a pixel's first hit is
+    the person, black elsewhere -- the ``_seg`` image ``DataProcessor`` crops with (preprocessing/data.py:165-178).
+    Two seeded defects exercise each rule of the crop: about 3 % of the person pixels have one or two zero channels
+    (a pixel is person only when all three channels are non-zero), and a patch of the image that sees a far wall
+    (more than FAR_WALL_M away) is marked as person (the median gate has to remove it)."""
+    tab = xy_table(mode) if table is None else table
+    t, person, ok = _raycast(T_sensor, frame, tab)
+    n = tab.shape[0]
+    pix = np.arange(n, dtype=np.uint64)
+    key_a = np.uint64(frame) * np.uint64(16) + np.uint64(sensor) + np.uint64(1 << 40)
+    u = [_uniform(seed, key_a, pix * np.uint64(4) + np.uint64(k)) for k in range(4)]
+    rgb = np.zeros((n, 3), dtype=np.uint8)
+    shade = (np.stack(u[:3], axis=1) * 200.0 + 40.0).astype(np.uint8)      # 40..239 in every channel
+    rgb[person] = shade[person]
+    # defect 1: one or two zero channels on a few person pixels
+    bad = person & (u[3] < 0.03)
+    zero_a = (u[3] * 1000.0).astype(np.int64) % 3
+    rows = np.flatnonzero(bad)
+    rgb[rows, zero_a[rows]] = 0
+    two = rows[(rows % 2) == 0]
+    rgb[two, (zero_a[two] + 1) % 3] = 0
+    # defect 2: a false-positive patch on a far wall, in a fixed window of the image (an eighth of its width and height,
+    # right of and above the centre)
+    v, c = np.divmod(np.arange(n), mode.width)
+    window = (c >= (5 * mode.width) // 8) & (c < (6 * mode.width) // 8) & (v >= (3 * mode.height) // 8) & (v < (4 * mode.height) // 8)
+    patch = ok & ~person & (t > FAR_WALL_M) & window
+    rgb[patch] = (200, 180, 160)
+    return rgb
 
 
 def render_sequence(mode: SensorMode, n_frames: int, n_sensors: int = 3, seed: int = 1234, first_frame: int = 0,
