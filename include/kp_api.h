@@ -288,7 +288,7 @@ KP_EXPORT int kp_resample_batch(kp_ctx *ctx, const float *d_xyz, const int64_t *
 
 /* ------------------------------------------------ whole-frame driver --- */
 /* Batched, device-driven driver for BASELINE config C4: per frame unproject ->
- * transform -> fuse -> voxel -> SOR -> floor removal (band + RANSAC + merge +
+ * transform -> fuse -> voxel -> SOR [-> radius outlier removal] -> floor removal (band + RANSAC + merge +
  * SOR) -> ICP refinement of every sub extrinsic (the per-frame body of
  * preprocessing/data.py:35-69 followed by floor_removal.py:57-73 and
  * preprocessing/registration.py:65-86).  Frames are processed in batches of B
@@ -316,6 +316,12 @@ typedef struct {
     int32_t do_crop;        double crop_gate;
     /* fixed-N output (kp_resample_batch on each frame's final cloud, stream = frame id): 0 = off, else 1..16384 */
     int32_t resample_n;     int32_t resample_mode;   /* KP_RESAMPLE_RANDOM / KP_RESAMPLE_PREFIX */
+    /* radius outlier removal (remove_radius_outlier) of the fused cloud after its SOR (after the voxel downsample when
+     * sor_k = 0), before floor removal: a point is kept iff more than ror_nb_points points (itself included) lie at
+     * d^2 < ror_radius^2, d^2 in double on the float32 coordinates; survivors keep their order.  Its output replaces the
+     * SOR output downstream; n_sor still counts the SOR survivors.  ror_nb_points = 0: off; else ror_radius > 0, in the
+     * cloud's unit (it follows `scale`, like voxel_size).  The ICP inputs are not filtered. */
+    int32_t ror_nb_points;  double ror_radius;
 } kp_pipeline_cfg;
 typedef struct {
     int64_t n_fused, n_voxel, n_sor, n_floor_inliers, n_out;
@@ -358,7 +364,8 @@ KP_EXPORT int kp_pipeline_frames_in_flight(kp_pipeline *p, int *batch, int *slot
  * n_fused, n_voxel, n_sor, n_band, n_band_kept, n_merged, n_floor_sor, n_out, level-0 leftovers of the three
  * neighbour searches [3], level-1 leftovers [3], valid rows of the ICP inputs [6], their voxel counts [6];
  * with n >= 29 also the mid-level leftovers of the three searches [3] (entries 26-28); with n >= 35 also twice
- * the crop median of each sensor [6] (entries 29-34; 0 without the crop) */
+ * the crop median of each sensor [6] (entries 29-34; 0 without the crop); with n >= 36 also the survivors of the
+ * radius outlier removal (entry 35; 0 when it is off) */
 KP_EXPORT int kp_pipeline_frame_counts(kp_pipeline *p, int64_t *h_counts, int n);
 KP_EXPORT int kp_pipeline_profile(kp_pipeline *p, int enable_or_read, int max_entries,
                                   const char **h_names, double *h_ms, int64_t *h_calls, double *h_bytes, int *h_n);

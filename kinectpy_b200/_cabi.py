@@ -41,6 +41,7 @@ class PipelineCfg(C.Structure):
         ("normals_max_nn", C.c_int32), ("normals_radius", C.c_double),
         ("seed", C.c_uint64), ("n_streams", C.c_int32),
         ("do_crop", C.c_int32), ("crop_gate", C.c_double), ("resample_n", C.c_int32), ("resample_mode", C.c_int32),
+        ("ror_nb_points", C.c_int32), ("ror_radius", C.c_double),
     ]
 
 

@@ -45,7 +45,7 @@ struct EngCloud {
 // per-frame state produced and consumed on the device
 struct EngDyn {
     int32_t n_fused, n_voxel, n_sor, n_lo, n_rest, n_merged, n_fsor, n_out;
-    int32_t status, floor_skip, ymax_enc, pad0;
+    int32_t status, floor_skip, ymax_enc, n_ror;    // n_ror: survivors of the radius outlier removal (0 when it is off)
     int32_t nocc[4];                    // occupied cells of grid g[0..3]
     int32_t cnt_l0[3], cnt_l1[3];       // level-0 / level-1 leftover lists of the three neighbour searches
     int32_t cnt_lm[3], nocc_m[2], pad3; // leftovers of the mid level; occupied cells of the mid grids
@@ -689,6 +689,58 @@ __global__ void __launch_bounds__(256) k_e_sor_mask(const __grid_constant__ SorM
         keep[i] = (m > 0 && m < thr) ? 1 : 0;
     }
 }
+// remove_radius_outlier (SURVEY A.4): keep[row] = #{j : d2(i, j) < r2} > nb, the point itself included.  One thread per
+// query in the grid's cell-sorted order, so that neighbouring threads read the same candidate cells (L1).  The cell is
+// >= the radius: every neighbour lies in the 27-cell block, whose 9 z-columns are one run each.  fp32 chooses and double
+// decides: a candidate whose fp32 d2 lies within the 1e-6 margins of r2 is decided by kp_d2 (DESIGN §3).  Counting stops
+// at nb + 1, so a dense surface costs a few candidates per query whatever nb is.
+struct RorArgs {
+    const KpGridDev *g; int64_t g_stride;      // bytes between the segments' grids
+    DCnt n;
+    int nb; double r2; float r2_lo, r2_hi;     // r2_lo / r2_hi: r2 (1 -+ 1e-6) rounded down / up to fp32
+    uint8_t *keep; int64_t keep_stride;
+};
+__global__ void __launch_bounds__(128, 8) k_e_ror_count(const __grid_constant__ RorArgs a)
+{
+    const int seg = blockIdx.y;
+    const int n = a.n.at(seg);
+    const KpGridDev g = *reinterpret_cast<const KpGridDev *>(reinterpret_cast<const char *>(a.g) + seg * a.g_stride);
+    uint8_t *keep = a.keep + seg * a.keep_stride;
+    for (int w = blockIdx.x * blockDim.x + threadIdx.x; w < n; w += gridDim.x * blockDim.x) {
+        const float4 me = __ldg(g.pts + w);
+        int cnt = 0;
+        if (!isnan(me.x)) {
+            const int cx = min(max(kp_cell_coord(g, (double)me.x, 0), 0), g.dim[0] - 1);
+            const int cy = min(max(kp_cell_coord(g, (double)me.y, 1), 0), g.dim[1] - 1);
+            const int cz = min(max(kp_cell_coord(g, (double)me.z, 2), 0), g.dim[2] - 1);
+            int2 rng[9];
+#pragma unroll
+            for (int ci = 0; ci < 9; ++ci) {
+                constexpr int order[9] = {4, 1, 3, 5, 7, 0, 2, 6, 8};     // own column first: the likeliest to end the count
+                rng[ci] = kp_row_range(g, cx + order[ci] / 3 - 1, cy + order[ci] % 3 - 1, cz);
+            }
+#pragma unroll
+            for (int ci = 0; ci < 9; ++ci) {
+                // four candidates per trip: their loads are in flight together
+                for (int t = rng[ci].x; t < rng[ci].y && cnt <= a.nb; t += 4) {
+                    float4 c[4];
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) c[u] = __ldg(g.pts + min(t + u, rng[ci].y - 1));
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        if (t + u >= rng[ci].y) break;
+                        const float d = hq_d32(me.x, me.y, me.z, c[u]);
+                        if (d < a.r2_lo) ++cnt;
+                        else if (!(d > a.r2_hi) && kp_d2((double)me.x, (double)me.y, (double)me.z, (double)c[u].x, (double)c[u].y, (double)c[u].z) < a.r2)
+                            ++cnt;
+                    }
+                }
+            }
+        }
+        keep[__float_as_int(me.w)] = cnt > a.nb ? 1 : 0;
+    }
+}
+
 struct BandArgs {
     const float *xyz; int64_t stride; DCnt n; EngDyn *dyn; int axis; double band; int ransac_n;
     uint8_t *lower; int64_t mask_stride;
@@ -971,12 +1023,13 @@ __global__ void __launch_bounds__(256) k_e_append_rows(const __grid_constant__ A
             a.aux_dst[seg * a.stride + off + e] = a.aux_src[seg * a.stride + e];
     if (blockIdx.x == 0 && threadIdx.x == 0) a.total.at(seg) = off + n;
 }
-// n_up = n_sor - n_lo is not stored anywhere: a tiny kernel derives the per-frame scalars between stages
-struct DeriveArgs { EngDyn *dyn; int32_t *n_up; int do_floor, do_fsor; };
+// n_up = n_in - n_lo (n_in: the floor stage's input) is not stored anywhere: a tiny kernel derives the per-frame scalars
+// between stages
+struct DeriveArgs { EngDyn *dyn; DCnt n_in; int32_t *n_up; int do_floor, do_fsor; };
 __global__ void k_e_derive_up(const __grid_constant__ DeriveArgs a, int B)
 {
     const int f = blockIdx.x * blockDim.x + threadIdx.x;
-    if (f < B) a.n_up[f] = a.dyn[f].n_sor - a.dyn[f].n_lo;
+    if (f < B) a.n_up[f] = a.n_in.at(f) - a.dyn[f].n_lo;
 }
 
 // points left to the grid level 0: none when the cloud's voxel-brick index was built
@@ -992,14 +1045,15 @@ __global__ void k_e_nold(const __grid_constant__ NoldArgs a, int nseg)
 // final cloud + result record of every frame
 struct FinishArgs {
     EngDyn *dyn; kp_frame_result *res; int S;
-    const float *sor_out, *merged, *fsor_out; int64_t stride;       // candidates for the final cloud
+    const float *filt_out, *merged, *fsor_out; int64_t stride;      // candidates for the final cloud
+    DCnt n_filt;                                                    // rows of filt_out (the voxel + SOR [+ ROR] output)
     int do_floor, do_fsor;
     float *out; int64_t out_stride;                                 // rows; NULL -> no copy
 };
 __device__ __forceinline__ void finish_pick(const FinishArgs &a, int f, const float *&src, int &n)
 {
     const EngDyn &d = a.dyn[f];
-    if (!a.do_floor || d.floor_skip) { src = a.sor_out + 3 * f * a.stride; n = d.n_sor; }
+    if (!a.do_floor || d.floor_skip) { src = a.filt_out + 3 * f * a.stride; n = a.n_filt.at(f); }
     else if (!a.do_fsor) { src = a.merged + 3 * f * a.stride; n = d.n_merged; }
     else { src = a.fsor_out + 3 * f * a.stride; n = d.n_fsor; }
 }
@@ -1375,8 +1429,48 @@ int stage_sor(kp_pipeline *pl, EngSlot &s, int use, const float *in, const uint3
     return kp_b_compact_rows(L, s.scan, n, s.mask, NPs, 0, in, out, NPs, n_out, vout ? vin : nullptr, vout);
 }
 
+// the fused branch's filter output, which the floor stage, k_e_finish and the copy-out read: voxel (A) -> SOR (Bb) -> ROR
+// (into whichever of A / Bb is not its input)
+struct FilterOut { float *xyz; uint32_t *vijk; DCnt n; };
+FilterOut filter_output(const kp_pipeline *pl, EngSlot &s)
+{
+    const kp_pipeline_cfg &c = pl->cfg;
+    const bool in_b = (c.sor_k > 0) != (c.ror_nb_points > 0);
+    return FilterOut{in_b ? s.Bb : s.A, in_b ? s.vB : s.vA, c.ror_nb_points > 0 ? DYN_CNT(s, n_ror) : DYN_CNT(s, n_sor)};
+}
+
+// fp32 bounds of a double: the largest float <= v, the smallest float >= v
+inline float f32_down(double v) { const float f = (float)v; return (double)f > v ? nextafterf(f, -INFINITY) : f; }
+inline float f32_up(double v) { const float f = (float)v; return (double)f < v ? nextafterf(f, INFINITY) : f; }
+
+// ---- stage: remove_radius_outlier of the batch's clouds `in` (n rows each, voxel coordinates vin) -> `out`, n_ror
+int stage_ror(kp_pipeline *pl, EngSlot &s, const float *in, const uint32_t *vin, DCnt n, float *out, uint32_t *vout)
+{
+    kp_ctx *ctx = s.ctx;
+    const kp_pipeline_cfg &c = pl->cfg;
+    const int B = pl->B;
+    const int64_t NPs = pl->NPr;
+    KP_PROF(ctx, "ror");
+    // the SOR's level-0 grid arrays (free once it is done); the cell is the radius with kp_radius_mask's margin.  k_eg_setup
+    // may double it to fit cap_cells: any cell >= the radius keeps every neighbour inside the 27-cell block.
+    GridArgs g = main_grid_args(pl, s, 0, in, n, 0.0);
+    g.cell = c.ror_radius * (1.0 + 1e-6);
+    KP_TRY(stage_grid(pl, ctx, g, B, NPs, s.scan, dout(s.sink, 4)));
+    {
+        KP_PROFB(ctx, "ror_count", 0.0);
+        const double r2 = c.ror_radius * c.ror_radius;
+        RorArgs a{&s.dyn->g[0], sizeof(EngDyn), n, c.ror_nb_points, r2, f32_down(r2 * (1.0 - 1e-6)), f32_up(r2 * (1.0 + 1e-6)), s.mask, NPs};
+        int64_t gx = (NPs + 127) / 128;
+        if (gx > ctas_for(pl, 8)) gx = ctas_for(pl, 8);
+        k_e_ror_count<<<dim3((unsigned)gx, (unsigned)B), 128, 0, ctx->stream>>>(a);
+        KP_LAUNCH_CHECK(ctx);
+    }
+    BLaunch L{ctx, B, NPs, ctas_for(pl, 4)};
+    return kp_b_compact_rows(L, s.scan, n, s.mask, NPs, 0, in, out, NPs, DYN_OUT(s, n_ror), vout ? vin : nullptr, vout);
+}
+
 // ---- stage: floor removal (band split, RANSAC plane on the band, band outliers + upper part)
-int stage_floor(kp_pipeline *pl, EngSlot &s, const float *in, const uint32_t *vin)
+int stage_floor(kp_pipeline *pl, EngSlot &s, const float *in, const uint32_t *vin, DCnt n_in)
 {
     kp_ctx *ctx = s.ctx;
     const kp_pipeline_cfg &c = pl->cfg;
@@ -1386,16 +1480,16 @@ int stage_floor(kp_pipeline *pl, EngSlot &s, const float *in, const uint32_t *vi
     BLaunch L{ctx, B, NPs, ctas_for(pl, 4)};
     {
         KP_PROFB(ctx, "band_mask", 0.0);
-        BandArgs a{in, NPs, DYN_CNT(s, n_sor), s.dyn, 1, c.floor_band, c.ransac_n, s.mask, NPs};
+        BandArgs a{in, NPs, n_in, s.dyn, 1, c.floor_band, c.ransac_n, s.mask, NPs};
         k_e_axis_max<<<grid, 256, 0, ctx->stream>>>(a);
         KP_LAUNCH_CHECK(ctx);
         k_e_band_mask<<<grid, 256, 0, ctx->stream>>>(a);
         KP_LAUNCH_CHECK(ctx);
     }
     // lower band -> C, upper part -> D
-    KP_TRY(kp_b_partition_rows(L, s.scan, DYN_CNT(s, n_sor), s.mask, NPs, in, s.C, s.D, NPs, DYN_OUT(s, n_lo), vin, s.vC, s.vD));
+    KP_TRY(kp_b_partition_rows(L, s.scan, n_in, s.mask, NPs, in, s.C, s.D, NPs, DYN_OUT(s, n_lo), vin, s.vC, s.vD));
     {
-        DeriveArgs d{s.dyn, s.n_up, c.do_floor, c.floor_sor_k > 0};
+        DeriveArgs d{s.dyn, n_in, s.n_up, c.do_floor, c.floor_sor_k > 0};
         k_e_derive_up<<<kp_blocks(B, 64), 64, 0, ctx->stream>>>(d, B);
         KP_LAUNCH_CHECK(ctx);
     }
@@ -1702,9 +1796,12 @@ int enqueue_core(kp_pipeline *pl, EngSlot &s, bool fork)
         k_e_copy_cnt<<<kp_blocks(B, 64), 64, 0, ctx->stream>>>(DYN_CNT(s, n_voxel), DYN_OUT(s, n_sor), B);
         KP_LAUNCH_CHECK(ctx);
     }
+    // ---- radius outlier removal (optional): its output replaces the SOR output downstream
+    const FilterOut fo = filter_output(pl, s);
+    if (c.ror_nb_points > 0) KP_TRY(stage_ror(pl, s, sor_out, v_sor_out, DYN_CNT(s, n_sor), fo.xyz, fo.vijk));
     // ---- floor removal + SOR
     if (c.do_floor) {
-        KP_TRY(stage_floor(pl, s, sor_out, v_sor_out));
+        KP_TRY(stage_floor(pl, s, fo.xyz, fo.vijk, fo.n));
         if (c.floor_sor_k > 0)
             KP_TRY(stage_sor(pl, s, 1, s.E, s.vE, DYN_CNT(s, n_merged), c.floor_sor_k, c.floor_sor_ratio, s.Fin, nullptr, DYN_OUT(s, n_fsor)));
     }
@@ -1714,7 +1811,7 @@ int enqueue_core(kp_pipeline *pl, EngSlot &s, bool fork)
         KP_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, s.ev_join, 0));
     }
     {
-        FinishArgs fa{s.dyn, s.d_res, S, sor_out, s.E, s.Fin, NPr, c.do_floor, c.floor_sor_k > 0, nullptr, 0};
+        FinishArgs fa{s.dyn, s.d_res, S, fo.xyz, s.E, s.Fin, NPr, fo.n, c.do_floor, c.floor_sor_k > 0, nullptr, 0};
         k_e_finish<<<kp_blocks(B, 32), 32, 0, ctx->stream>>>(fa, B);
         KP_LAUNCH_CHECK(ctx);
     }
@@ -1799,9 +1896,10 @@ int run_impl(kp_pipeline *p, const uint16_t *depth, const uint8_t *rgb, int dept
             PL_CUDA(p, cudaGraphLaunch(s.graph, ctx->stream));
             p->launches += s.graph_nodes;
         }
+        const FilterOut fo = filter_output(p, s);
         if (out_xyz) {
-            FinishArgs fa{s.dyn, s.d_res, S, c.sor_k > 0 ? s.Bb : s.A, s.E, s.Fin, p->NPr, c.do_floor, c.floor_sor_k > 0,
-                          out_xyz + 3 * f0 * out_stride, out_stride};
+            FinishArgs fa{s.dyn, s.d_res, S, fo.xyz, s.E, s.Fin, p->NPr, fo.n, c.do_floor, c.floor_sor_k > 0, out_xyz + 3 * f0 * out_stride,
+                          out_stride};
             k_e_copy_out<<<dim3((unsigned)p->sm_count, (unsigned)nf), 256, 0, ctx->stream>>>(fa);
             ctx->launches++;
             k_e_check_stride<<<kp_blocks(nf, 32), 32, 0, ctx->stream>>>(s.dyn, s.d_res, nf, out_stride);
@@ -1812,7 +1910,7 @@ int run_impl(kp_pipeline *p, const uint16_t *depth, const uint8_t *rgb, int dept
             // get their status in the result record (written by the graph's k_e_finish just before)
             int64_t ids[16];
             for (int b = 0; b < nf; ++b) ids[b] = h_frame_ids ? h_frame_ids[f0 + b] : f0 + b;
-            FinishArgs fa{s.dyn, s.d_res, S, c.sor_k > 0 ? s.Bb : s.A, s.E, s.Fin, p->NPr, c.do_floor, c.floor_sor_k > 0, nullptr, 0};
+            FinishArgs fa{s.dyn, s.d_res, S, fo.xyz, s.E, s.Fin, p->NPr, fo.n, c.do_floor, c.floor_sor_k > 0, nullptr, 0};
             k_e_final_src<<<kp_blocks(nf, 32), 32, 0, ctx->stream>>>(fa, nf, s.fin_src);
             ctx->launches++;
             rc = kp_resample_engine(ctx, s.fin_src, p->NPr, &s.dyn->n_out, (int64_t)(sizeof(EngDyn) / 4), nf, c.resample_n, c.resample_mode,
@@ -1864,6 +1962,8 @@ int kp_pipeline_create(int device, const kp_pipeline_cfg *cfg, const float *h_xy
         return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: resample_n must be 0 (off) or 1..16384 (got %d)", cfg->resample_n);
     if (cfg->resample_n != 0 && cfg->resample_mode != KP_RESAMPLE_RANDOM && cfg->resample_mode != KP_RESAMPLE_PREFIX)
         return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: resample_mode must be KP_RESAMPLE_RANDOM or KP_RESAMPLE_PREFIX");
+    if (cfg->ror_nb_points < 0 || (cfg->ror_nb_points > 0 && !(cfg->ror_radius > 0.0)))
+        return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: ror_nb_points must be >= 0 (0 = off), and ror_radius > 0 when it is on");
     *out = nullptr;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
@@ -2022,7 +2122,8 @@ int kp_pipeline_frame_counts(kp_pipeline *p, int64_t *h_counts, int n)
 {
     // the device-side counts of the first frame of batch slot 0 after its last batch (diagnostics / byte accounting):
     // n_fused, n_voxel, n_sor, n_lo, n_rest, n_merged, n_fsor, n_out, level-0 leftovers [3], level-1 leftovers [3],
-    // valid rows of the S ICP inputs [6], their voxel counts [6]; with n >= 29 also mid-level leftovers [3]
+    // valid rows of the S ICP inputs [6], their voxel counts [6]; with n >= 29 also mid-level leftovers [3], with n >= 35
+    // twice the crop medians [6], with n >= 36 the radius outlier removal's survivors
     if (!p || !h_counts || n < 26) return KP_E_ARG;
     cudaSetDevice(p->device);
     EngSlot &s = p->slots[0];
@@ -2043,6 +2144,7 @@ int kp_pipeline_frame_counts(kp_pipeline *p, int64_t *h_counts, int n)
         if (p->cfg.do_crop && cudaMemcpy(med, s.crop_med, sizeof(double) * p->cfg.S, cudaMemcpyDeviceToHost) != cudaSuccess) return KP_E_CUDA;
         for (int i = 0; i < 6; ++i) h_counts[29 + i] = i < p->cfg.S ? (int64_t)(2.0 * med[i]) : 0;
     }
+    if (n >= 36) h_counts[35] = p->cfg.ror_nb_points > 0 ? d.n_ror : 0;
     return KP_OK;
 }
 

@@ -709,11 +709,6 @@ constexpr int HQ_KMAX = 64;
 constexpr float HQ_MAGIC = 8388608.0f;          // 2^23: adding it leaves round(x) in the low mantissa bits
 constexpr int HQ_MAGIC_BITS = 0x4B000000;
 
-__device__ __forceinline__ float hq_d32(float qx, float qy, float qz, const float4 &c)
-{
-    const float dx = qx - c.x, dy = qy - c.y, dz = qz - c.z;
-    return __fmaf_rn(dz, dz, __fmaf_rn(dy, dy, dx * dx));
-}
 __device__ __forceinline__ int hq_bin(float d, float scale)
 {
     return __float_as_int(__fmaf_rn(d, scale, HQ_MAGIC)) - HQ_MAGIC_BITS;   // round(d * scale), monotone in d

@@ -51,6 +51,13 @@ __device__ __forceinline__ int2 kp_map_range(const KpGridDev &g, int cx, int cy,
     first = cnt ? first : 0;
     return make_int2(__ldg(g.run_start + first), __ldg(g.run_start + first + cnt));
 }
+// fp32 squared distance of the neighbour kernels' candidate passes (relative error < 6e-7, DESIGN §3): it chooses which
+// candidates the double expression kp_d2 has to decide, it never decides one itself
+__device__ __forceinline__ float hq_d32(float qx, float qy, float qz, const float4 &c)
+{
+    const float dx = qx - c.x, dy = qy - c.y, dz = qz - c.z;
+    return __fmaf_rn(dz, dz, __fmaf_rn(dy, dy, dx * dx));
+}
 // resolve a probe sequence that starts at slot h with the already loaded slot s
 __device__ __forceinline__ int2 kp_slot_resolve(const KpGridDev &g, uint64_t key, uint32_t h, uint4 s)
 {

@@ -52,6 +52,10 @@ class PipelineConfig:
     # fixed-N output per frame (the PointNet input): 0 = off, else N in 1..16384
     resample_n: int = 0
     resample_mode: int = _cabi.RESAMPLE_RANDOM
+    # radius outlier removal after the SOR (remove_radius_outlier): 0 = off, else keep points with more than
+    # ror_nb_points points (themselves included) closer than ror_radius (in the cloud's unit)
+    ror_nb_points: int = 0
+    ror_radius: float = 0.0
 
     def to_c(self) -> PipelineCfg:
         c = PipelineCfg()
@@ -65,6 +69,7 @@ class PipelineConfig:
         c.seed, c.n_streams = self.seed, self.n_streams
         c.do_crop, c.crop_gate = int(self.do_crop), self.crop_gate
         c.resample_n, c.resample_mode = self.resample_n, self.resample_mode
+        c.ror_nb_points, c.ror_radius = self.ror_nb_points, self.ror_radius
         return c
 
 
@@ -211,8 +216,8 @@ class FramePipeline:
 
     def frame_counts(self) -> dict:
         """Device-side counts of the first frame of the last batch on slot 0 (diagnostics, byte accounting)."""
-        v = (C.c_int64 * 35)()
-        rc = self.lib.kp_pipeline_frame_counts(self.handle, v, 35)
+        v = (C.c_int64 * 36)()
+        rc = self.lib.kp_pipeline_frame_counts(self.handle, v, 36)
         if rc != 0:
             self._raise(rc)
         S = self.cfg.n_sensors
@@ -222,6 +227,7 @@ class FramePipeline:
         d["leftovers_mid"] = [int(x) for x in v[26:29]]      # (the ICP target's search has no mid level: [2] is 0)
         d["nv_icp"], d["n_icp"] = [int(x) for x in v[14:14 + S]], [int(x) for x in v[20:20 + S]]
         d["crop_median"] = [int(x) / 2.0 for x in v[29:29 + S]]     # (0.0 without the crop)
+        d["n_ror"] = int(v[35])                                      # (0 without the radius outlier removal)
         return d
 
     def launch_count(self) -> int:
