@@ -322,13 +322,30 @@ typedef struct {
      * SOR output downstream; n_sor still counts the SOR survivors.  ror_nb_points = 0: off; else ror_radius > 0, in the
      * cloud's unit (it follows `scale`, like voxel_size).  The ICP inputs are not filtered. */
     int32_t ror_nb_points;  double ror_radius;
+    /* floor stage (do_floor = 1), reading the filter output (the SOR output, or the ROR output when that stage is on):
+     *   KP_FLOOR_RANSAC (0, the default): band + segment_plane + merge + floor SOR, as above.  The frame's floor plane
+     *     is reported in kp_frame_result.floor_plane.
+     *   KP_FLOOR_PLANE (1): pcd_above_plane with floor_plane = (a, b, c, d): the rows with ((a*x + b*y) + c*z) + d < 0,
+     *     strict, in double on the float32 coordinates, no FMA, keep their order, then the floor SOR runs on them
+     *     (floor_sor_k = 0: off).  No band, RANSAC or floor-skip rule: every filter output is cut, an empty one too.
+     *     n_floor_inliers = filter-output rows - rows kept; kp_pipeline_frame_counts reports n_band = n_band_kept = 0
+     *     and n_merged = rows kept.  A zero normal keeps every row iff d < 0.  The plane is in the cloud's unit (d
+     *     follows `scale`, like floor_band) and is applied with the caller's sign.  Every coefficient must be finite.
+     * Create refuses any other floor_mode, and a non-finite coefficient in plane mode (KP_E_ARG). */
+    int32_t floor_mode;     double floor_plane[4];
 } kp_pipeline_cfg;
+enum { KP_FLOOR_RANSAC = 0, KP_FLOOR_PLANE = 1 };
 typedef struct {
     int64_t n_fused, n_voxel, n_sor, n_floor_inliers, n_out;
     double icp_T[5][16];    /* refined T_master<-sub_i, i = 1..S-1 */
     double icp_fitness[5], icp_rmse[5];
     int32_t icp_iters[5];
     int32_t status;
+    /* the frame's floor plane (a, b, c, d).  RANSAC mode: the plane segment_plane returns, i.e. the covariance refit on
+     * the winning hypothesis's inliers (the points removed), the hypothesis itself when that fit is degenerate, 0 x 4
+     * when no hypothesis is valid; NaN x 4 when the frame has no floor plane (floor stage skipped, band smaller than
+     * ransac_n, empty frame).  Plane mode: cfg.floor_plane, bit for bit.  NaN x 4 when do_floor = 0. */
+    double floor_plane[4];
 } kp_frame_result;
 KP_EXPORT int kp_pipeline_create(int device, const kp_pipeline_cfg *cfg, const float *h_xytab,
                                  const double *h_T, kp_pipeline **out);

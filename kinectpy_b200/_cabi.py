@@ -20,6 +20,7 @@ KP_OK, KP_E_ARG, KP_E_CUDA, KP_E_RANGE, KP_E_NOMEM, KP_E_NODEVICE = 0, -1, -2, -
 UNPROJECT_INT16 = 1
 UNPROJECT_DROP_ANY_ZERO = 2
 RESAMPLE_RANDOM, RESAMPLE_PREFIX = 0, 1
+FLOOR_RANSAC, FLOOR_PLANE = 0, 1
 
 
 class KinectPyB200Error(RuntimeError):
@@ -42,6 +43,7 @@ class PipelineCfg(C.Structure):
         ("seed", C.c_uint64), ("n_streams", C.c_int32),
         ("do_crop", C.c_int32), ("crop_gate", C.c_double), ("resample_n", C.c_int32), ("resample_mode", C.c_int32),
         ("ror_nb_points", C.c_int32), ("ror_radius", C.c_double),
+        ("floor_mode", C.c_int32), ("floor_plane", C.c_double * 4),
     ]
 
 
@@ -51,6 +53,7 @@ class FrameResult(C.Structure):
         ("n_out", C.c_int64),
         ("icp_T", (C.c_double * 16) * 5), ("icp_fitness", C.c_double * 5), ("icp_rmse", C.c_double * 5),
         ("icp_iters", C.c_int32 * 5), ("status", C.c_int32),
+        ("floor_plane", C.c_double * 4),
     ]
 
 

@@ -237,6 +237,24 @@ __device__ __forceinline__ double kp_affine(double a, double b, double c, double
 {
     return __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(a, x), __dmul_rn(b, y)), __dmul_rn(c, z)), d);
 }
+// covariance-determinant plane fit on pre-reduced centred moments m = (xx, xy, xz, yy, yz, zz) around (cx, cy, cz):
+// Open3D's segment_plane refit.  false: degenerate (zero or NaN normal).  Shared by kp_ransac_device (host) and the
+// frame engine's batched refit (device); the build has no FMA contraction on either side.
+__host__ __device__ __forceinline__ bool cov_fit_from_moments(const double *m, double cx, double cy, double cz, double *pl)
+{
+    const double xx = m[0], xy = m[1], xz = m[2], yy = m[3], yz = m[4], zz = m[5];
+    const double dx = yy * zz - yz * yz, dy = xx * zz - xz * xz, dz = xx * yy - xy * xy;
+    double a, b, c;
+    if (dx >= dy && dx >= dz) { a = dx; b = xz * yz - xy * zz; c = xy * yz - xz * yy; }
+    else if (dy >= dx && dy >= dz) { a = xz * yz - xy * zz; b = dy; c = xy * xz - yz * xx; }
+    else { a = xy * yz - xz * yy; b = xy * xz - yz * xx; c = dz; }
+    const double nn = sqrt((a * a + b * b) + c * c);
+    if (nn == 0.0 || nn != nn) return false;
+    a /= nn; b /= nn; c /= nn;
+    pl[0] = a; pl[1] = b; pl[2] = c;
+    pl[3] = -((a * cx + b * cy) + c * cz);
+    return true;
+}
 __device__ __forceinline__ double kp_dot3(double a, double b, double c, double x, double y, double z)
 {
     return __dadd_rn(__dadd_rn(__dmul_rn(a, x), __dmul_rn(b, y)), __dmul_rn(c, z));

@@ -61,6 +61,8 @@ struct EngDyn {
     double cand_sq[ENG_MAX_CAND];
     double icp_T[5][16], icp_fit[5], icp_rmse[5];
     int32_t icp_iters[5], pad1;
+    double refit_c[4];                  // floor refit: centroid of the winning hypothesis's inliers, their count
+    double floor_plane[4];              // the frame's floor plane (RANSAC mode): kp_frame_result.floor_plane
 };
 
 __device__ __forceinline__ int bit_length_dev(long long v)
@@ -1009,6 +1011,94 @@ __global__ void __launch_bounds__(256) k_e_plane_mask(const __grid_constant__ Ra
         mask[i] = plane_dist(pl, (double)xyz[3 * i], (double)xyz[3 * i + 1], (double)xyz[3 * i + 2]) < a.thr;
 }
 
+// The plane segment_plane returns: the covariance refit on the winning hypothesis's inliers (mask2 over the band), in
+// kp_ransac_device's two passes: pass 0 sums the inliers and counts them, pass 1 sums their moments around the
+// centroid.  Per-thread grid-stride sums, warp butterfly, warps in order, one slot per CTA; k_e_refit_fold adds the
+// slots in CTA order, so the plane is the same run to run and does not depend on the rest of the batch.
+constexpr int REFIT_NV = 6;
+struct RefitArgs {
+    const float *xyz; int64_t stride; DCnt n; EngDyn *dyn; int ransac_n;
+    const uint8_t *mask; int64_t mask_stride;
+    double *slots; int nblk;                                        // [seg][nblk][REFIT_NV]
+};
+template <int PASS>
+__global__ void __launch_bounds__(256) k_e_refit_sum(const __grid_constant__ RefitArgs a)
+{
+    constexpr int NV = PASS == 0 ? 4 : 6;                           // x, y, z, count  |  xx, xy, xz, yy, yz, zz
+    __shared__ double sh[8][NV];
+    const int seg = blockIdx.y;
+    const EngDyn &d = a.dyn[seg];
+    if (d.ransac_best < 0) return;
+    const int n = a.n.at(seg);
+    const float *xyz = a.xyz + 3 * seg * a.stride;
+    const uint8_t *mask = a.mask + seg * a.mask_stride;
+    const double cx = PASS ? d.refit_c[0] : 0.0, cy = PASS ? d.refit_c[1] : 0.0, cz = PASS ? d.refit_c[2] : 0.0;
+    double v[NV];
+#pragma unroll
+    for (int c = 0; c < NV; ++c) v[c] = 0.0;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        if (!mask[i]) continue;
+        const double x = DS((double)xyz[3 * i], cx), y = DS((double)xyz[3 * i + 1], cy), z = DS((double)xyz[3 * i + 2], cz);
+        if constexpr (PASS == 0) {
+            v[0] = DA(v[0], x); v[1] = DA(v[1], y); v[2] = DA(v[2], z); v[3] = DA(v[3], 1.0);
+        } else {
+            v[0] = DA(v[0], DM(x, x)); v[1] = DA(v[1], DM(x, y)); v[2] = DA(v[2], DM(x, z));
+            v[3] = DA(v[3], DM(y, y)); v[4] = DA(v[4], DM(y, z)); v[5] = DA(v[5], DM(z, z));
+        }
+    }
+#pragma unroll
+    for (int c = 0; c < NV; ++c) v[c] = kp_butterfly_sum(v[c]);
+    if ((threadIdx.x & 31) == 0)
+        for (int c = 0; c < NV; ++c) sh[threadIdx.x >> 5][c] = v[c];
+    __syncthreads();
+    if (threadIdx.x < NV) {
+        double s = 0.0;
+        for (int w = 0; w < 8; ++w) s = DA(s, sh[w][threadIdx.x]);
+        a.slots[((size_t)seg * a.nblk + blockIdx.x) * REFIT_NV + threadIdx.x] = s;
+    }
+}
+// pass 0: the centroid; pass 1: the frame's floor plane (NaN without a band of ransac_n points, 0 without a valid
+// hypothesis, the hypothesis when the refit is degenerate)
+__global__ void k_e_refit_fold(const __grid_constant__ RefitArgs a, int pass, int B)
+{
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= B) return;
+    EngDyn &d = a.dyn[f];
+    const double *sl = a.slots + (size_t)f * a.nblk * REFIT_NV;
+    const int nv = pass == 0 ? 4 : 6;
+    double s[REFIT_NV] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    if (d.ransac_best >= 0)
+        for (int b = 0; b < a.nblk; ++b)
+            for (int c = 0; c < nv; ++c) s[c] = DA(s[c], sl[(size_t)b * REFIT_NV + c]);
+    if (pass == 0) {
+        if (d.ransac_best >= 0) {
+            d.refit_c[0] = DD(s[0], s[3]); d.refit_c[1] = DD(s[1], s[3]); d.refit_c[2] = DD(s[2], s[3]); d.refit_c[3] = s[3];
+        }
+        return;
+    }
+    double pl[4] = {0.0, 0.0, 0.0, 0.0};
+    if (d.n_lo < a.ransac_n) {
+        pl[0] = pl[1] = pl[2] = pl[3] = NAN;
+    } else if (d.ransac_best >= 0) {
+        for (int c = 0; c < 4; ++c) pl[c] = d.plane[c];
+        double rp[4];
+        if (d.refit_c[3] >= 1.0 && cov_fit_from_moments(s, d.refit_c[0], d.refit_c[1], d.refit_c[2], rp))
+            for (int c = 0; c < 4; ++c) pl[c] = rp[c];
+    }
+    for (int c = 0; c < 4; ++c) d.floor_plane[c] = pl[c];
+}
+// pcd_above_plane (floor_removal.py:39-51) on the filter output: keep[i] = ((a*x + b*y) + c*z) + d < 0 in double, no FMA
+struct PlaneSideArgs { const float *xyz; int64_t stride; DCnt n; double pl[4]; uint8_t *keep; int64_t mask_stride; };
+__global__ void __launch_bounds__(256) k_e_plane_side(const __grid_constant__ PlaneSideArgs a)
+{
+    const int seg = blockIdx.y;
+    const int n = a.n.at(seg);
+    const float *xyz = a.xyz + 3 * seg * a.stride;
+    uint8_t *keep = a.keep + seg * a.mask_stride;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+        keep[i] = kp_affine(a.pl[0], a.pl[1], a.pl[2], a.pl[3], (double)xyz[3 * i], (double)xyz[3 * i + 1], (double)xyz[3 * i + 2]) < 0.0;
+}
+
 // rows src[0..n) appended to dst at row offset off[seg]; total[seg] = off + n
 struct AppendArgs { const float *src; float *dst; int64_t stride; DCnt n, off; DOut total; const uint32_t *aux_src; uint32_t *aux_dst; };
 __global__ void __launch_bounds__(256) k_e_append_rows(const __grid_constant__ AppendArgs a)
@@ -1049,6 +1139,7 @@ struct FinishArgs {
     DCnt n_filt;                                                    // rows of filt_out (the voxel + SOR [+ ROR] output)
     int do_floor, do_fsor;
     float *out; int64_t out_stride;                                 // rows; NULL -> no copy
+    int floor_mode; double floor_plane[4];                          // k_e_finish: the plane mode's plane
 };
 __device__ __forceinline__ void finish_pick(const FinishArgs &a, int f, const float *&src, int &n)
 {
@@ -1067,7 +1158,10 @@ __global__ void k_e_finish(const __grid_constant__ FinishArgs a, int B)
     d.n_out = n;
     kp_frame_result &r = a.res[f];
     r.n_fused = d.n_fused; r.n_voxel = d.n_voxel; r.n_sor = d.n_sor;
-    r.n_floor_inliers = (a.do_floor && !d.floor_skip) ? d.n_lo - d.n_rest : 0;
+    if (a.floor_mode == KP_FLOOR_PLANE)
+        r.n_floor_inliers = a.do_floor ? a.n_filt.at(f) - d.n_merged : 0;
+    else
+        r.n_floor_inliers = (a.do_floor && !d.floor_skip) ? d.n_lo - d.n_rest : 0;
     r.n_out = n;
     for (int i = 0; i < 5; ++i) {
         for (int e = 0; e < 16; ++e) r.icp_T[i][e] = i < a.S - 1 ? d.icp_T[i][e] : 0.0;
@@ -1076,6 +1170,7 @@ __global__ void k_e_finish(const __grid_constant__ FinishArgs a, int B)
         r.icp_iters[i] = i < a.S - 1 ? d.icp_iters[i] : 0;
     }
     r.status = d.status;
+    for (int c = 0; c < 4; ++c) r.floor_plane[c] = !a.do_floor ? NAN : (a.floor_mode == KP_FLOOR_PLANE ? a.floor_plane[c] : d.floor_plane[c]);
 }
 // the final cloud of every frame into the caller's buffer (device memory, or pinned host memory written through
 // the unified address space: the row count is only known on the device)
@@ -1521,6 +1616,20 @@ int stage_floor(kp_pipeline *pl, EngSlot &s, const float *in, const uint32_t *vi
         k_e_plane_mask<<<grid, 256, 0, ctx->stream>>>(r);
         KP_LAUNCH_CHECK(ctx);
     }
+    {
+        // the reported plane: refit on the inliers (the tie slots are free again: k_e_ransac_final has read them)
+        KP_PROFB(ctx, "floor_refit", 0.0);
+        RefitArgs f{s.C, NPs, DYN_CNT(s, n_lo), s.dyn, c.ransac_n, s.mask2, NPs, s.tie_slots, r.nblk};
+        const dim3 rg((unsigned)r.nblk, (unsigned)B);
+        k_e_refit_sum<0><<<rg, 256, 0, ctx->stream>>>(f);
+        KP_LAUNCH_CHECK(ctx);
+        k_e_refit_fold<<<kp_blocks(B, 32), 32, 0, ctx->stream>>>(f, 0, B);
+        KP_LAUNCH_CHECK(ctx);
+        k_e_refit_sum<1><<<rg, 256, 0, ctx->stream>>>(f);
+        KP_LAUNCH_CHECK(ctx);
+        k_e_refit_fold<<<kp_blocks(B, 32), 32, 0, ctx->stream>>>(f, 1, B);
+        KP_LAUNCH_CHECK(ctx);
+    }
     // outlier_cloud + upper (floor_removal.py:71-72): band outliers first, then the upper part
     KP_TRY(kp_b_compact_rows(L, s.scan, DYN_CNT(s, n_lo), s.mask2, NPs, 1, s.C, s.E, NPs, DYN_OUT(s, n_rest), vin ? s.vC : nullptr, s.vE));
     {
@@ -1530,6 +1639,23 @@ int stage_floor(kp_pipeline *pl, EngSlot &s, const float *in, const uint32_t *vi
         KP_LAUNCH_CHECK(ctx);
     }
     return KP_OK;
+}
+
+// ---- stage: floor removal at the caller's plane (pcd_above_plane): the kept rows of the filter output -> E, n_merged
+int stage_floor_plane(kp_pipeline *pl, EngSlot &s, const float *in, const uint32_t *vin, DCnt n_in)
+{
+    kp_ctx *ctx = s.ctx;
+    const kp_pipeline_cfg &c = pl->cfg;
+    const int B = pl->B;
+    const int64_t NPs = pl->NPr;
+    {
+        KP_PROFB(ctx, "plane_side", 0.0);
+        PlaneSideArgs a{in, NPs, n_in, {c.floor_plane[0], c.floor_plane[1], c.floor_plane[2], c.floor_plane[3]}, s.mask, NPs};
+        k_e_plane_side<<<dim3((unsigned)ctas_for(pl, 4), (unsigned)B), 256, 0, ctx->stream>>>(a);
+        KP_LAUNCH_CHECK(ctx);
+    }
+    BLaunch L{ctx, B, NPs, ctas_for(pl, 4)};
+    return kp_b_compact_rows(L, s.scan, n_in, s.mask, NPs, 0, in, s.E, NPs, DYN_OUT(s, n_merged), vin, vin ? s.vE : nullptr);
 }
 
 // ---- stage: ICP branch (voxel of the master and of every raw sub cloud, target grid + normals, all pairs together)
@@ -1801,7 +1927,8 @@ int enqueue_core(kp_pipeline *pl, EngSlot &s, bool fork)
     if (c.ror_nb_points > 0) KP_TRY(stage_ror(pl, s, sor_out, v_sor_out, DYN_CNT(s, n_sor), fo.xyz, fo.vijk));
     // ---- floor removal + SOR
     if (c.do_floor) {
-        KP_TRY(stage_floor(pl, s, fo.xyz, fo.vijk, fo.n));
+        if (c.floor_mode == KP_FLOOR_PLANE) KP_TRY(stage_floor_plane(pl, s, fo.xyz, fo.vijk, fo.n));
+        else KP_TRY(stage_floor(pl, s, fo.xyz, fo.vijk, fo.n));
         if (c.floor_sor_k > 0)
             KP_TRY(stage_sor(pl, s, 1, s.E, s.vE, DYN_CNT(s, n_merged), c.floor_sor_k, c.floor_sor_ratio, s.Fin, nullptr, DYN_OUT(s, n_fsor)));
     }
@@ -1811,7 +1938,8 @@ int enqueue_core(kp_pipeline *pl, EngSlot &s, bool fork)
         KP_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, s.ev_join, 0));
     }
     {
-        FinishArgs fa{s.dyn, s.d_res, S, fo.xyz, s.E, s.Fin, NPr, fo.n, c.do_floor, c.floor_sor_k > 0, nullptr, 0};
+        FinishArgs fa{s.dyn, s.d_res, S, fo.xyz, s.E, s.Fin, NPr, fo.n, c.do_floor, c.floor_sor_k > 0, nullptr, 0, c.floor_mode,
+                      {c.floor_plane[0], c.floor_plane[1], c.floor_plane[2], c.floor_plane[3]}};
         k_e_finish<<<kp_blocks(B, 32), 32, 0, ctx->stream>>>(fa, B);
         KP_LAUNCH_CHECK(ctx);
     }
@@ -1952,7 +2080,12 @@ int kp_pipeline_create(int device, const kp_pipeline_cfg *cfg, const float *h_xy
     if (!cfg || !h_xytab || !out) return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: NULL argument");
     if (cfg->S < 1 || cfg->S > ENG_MAX_S || cfg->P < 1) return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: need 1..6 sensors and P >= 1");
     if (!(cfg->voxel_size > 0.0)) return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: voxel_size <= 0");
-    if (cfg->do_floor && (cfg->ransac_n < 3 || cfg->ransac_n > RS_MAX_N || cfg->ransac_iters < 1 || !(cfg->ransac_thr > 0.0)))
+    if (cfg->floor_mode != KP_FLOOR_RANSAC && cfg->floor_mode != KP_FLOOR_PLANE)
+        return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: floor_mode must be KP_FLOOR_RANSAC or KP_FLOOR_PLANE (got %d)", cfg->floor_mode);
+    if (cfg->floor_mode == KP_FLOOR_PLANE && !(isfinite(cfg->floor_plane[0]) && isfinite(cfg->floor_plane[1]) && isfinite(cfg->floor_plane[2]) &&
+                                               isfinite(cfg->floor_plane[3])))
+        return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: the floor plane of KP_FLOOR_PLANE must have finite coefficients");
+    if (cfg->do_floor && cfg->floor_mode == KP_FLOOR_RANSAC && (cfg->ransac_n < 3 || cfg->ransac_n > RS_MAX_N || cfg->ransac_iters < 1 || !(cfg->ransac_thr > 0.0)))
         return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: segment_plane needs 3 <= ransac_n <= %d, iterations >= 1, threshold > 0", RS_MAX_N);
     if (cfg->do_icp && cfg->S > 1 && (!(cfg->icp_voxel > 0.0) || !(cfg->icp_max_corr > 0.0) || cfg->normals_max_nn < 1 || !(cfg->normals_radius > 0.0)))
         return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: ICP needs icp_voxel, icp_max_corr, normals_radius > 0 and normals_max_nn >= 1");

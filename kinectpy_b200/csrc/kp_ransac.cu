@@ -209,22 +209,6 @@ __global__ void k_plane_side(const float *xyz, int64_t n, double a, double b, do
     mask[i] = v < 0.0;
 }
 
-// host mirror of the covariance-determinant fit on pre-reduced moments
-bool cov_fit_from_moments(const double *m /*xx,xy,xz,yy,yz,zz*/, double cx, double cy, double cz, double *pl)
-{
-    double xx = m[0], xy = m[1], xz = m[2], yy = m[3], yz = m[4], zz = m[5];
-    double dx = yy * zz - yz * yz, dy = xx * zz - xz * xz, dz = xx * yy - xy * xy;
-    double a, b, c;
-    if (dx >= dy && dx >= dz) { a = dx; b = xz * yz - xy * zz; c = xy * yz - xz * yy; }
-    else if (dy >= dx && dy >= dz) { a = xz * yz - xy * zz; b = dy; c = xy * xz - yz * xx; }
-    else { a = xy * yz - xz * yy; b = xy * xz - yz * xx; c = dz; }
-    double nn = sqrt((a * a + b * b) + c * c);
-    if (nn == 0.0 || nn != nn) return false;
-    a /= nn; b /= nn; c /= nn;
-    pl[0] = a; pl[1] = b; pl[2] = c;
-    pl[3] = -((a * cx + b * cy) + c * cz);
-    return true;
-}
 }  // namespace
 
 // internal form (no workspace reset): used by the public entry and the frame pipeline

@@ -56,6 +56,11 @@ class PipelineConfig:
     # ror_nb_points points (themselves included) closer than ror_radius (in the cloud's unit)
     ror_nb_points: int = 0
     ror_radius: float = 0.0
+    # floor stage: FLOOR_RANSAC (band + segment_plane per frame; FrameOutput.floor_plane reports the plane) or
+    # FLOOR_PLANE (pcd_above_plane: keep the rows with a*x + b*y + c*z + d < 0 at floor_plane = (a, b, c, d), in the
+    # cloud's unit, then the floor SOR)
+    floor_mode: int = _cabi.FLOOR_RANSAC
+    floor_plane: tuple = (0.0, 0.0, 0.0, 0.0)
 
     def to_c(self) -> PipelineCfg:
         c = PipelineCfg()
@@ -70,6 +75,11 @@ class PipelineConfig:
         c.do_crop, c.crop_gate = int(self.do_crop), self.crop_gate
         c.resample_n, c.resample_mode = self.resample_n, self.resample_mode
         c.ror_nb_points, c.ror_radius = self.ror_nb_points, self.ror_radius
+        c.floor_mode = self.floor_mode
+        pl = [float(x) for x in self.floor_plane]
+        if len(pl) != 4:
+            raise ValueError("floor_plane must hold 4 coefficients (a, b, c, d)")
+        c.floor_plane[:] = pl
         return c
 
 
@@ -87,6 +97,7 @@ class FrameOutput:
     points: Optional[np.ndarray] = None
     fixed: Optional[np.ndarray] = None     # [N,3] fixed-N slot (want_fixed); zeros for a frame with status != 0
     status: int = 0
+    floor_plane: Optional[np.ndarray] = None   # float64 (4,): the frame's floor plane (NaN without one), see kp_api.h
 
 
 class FramePipeline:
@@ -183,6 +194,7 @@ class FramePipeline:
                              np.array(list(r.icp_fitness)[:S - 1]), np.array(list(r.icp_rmse)[:S - 1]),
                              np.array(list(r.icp_iters)[:S - 1]))
             fo.status = int(r.status)
+            fo.floor_plane = np.array(list(r.floor_plane), dtype=np.float64)
             if host is not None:
                 fo.points = host[f, :r.n_out].copy()
             if hfixed is not None:
