@@ -189,17 +189,21 @@ int kp_grid_build(kp_ctx *ctx, const float *d_xyz, int64_t n, double cell, const
     int total_bits = 0;
     KP_TRY(grid_layout(ctx, h_bounds6, cell, g, &total_bits));
     unsigned long long sentinel = 1ull << total_bits;   // total_bits <= 63
-    // hash capacity: power of two >= 2 * min(n, #cells)
+    // hash capacity: power of two >= 2 * min(n, #cells), in 64 bits (2 * n can exceed 2^32); the probe index is 32-bit
     double ncell = (double)g->dim[0] * g->dim[1] * g->dim[2];
     double want = 2.0 * ((double)n < ncell ? (double)n : ncell);
-    uint32_t cap = 1024;
+    uint64_t cap = 1024;
     while ((double)cap < want) cap <<= 1;
-    KP_TRY(kp_ws(ctx, (size_t)n, &g->d_sorted));
     const bool force_hash = getenv("KP_GRID_FORCE_HASH") != nullptr;   // test hook: exercise the huge-grid path
-    if (ncell <= 134217728.0 && !force_hash) {   // <= 32 MiB of cell map
+    const bool use_map = ncell <= 134217728.0 && !force_hash;           // <= 32 MiB of cell map
+    if (!use_map && cap > (1ull << 31))
+        return kp_set_err(ctx, KP_E_RANGE, "grid hash of %llu slots for %lld points over %.3g cells exceeds 2^31 slots",
+                          (unsigned long long)cap, (long long)n, ncell);
+    KP_TRY(kp_ws(ctx, (size_t)n, &g->d_sorted));
+    if (use_map) {
         KP_TRY(kp_ws(ctx, (size_t)(ncell / 32.0) + 2, &g->d_cellmap));
     } else {
-        g->hmask = cap - 1;
+        g->hmask = (uint32_t)(cap - 1);
         KP_TRY(kp_ws(ctx, (size_t)cap, &g->d_slots));
     }
     if (total_bits + 1 <= 32) return grid_sort_build<uint32_t>(ctx, d_xyz, n, g, total_bits, sentinel, nullptr, nullptr, true);
@@ -1341,7 +1345,9 @@ __device__ __forceinline__ void knn_wbf_body(const KnnParams &p)
             const int b1 = wh_select(hist, k, lane, cum);
             if (b1 >= 0) U2 = fmin(((double)b1 + 1.0) / (double)scale, capw);
             else if (cap_binding) U2 = capw;                  // fewer than k inside the cap: all of them are wanted
-            else { fail = true; if (p.dbg && lane == 0) atomicAdd(p.dbg + 1, 1); }   // (cannot happen: the cube holds k points within range)
+            // no bound: the cube holds k points but, with a radius cap, fewer than k of them lie inside it while the cube does
+            // not cover the cap ball (without a cap the cube's k points are all within range, and this cannot happen)
+            else { fail = true; if (p.dbg && lane == 0) atomicAdd(p.dbg + 1, 1); }
             cap_binding = p.r2cap > 0 && U2 >= capw;          // step 3 visits the whole cap ball: nothing eligible is missed
         }
         // ---- (3) + (4), retried once with shifted bin edges when the k-th distance sits within rounding of an

@@ -178,7 +178,9 @@ def test_voxel_nan_rows_wide_keys_and_errors(ctx, oracle):
 
 
 # ------------------------------------------------------------------ K3 ----
-@pytest.mark.parametrize("n,k,quantum", [(20000, 20, None), (8000, 50, 0.01), (3000, 200, None), (5000, 1, 0.02), (40, 64, None)])
+@pytest.mark.parametrize("n,k,quantum", [(20000, 20, None), (8000, 50, 0.01), (3000, 200, None), (5000, 1, 0.02), (40, 64, None),
+                                         (6000, 31, None), (6000, 32, 0.01), (6000, 33, None), (6000, 65, None),
+                                         (3000, 1000, None)])
 def test_knn_indices_bit_exact(ctx, oracle, n, k, quantum):
     pts = make_surface_cloud(n, seed=100 + k, quantum=quantum, outliers=0.02)
     ri, rd, rc = oracle.knn(pts, k)
