@@ -92,6 +92,12 @@ size_t kp_b_sort_hist_elems(int64_t n);   // int32 elements of g_hist for one se
 int kp_b_csum(const BLaunch &L, DCnt n, const double *x, int64_t x_stride, int mode, const double *aux, int64_t aux_stride,
               double *tmp, int64_t tmp_stride, double *out, int64_t out_stride);
 
+// Neighbour lists the normals search hands to the ICP (both run on the same grid over the target): for every target
+// position p whose search level 0 certified, up to KP_NLIST entries {position, d2 rounded down to float} of its certified
+// neighbours in canonical (d2, index) order, p itself left out, closed by a {-1, +inf} entry when shorter; and rho2[p], a
+// float lower bound of a squared radius inside which every other target point is in the list (0: no list).
+constexpr int KP_NLIST = 12;
+
 // ---- batched neighbour searches (kp_grid.cu): level 0 (thread per query, histogram select) -> level 1 (warp per
 // leftover query on a coarser grid) -> ring-expanding stragglers; the engine runs the list compactions and the
 // coarse grid build in between
@@ -108,10 +114,12 @@ struct KpKnnSegDesc {
     double *mean;                 // SOR: mean distance to the k nearest (by original index)
     const float *cloud;           // normals mode: the cloud, by original index
     float *normals;               // normals mode: output
+    int2 *nlist; float *nrho;     // normals mode, nullable: [cap][KP_NLIST] neighbour lists and [cap] rho2, by level-0 position
 };
 struct KpKnnBatch {
     void *d_params = nullptr, *h_params = nullptr;     // [3 levels][nseg] parameter blocks on the device and their host copy
     int nseg = 0, k = 0, mode = 0, cap_hist = 0, cap_warp = 0, rad = 1, cap_mid = 0, has_mid = 0;
+    int lists = 0;                // level 0 writes the neighbour lists (nlist / nrho of the segments)
 };
 // mode 0: mean distance of the k nearest (SOR); mode 1: normals from the <= k nearest inside `radius`
 // rho_a / rho_b: the two search radii of the voxel-brick level 0 (ignored without an index)
@@ -130,6 +138,8 @@ struct KpIcpPairDesc {
     const KpGridDev *tgt_grid;    // device: grid over the target (cell >= max_corr)
     const KpVbiDev *tgt_vbi;      // device, nullable: voxel-brick index over the target (preferred when it was built)
     const float *tgt_normals;     // by original target index
+    const int2 *tgt_list;         // nullable: neighbour lists of the target's grid positions (KP_NLIST per position)
+    const float *tgt_rho;         // with tgt_list: their rho2
     const float *src;             // source cloud (device), n_src rows
     const int32_t *n_src;         // device
     double init_T[16];
@@ -139,6 +149,7 @@ struct KpIcpBatch {
     void *d_params = nullptr, *d_work = nullptr;
     int npairs = 0, max_iter = 0, grid = 0;
     int64_t cap_src = 0;
+    int32_t *d_tally = nullptr;   // KP_DEBUG_ICP: [npairs][max_iter + 1][2] points decided by the list / searched in the grid
 };
 int kp_icp_batch_create(kp_ctx *ctx, const KpIcpPairDesc *pairs, int npairs, int64_t cap_src, double max_corr, int max_iter,
                         double rel_fitness, double rel_rmse, KpIcpBatch *out);

@@ -1267,6 +1267,7 @@ struct EngSlot {
     uint8_t *iflags[2] = {nullptr, nullptr};
     int32_t *ilist[2] = {nullptr, nullptr};
     float *nrm = nullptr;                             // [B][P][3]
+    int2 *ilists = nullptr; float *irho = nullptr;    // [B][Pr][KP_NLIST], [B][Pr]: the target's neighbour lists for the ICP
     uint32_t *ivijk = nullptr, *ivijk_sorted = nullptr;   // packed voxel coordinates of the ICP clouds / of the indexed target
     uint2 *ibricks = nullptr;
     KpIcpBatch icp;
@@ -1281,6 +1282,7 @@ struct kp_pipeline {
     int64_t cap_bricks = 1 << 23;
     int64_t NPr = 0, Pr = 0;          // row strides of the engine's own arrays: S*P and P rounded up to 64 (aligned vector access)
     bool use_graph = true, profiling = false, use_vbi_icp = false, use_vbi_knn = false;
+    bool icp_lists = true;            // ICP passes take the partner from the target's neighbour lists where they decide it (KP_ICP_LISTS)
     double rho_mult_a = 1.15, rho_mult_b = 2.0;
     double knn_mid = 1.5;             // cell of the mid level (x the level-0 cell); 0 = no mid level (KP_KNN_MID)
     int knn_rad = 1;                  // level-0 block radius in cells (KP_KNN_RAD): 1 = 27 cells of the full edge, 2 = 125 cells of half the edge
@@ -1832,6 +1834,7 @@ int slot_create(kp_pipeline *pl, EngSlot &s)
         SA(s.ig_rank, B * Pr); SA(s.ig_loc, B * Pr);
         if (pl->knn_mid > 0.0) { SA(s.isorted_m, B * Pr); SA(s.iflags_m, B * Pr); SA(s.ilist_m, B * Pr); }
         SA(s.nrm, B * Pr * 3);
+        if (pl->icp_lists) { SA(s.ilists, (size_t)B * Pr * KP_NLIST); SA(s.irho, B * Pr); }
         SA(s.ivijk, (size_t)B * S * Pr); SA(s.ivijk_sorted, B * Pr); SA(s.ibricks, (size_t)B * pl->cap_bricks);
         SAZ(s.isink, (size_t)B * S);
         for (int b = 0; b < B; ++b) {
@@ -1846,6 +1849,7 @@ int slot_create(kp_pipeline *pl, EngSlot &s)
             e.cnt0 = &s.dyn[b].cnt_l0[2]; e.cnt1 = &s.dyn[b].cnt_l1[2];
             e.cloud = s.ivox + 3 * (size_t)b * S * Pr;
             e.normals = s.nrm + 3 * (size_t)b * Pr;
+            if (pl->icp_lists) { e.nlist = s.ilists + (size_t)b * Pr * KP_NLIST; e.nrho = s.irho + (size_t)b * Pr; }
         }
         rc = kp_knn_batch_create(s.ctx, d.data(), B, c.normals_max_nn, 1, c.normals_radius, c.normals_radius * 1.001, c.normals_radius * 1.001,
                                  &s.knn_nrm);
@@ -1857,6 +1861,8 @@ int slot_create(kp_pipeline *pl, EngSlot &s)
                 e.tgt_grid = &s.dyn[b].g[2];
                 e.tgt_vbi = pl->use_vbi_icp ? &s.dyn[b].vbi[1] : nullptr;
                 e.tgt_normals = s.nrm + 3 * (size_t)b * Pr;
+                e.tgt_list = pl->icp_lists ? s.ilists + (size_t)b * Pr * KP_NLIST : nullptr;
+                e.tgt_rho = pl->icp_lists ? s.irho + (size_t)b * Pr : nullptr;
                 e.src = s.ivox + 3 * ((size_t)b * S + sn) * Pr;
                 e.n_src = &s.icl[(size_t)b * S + sn].n;
                 for (int i = 0; i < 16; ++i) e.init_T[i] = pl->T_icp[16 * sn + i];
@@ -2123,6 +2129,8 @@ int kp_pipeline_create(int device, const kp_pipeline_cfg *cfg, const float *h_xy
     p->B = B; p->W = W;
     p->use_graph = !(getenv("KP_PIPE_GRAPH") && atoi(getenv("KP_PIPE_GRAPH")) == 0);
     p->use_vbi_icp = getenv("KP_ICP_VBI") && atoi(getenv("KP_ICP_VBI")) != 0;   // 8 % fewer ICP pass time, paid back by the index build: off unless asked for
+    // the lists come from the normals search on the target grid, which the voxel-brick index replaces
+    p->icp_lists = !(getenv("KP_ICP_LISTS") && atoi(getenv("KP_ICP_LISTS")) == 0) && !p->use_vbi_icp;
     p->use_vbi_knn = getenv("KP_KNN_VBI") && atoi(getenv("KP_KNN_VBI")) != 0;   // measured slower than the grid level 0: off unless asked for
     p->knn_rad = (getenv("KP_KNN_RAD") && atoi(getenv("KP_KNN_RAD")) == 2) ? 2 : 1;
     if (getenv("KP_KNN_MID")) p->knn_mid = atof(getenv("KP_KNN_MID"));

@@ -278,6 +278,7 @@ struct KnnParams {
     const int32_t *nq_dev;                         // non-NULL: replaces nq
     const KpVbiDev *vbi;                           // voxel-brick index of the cloud (k_knn_vbi_b)
     double rho_a, rho_b;                           // its two search radii
+    int2 *nlist; float *nrho;                      // normals level 0 (k_knn_hist_b<..., true>): neighbour lists for the ICP
 };
 
 // batched launches read their parameter block from device memory (blockIdx.y selects the frame): uniform, cached
@@ -832,7 +833,9 @@ __device__ void kq_finish_normal(const KnnParams &p, int64_t row, int cnt, doubl
     p.normals[3 * row] = (float)nr[0]; p.normals[3 * row + 1] = (float)nr[1]; p.normals[3 * row + 2] = (float)nr[2];
 }
 
-template <int NB, int R, int HQT>
+// LIST (normals level 0 of the frame engine): also write the query's neighbour list and rho2 (kp_batch.cuh, KP_NLIST).
+// A template flag, so that the SOR searches, which share the <NB, R, HQT> instantiations, do not carry it.
+template <int NB, int R, int HQT, bool LIST = false>
 __device__ __forceinline__ void hq_query(const KnnParams &p, const KpGridDev &g, const int64_t q, unsigned char *smem_raw)
 {
     const int tid = threadIdx.x;
@@ -842,6 +845,7 @@ __device__ __forceinline__ void hq_query(const KnnParams &p, const KpGridDev &g,
     const float4 me = __ldg(p.qpts + q);
     const int64_t row = __float_as_int(me.w);
     const double qx = (double)me.x, qy = (double)me.y, qz = (double)me.z;
+    if constexpr (LIST) p.nrho[q] = 0.0f;        // no list unless this level certifies the query
     if (isnan(me.x)) {
         if (p.mode == KQ_MODE_KNN) kq_finalize(p, row, 0, nullptr, nullptr, 0);
         else { double sm[9]; kq_finish_normal(p, row, 0, sm); }
@@ -985,6 +989,8 @@ __device__ __forceinline__ void hq_query(const KnnParams &p, const KpGridDev &g,
     double sm[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
     int cnt = 0;
     bool bad = false, closed = false;
+    int nl = 0;                 // LIST: entries written
+    double dcut = -1.0;         // LIST: d2 of the first certified neighbour the list had no room for
     float4 cn = m > 0 ? __ldg(g.pts + buf[0]) : make_float4(0.f, 0.f, 0.f, 0.f);
     for (int i = 0; i < m; ++i) {
         const float4 c = cn;
@@ -999,6 +1005,15 @@ __device__ __forceinline__ void hq_query(const KnnParams &p, const KpGridDev &g,
                 const double x = (double)c.x, y = (double)c.y, z = (double)c.z;
                 sm[0] += x; sm[1] += y; sm[2] += z;
                 sm[3] += x * x; sm[4] += x * y; sm[5] += x * z; sm[6] += y * y; sm[7] += y * z; sm[8] += z * z;
+                if constexpr (LIST) {
+                    // the query's own position is left out wherever it sits (a duplicate point with a lower index
+                    // precedes it at d2 = 0); the list is only trusted below once the query is certified
+                    const int pos = (int)buf[i * HQT];
+                    if (pos != (int)q) {
+                        if (nl < KP_NLIST) p.nlist[q * KP_NLIST + nl++] = make_int2(pos, __float_as_int(__double2float_rd(d)));
+                        else if (dcut < 0.0) dcut = d;
+                    }
+                }
             } else {
                 if (p.idx) p.idx[row * k + cnt] = id;
                 if (p.d2) p.d2[row * k + cnt] = d;
@@ -1013,6 +1028,13 @@ __device__ __forceinline__ void hq_query(const KnnParams &p, const KpGridDev &g,
     if (all && G.cap_binding) exact = true;
     else exact = cnt == k && pd < hq_lower_edge(b, G.scale) && (G.cap_binding || pd < G.Rcert2);
     if (bad || !exact) { p.strag_flags[q] = 1; return; }
+    if constexpr (LIST) {
+        // every other point closer than rho lies in the list: the first one cut off bounds it when the list is full;
+        // else all of them inside the radius when fewer than k qualified, else the k-th neighbour (the query's own
+        // entry counts towards k)
+        if (nl < KP_NLIST) p.nlist[q * KP_NLIST + nl] = make_int2(-1, __float_as_int(INFINITY));
+        p.nrho[q] = __double2float_rd(dcut >= 0.0 ? dcut : (cnt < k ? p.r2cap : pd));
+    }
     if (normals) { kq_finish_normal(p, row, cnt, sm); return; }
     if (p.idx) for (int t = cnt; t < k; ++t) p.idx[row * k + t] = -1;
     if (p.d2) for (int t = cnt; t < k; ++t) p.d2[row * k + t] = INFINITY;
@@ -1035,7 +1057,7 @@ struct KnnBatchArgs { KnnParams p[KNN_ARG_SEGS]; };
 #ifndef KNN_MIN_CTAS_T
 #define KNN_MIN_CTAS_T 0
 #endif
-template <int NB, int R, int HQT>
+template <int NB, int R, int HQT, bool LIST = false>
 __device__ __forceinline__ void knn_hist_b_body(const KnnBatchArgs &a, unsigned char *smem_raw)
 {
     const KnnParams &p = a.p[blockIdx.y];
@@ -1043,13 +1065,13 @@ __device__ __forceinline__ void knn_hist_b_body(const KnnBatchArgs &a, unsigned 
     // level 0: every point of the cloud; coarser levels: the positions the level before could not certify (qlist)
     const int64_t nq = p.qlist ? (int64_t)*p.qcount : (int64_t)*p.nq_dev;
     for (int64_t w = (int64_t)blockIdx.x * HQT + threadIdx.x; w < nq; w += (int64_t)gridDim.x * HQT)
-        hq_query<NB, R, HQT>(p, g, p.qlist ? (int64_t)p.qlist[w] : w, smem_raw);
+        hq_query<NB, R, HQT, LIST>(p, g, p.qlist ? (int64_t)p.qlist[w] : w, smem_raw);
 }
-template <int NB, int R, int HQT>
+template <int NB, int R, int HQT, bool LIST = false>
 __global__ void __launch_bounds__(HQT, KNN_MIN_CTAS_T > 0 ? KNN_MIN_CTAS_T / HQT : 1) k_knn_hist_b(const __grid_constant__ KnnBatchArgs a)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    knn_hist_b_body<NB, R, HQT>(a, smem_raw);
+    knn_hist_b_body<NB, R, HQT, LIST>(a, smem_raw);
 }
 // the mid level (leftover list on the 1.5 x grid): the same code under its own name, so that launch lists and profiles
 // tell the two levels apart
@@ -1679,6 +1701,7 @@ int kp_knn_batch_create(kp_ctx *ctx, const KpKnnSegDesc *segs, int nseg, int k, 
                         KpKnnBatch *out)
 {
     out->nseg = nseg; out->k = k; out->mode = mode;
+    out->lists = mode == 1 && nseg > 0 && segs[0].nlist != nullptr && segs[0].vbi == nullptr;
     out->rad = (getenv("KP_KNN_RAD") && atoi(getenv("KP_KNN_RAD")) == 2) ? 2 : 1;
     static const int slack = getenv("KP_KNN_SLACK") ? atoi(getenv("KP_KNN_SLACK")) : 8;
     out->cap_hist = k + slack;
@@ -1701,6 +1724,7 @@ int kp_knn_batch_create(kp_ctx *ctx, const KpKnnSegDesc *segs, int nseg, int k, 
         KnnParams a = p;
         a.cap = out->cap_hist; a.gdev = d.g0; a.nq_dev = d.n; a.strag_flags = d.flags0;
         a.vbi = d.vbi; a.rho_a = rho_a; a.rho_b = rho_b;
+        a.nlist = d.nlist; a.nrho = d.nrho;
         h[s] = a;
         // level 1: the leftovers of the level before (list0, or the mid level's list), one warp each, against the coarse grid
         KnnParams b = p;
@@ -1730,10 +1754,14 @@ int kp_knn_batch_create(kp_ctx *ctx, const KpKnnSegDesc *segs, int nseg, int k, 
         if (k <= 32) {
             KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_hist_b<32, 2, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h));
             KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_hist_b<32, 1, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h));
+            KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_hist_b<32, 2, 128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h));
+            KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_hist_b<32, 1, 128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h));
             KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_vbi_b<32, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h));
         } else {
             KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_hist_b<64, 2, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h));
             KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_hist_b<64, 1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h));
+            KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_hist_b<64, 2, 64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h));
+            KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_hist_b<64, 1, 64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h));
             KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_vbi_b<64, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h));
         }
     }
@@ -1742,6 +1770,8 @@ int kp_knn_batch_create(kp_ctx *ctx, const KpKnnSegDesc *segs, int nseg, int k, 
         const int pct = atoi(getenv("KP_KNN_CARVEOUT"));
         KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_hist_b<32, 1, 128>, cudaFuncAttributePreferredSharedMemoryCarveout, pct));
         KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_hist_b<64, 1, 64>, cudaFuncAttributePreferredSharedMemoryCarveout, pct));
+        KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_hist_b<32, 1, 128, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct));
+        KP_CUDA(ctx, cudaFuncSetAttribute(k_knn_hist_b<64, 1, 64, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct));
     }
     return KP_OK;
 }
@@ -1750,7 +1780,7 @@ void kp_knn_batch_destroy(KpKnnBatch *b)
     if (b && b->d_params) { cudaFree(b->d_params); b->d_params = nullptr; }
     if (b && b->h_params) { free(b->h_params); b->h_params = nullptr; }
 }
-template <int NB, int R, int T>
+template <int NB, int R, int T, bool LIST = false>
 static int knn_level0_launch(kp_ctx *ctx, const KpKnnBatch &b, int64_t cap_rows, int per_sm, int level = 0)
 {
     const KnnParams *hp = (const KnnParams *)b.h_params + (size_t)level * b.nseg;
@@ -1763,7 +1793,7 @@ static int knn_level0_launch(kp_ctx *ctx, const KpKnnBatch &b, int64_t cap_rows,
         memset(&a, 0, sizeof a);
         for (int i = 0; i < ns; ++i) a.p[i] = hp[s0 + i];
         if (level == 3 && NB == 64 && R == 1 && T == 64) k_knn_mid_b<<<dim3((unsigned)(gx > 0 ? gx : 1), (unsigned)ns), T, smem, ctx->stream>>>(a);
-        else k_knn_hist_b<NB, R, T><<<dim3((unsigned)(gx > 0 ? gx : 1), (unsigned)ns), T, smem, ctx->stream>>>(a);
+        else k_knn_hist_b<NB, R, T, LIST><<<dim3((unsigned)(gx > 0 ? gx : 1), (unsigned)ns), T, smem, ctx->stream>>>(a);
         KP_LAUNCH_CHECK(ctx);
     }
     return KP_OK;
@@ -1773,6 +1803,10 @@ int kp_knn_batch_level0(kp_ctx *ctx, const KpKnnBatch &b, int64_t cap_rows)
     KP_PROFB(ctx, "knn_level0", 0.0);
     // persistent CTAs per SM and segment (KP_KNN_CTAS): fewer leave registers for another batch's kernels on the same SM
     static const int per_sm = getenv("KP_KNN_CTAS") ? atoi(getenv("KP_KNN_CTAS")) : 24;
+    if (b.lists) {
+        if (b.k <= 32) return b.rad == 2 ? knn_level0_launch<32, 2, 128, true>(ctx, b, cap_rows, per_sm) : knn_level0_launch<32, 1, 128, true>(ctx, b, cap_rows, per_sm);
+        return b.rad == 2 ? knn_level0_launch<64, 2, 64, true>(ctx, b, cap_rows, per_sm * 4 / 3) : knn_level0_launch<64, 1, 64, true>(ctx, b, cap_rows, per_sm * 4 / 3);
+    }
     if (b.k <= 32) return b.rad == 2 ? knn_level0_launch<32, 2, 128>(ctx, b, cap_rows, per_sm) : knn_level0_launch<32, 1, 128>(ctx, b, cap_rows, per_sm);
     return b.rad == 2 ? knn_level0_launch<64, 2, 64>(ctx, b, cap_rows, per_sm * 4 / 3) : knn_level0_launch<64, 1, 64>(ctx, b, cap_rows, per_sm * 4 / 3);
 }

@@ -13,6 +13,7 @@
 // same order), composes T and publishes the next update, the pass counter and a `done` flag.  The host enqueues
 // max_iter+1 passes without reading anything back; passes after `done` return immediately.
 #include <math.h>
+#include <stdio.h>
 #include <string.h>
 #include <stdlib.h>
 #include <vector>
@@ -71,6 +72,9 @@ struct IcpParams {
     double init_T[16];
     double *res_T, *res_fit, *res_rmse; int32_t *res_iters;   // where the converged state of the pair goes
     const KpVbiDev *vbi;        // voxel-brick index over the target (device); used instead of the grid when it was built
+    const int2 *tlist;          // nullable: the target's neighbour lists by grid position (kp_batch.cuh, KP_NLIST)
+    const float *trho;          // with tlist: their rho2
+    int32_t *tally;             // nullable (KP_DEBUG_ICP): [max_iter + 1][2] points decided by the list / searched in the grid
 };
 
 __device__ __forceinline__ double icp_slack(const KpGridDev &g, double max_corr)
@@ -185,6 +189,48 @@ __device__ __forceinline__ int icp_nearest(const KpGridDev &g, double sx, double
                 }
             }
         }
+    }
+    return bpos;
+}
+
+// The same answer from the neighbour list of the previous partner t (position prev, squared distance d2t < r2 from the
+// point), for a point with 4 * d2t * (1 + 1e-6) < rho2(t): every target point at least as close as t lies within 2
+// sqrt(d2t) of t (triangle inequality), so inside rho(t), so in t's list, which is in canonical order; the scan stops at
+// the first entry beyond that bound.  Candidates are tested exactly as in icp_nearest, so the result is the same.
+__device__ __forceinline__ int icp_nearest_list(const KpGridDev &g, const int4 *__restrict__ list, double sx, double sy, double sz,
+                                                double r2, double slack, int prev, double d2t, int idt, float stop)
+{
+    double bd = d2t;
+    int bi = idt, bpos = prev;
+    const float fx32 = (float)sx, fy32 = (float)sy, fz32 = (float)sz;
+    float lim32 = __double2float_ru(bd + slack);
+    // four entries (one 32-byte sector) per trip, their points requested together
+    for (int j = 0; j < KP_NLIST; j += 4) {
+        const int4 e01 = __ldg(list + (size_t)prev * (KP_NLIST / 2) + j / 2), e23 = __ldg(list + (size_t)prev * (KP_NLIST / 2) + j / 2 + 1);
+        const int pos[4] = {e01.x, e01.z, e23.x, e23.z};
+        const float ed[4] = {__int_as_float(e01.y), __int_as_float(e01.w), __int_as_float(e23.y), __int_as_float(e23.w)};
+        // an entry counts only while every entry before it did: the closing {-1, +inf} entry ends the list, and the
+        // words behind it were never written
+        bool in[4];
+        in[0] = ed[0] <= stop;
+#pragma unroll
+        for (int u = 1; u < 4; ++u) in[u] = in[u - 1] && ed[u] <= stop;
+        float4 q[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) q[u] = __ldg(g.pts + (in[u] ? pos[u] : prev));
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            if (!in[u]) break;                           // the first entry beyond the bound, or the end of the list
+            const float ex = fx32 - q[u].x, ey = fy32 - q[u].y, ez = fz32 - q[u].z;
+            if (__fmaf_rn(ez, ez, __fmaf_rn(ey, ey, ex * ex)) > lim32) continue;
+            const double d2 = kp_d2(sx, sy, sz, (double)q[u].x, (double)q[u].y, (double)q[u].z);
+            const int id = __float_as_int(q[u].w);
+            if (d2 < r2 && (d2 < bd || (d2 == bd && id < bi))) {
+                bd = d2; bi = id; bpos = pos[u];
+                lim32 = __double2float_ru(bd + slack);
+            }
+        }
+        if (!in[3]) break;
     }
     return bpos;
 }
@@ -324,54 +370,24 @@ __device__ void icp_finish(const IcpParams &p, IcpState *st, const double *tot, 
     __threadfence();
 }
 
-// One pass: update + correspondence + accumulation, one thread per source point; the last CTA solves and
-// publishes the next update.
+// The per-point terms of one tile of ICP_THREADS source points (point i of this thread at (sx, sy, sz), partner bpos),
+// reduced over each warp into sh[warp][*].  Warp reduction of the 29 scalars by halving exchange: at step s a lane keeps
+// one half of its values and trades the other half with lane^s, so 32 values are fully reduced in 31 exchanges (lane L
+// ends up with the warp total of value L) instead of 32 butterflies of 5.  Fixed tree -> deterministic.
 template <int MODE>
-__device__ __forceinline__ void icp_iter_body(const IcpParams &p)
+__device__ __forceinline__ void icp_tile_terms(const IcpParams &p, const float4 *tpts, int i, double sx, double sy, double sz, int bpos,
+                                               double (*sh)[ICP_NV], int lane, int warp)
 {
-    __shared__ double sh[ICP_THREADS / 32][ICP_NV];
-    __shared__ double part[ICP_THREADS / 32][32];
-    __shared__ double tot[ICP_NV];
-    __shared__ unsigned int s_ticket;
-    IcpState *st = p.st;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int i = blockIdx.x * ICP_THREADS + tid;
-    // the point, its last partner and the state words are requested together: one memory round trip before the
-    // first arithmetic instead of two (a pass launched after `done` only wastes these few loads)
-    double sx0 = 0.0, sy0 = 0.0, sz0 = 0.0;
-    int prev0 = -1;
-    if (i < p.ns) {
-        sx0 = p.cur[3 * (int64_t)i]; sy0 = p.cur[3 * (int64_t)i + 1]; sz0 = p.cur[3 * (int64_t)i + 2];
-        prev0 = p.corr[i];              // (not yet written in pass 0: ignored there)
-    }
-    if (st->done) return;
-    const int pass = st->pass;          // advanced only after every CTA has taken its ticket
-    const KpGridDev &g = p.g;
     bool has = false;
     // plane / colored: J (6) and r of the geometric term; colored adds the photometric row J2, r2;
     // point-to-point: J[0..2] = s, J[3..5] = t
     double J[6] = {0, 0, 0, 0, 0, 0}, r = 0.0, bd = 0.0;
     double J2[6] = {0, 0, 0, 0, 0, 0}, r2v = 0.0;
     if (i < p.ns) {
-        double sx = sx0, sy = sy0, sz = sz0;
-        int prev = pass > 0 ? prev0 : -1;
-        if (pass > 0) {
-            const double *U = st->U;
-            const double x2 = kp_affine(U[0], U[1], U[2], U[3], sx, sy, sz);
-            const double y2 = kp_affine(U[4], U[5], U[6], U[7], sx, sy, sz);
-            const double z2 = kp_affine(U[8], U[9], U[10], U[11], sx, sy, sz);
-            sx = x2; sy = y2; sz = z2;
-            p.cur[3 * (int64_t)i] = sx; p.cur[3 * (int64_t)i + 1] = sy; p.cur[3 * (int64_t)i + 2] = sz;
-        }
-        int bpos = -1;
-        const bool use_vbi = p.vbi != nullptr && p.vbi->ok;
-        if (use_vbi) {
-            if (!isnan(sx)) { const KpVbiDev v = *p.vbi; bpos = icp_nearest_vbi(v, sx, sy, sz, p.r2, p.slack, prev); }
-        } else if (!isnan(sx) && g.dim[0] > 0) bpos = icp_nearest(g, sx, sy, sz, p.r2, p.slack, prev);
         p.corr[i] = bpos;
         if (bpos >= 0) {
             has = true;
-            const float4 q = __ldg((use_vbi ? p.vbi->pts : g.pts) + bpos);
+            const float4 q = __ldg(tpts + bpos);
             const int bi = __float_as_int(q.w);
             const double ex = sx - (double)q.x, ey = sy - (double)q.y, ez = sz - (double)q.z;
             bd = (ex * ex + ey * ey) + ez * ez;
@@ -404,9 +420,6 @@ __device__ __forceinline__ void icp_iter_body(const IcpParams &p)
             }
         }
     }
-    // Warp reduction of the 29 scalars by halving exchange: at step s a lane keeps one half of its values and
-    // trades the other half with lane^s, so 32 values are fully reduced in 31 exchanges (lane L ends up with
-    // the warp total of value L) instead of 32 butterflies of 5.  Fixed tree -> deterministic.
     if (__any_sync(KP_FULL, has)) {
         double v[32];
         if (MODE == ICP_POINT) {
@@ -442,22 +455,161 @@ __device__ __forceinline__ void icp_iter_body(const IcpParams &p)
     } else if (lane < ICP_NV) {
         sh[warp][lane] = 0.0;
     }
-    __syncthreads();
-    if (tid < ICP_NV) {
-        double s = 0;
-        for (int w = 0; w < ICP_THREADS / 32; ++w) s += sh[w][tid];
-        p.slots[(size_t)blockIdx.x * ICP_NV + tid] = s;
+}
+
+// One pass: update + correspondence + accumulation, one thread per source point of a tile of ICP_THREADS; every tile
+// leaves one slot row; the last CTA solves and publishes the next update.
+// QUEUE (batched kernel): a CTA owns ICP_B_TILES tiles.  A point whose partner the target's neighbour list decides skips
+// the grid search (icp_nearest_list); the others are packed into a CTA-wide queue and searched by consecutive threads,
+// so the searches run in dense warps and a CTA's threads each search about once per pass however many points the lists
+// decide.  Each result goes back to the point's slot, and its own thread then goes on as without the queue: the same
+// per-point terms and the same per-tile reduction tree, so the sums are bit-identical.
+constexpr int ICP_B_TILES = 4;
+constexpr int ICP_PENDING = -2;    // queue path: a point waiting for its grid search
+template <int MODE, bool QUEUE = false>
+__device__ __forceinline__ void icp_iter_body(const IcpParams &p)
+{
+    constexpr int TPC = QUEUE ? ICP_B_TILES : 1;       // tiles per CTA
+    constexpr int W = ICP_THREADS / 32;
+    __shared__ double sh[ICP_THREADS / 32][ICP_NV];
+    __shared__ double part[ICP_THREADS / 32][32];
+    __shared__ double tot[ICP_NV];
+    __shared__ unsigned int s_ticket;
+    IcpState *st = p.st;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const unsigned ntiles = max(1u, ((unsigned)p.ns + ICP_THREADS - 1) / ICP_THREADS);
+    const KpGridDev &g = p.g;
+    const bool use_vbi = p.vbi != nullptr && p.vbi->ok;
+    const float4 *tpts = use_vbi ? p.vbi->pts : g.pts;
+    int pass;
+    if constexpr (!QUEUE) {
+        const int i = blockIdx.x * ICP_THREADS + tid;
+        // the point, its last partner and the state words are requested together: one memory round trip before the
+        // first arithmetic instead of two (a pass launched after `done` only wastes these few loads)
+        double sx = 0.0, sy = 0.0, sz = 0.0;
+        int prev0 = -1;
+        if (i < p.ns) {
+            sx = p.cur[3 * (int64_t)i]; sy = p.cur[3 * (int64_t)i + 1]; sz = p.cur[3 * (int64_t)i + 2];
+            prev0 = p.corr[i];              // (not yet written in pass 0: ignored there)
+        }
+        if (st->done) return;
+        pass = st->pass;                    // advanced only after every CTA has taken its ticket
+        int bpos = -1;
+        if (i < p.ns) {
+            const int prev = pass > 0 ? prev0 : -1;
+            if (pass > 0) {
+                const double *U = st->U;
+                const double x2 = kp_affine(U[0], U[1], U[2], U[3], sx, sy, sz);
+                const double y2 = kp_affine(U[4], U[5], U[6], U[7], sx, sy, sz);
+                const double z2 = kp_affine(U[8], U[9], U[10], U[11], sx, sy, sz);
+                sx = x2; sy = y2; sz = z2;
+                p.cur[3 * (int64_t)i] = sx; p.cur[3 * (int64_t)i + 1] = sy; p.cur[3 * (int64_t)i + 2] = sz;
+            }
+            if (use_vbi) {
+                if (!isnan(sx)) { const KpVbiDev v = *p.vbi; bpos = icp_nearest_vbi(v, sx, sy, sz, p.r2, p.slack, prev); }
+            } else if (!isnan(sx) && g.dim[0] > 0) bpos = icp_nearest(g, sx, sy, sz, p.r2, p.slack, prev);
+        }
+        icp_tile_terms<MODE>(p, tpts, i, sx, sy, sz, bpos, sh, lane, warp);
+        __syncthreads();
+        if (tid < ICP_NV) {
+            double s = 0;
+            for (int w = 0; w < W; ++w) s += sh[w][tid];
+            p.slots[(size_t)blockIdx.x * ICP_NV + tid] = s;
+        }
+    } else {
+        constexpr int NPC = TPC * ICP_THREADS;
+        __shared__ double s_x[NPC], s_y[NPC], s_z[NPC];
+        __shared__ int s_prev[NPC], s_bpos[NPC], s_queue[NPC], s_wn[TPC * W];
+        if (st->done) return;
+        pass = st->pass;
+        const double *U = st->U;
+        // 1. update every point; the list decides what it can, the rest is marked pending
+#pragma unroll 1
+        for (int h = 0; h < TPC; ++h) {
+            const int i = (blockIdx.x * TPC + h) * ICP_THREADS + tid, slot = h * ICP_THREADS + tid;
+            double sx = 0.0, sy = 0.0, sz = 0.0;
+            int prev = -1, bpos = -1;
+            bool listed = false;
+            if (i < p.ns) {
+                sx = p.cur[3 * (int64_t)i]; sy = p.cur[3 * (int64_t)i + 1]; sz = p.cur[3 * (int64_t)i + 2];
+                if (pass > 0) {
+                    prev = p.corr[i];
+                    const double x2 = kp_affine(U[0], U[1], U[2], U[3], sx, sy, sz);
+                    const double y2 = kp_affine(U[4], U[5], U[6], U[7], sx, sy, sz);
+                    const double z2 = kp_affine(U[8], U[9], U[10], U[11], sx, sy, sz);
+                    sx = x2; sy = y2; sz = z2;
+                    p.cur[3 * (int64_t)i] = sx; p.cur[3 * (int64_t)i + 1] = sy; p.cur[3 * (int64_t)i + 2] = sz;
+                }
+                if (!isnan(sx) && (use_vbi || g.dim[0] > 0)) {
+                    bpos = ICP_PENDING;
+                    if (p.tlist && prev >= 0) {
+                        const float4 t = __ldg(g.pts + prev);
+                        const float rho2 = __ldg(p.trho + prev);
+                        const double d2t = kp_d2(sx, sy, sz, (double)t.x, (double)t.y, (double)t.z);
+                        // 4 d2t (1 + 1e-6), rounded up: the 1e-6 covers the rounding of the distances and of rho2 (DESIGN §3)
+                        const float stop = __double2float_ru(4.0 * d2t * (1.0 + 1e-6));
+                        if (d2t < p.r2 && stop < rho2) {
+                            bpos = icp_nearest_list(g, reinterpret_cast<const int4 *>(p.tlist), sx, sy, sz, p.r2, p.slack, prev, d2t, __float_as_int(t.w), stop);
+                            listed = true;
+                        }
+                    }
+                }
+            }
+            s_x[slot] = sx; s_y[slot] = sy; s_z[slot] = sz; s_prev[slot] = prev; s_bpos[slot] = bpos;
+            const unsigned need = __ballot_sync(KP_FULL, bpos == ICP_PENDING);
+            if (lane == 0) s_wn[h * W + warp] = __popc(need);
+            if (p.tally) {
+                const unsigned nl = __ballot_sync(KP_FULL, listed);
+                if (lane == 0) { atomicAdd(p.tally + 2 * pass, __popc(nl)); atomicAdd(p.tally + 2 * pass + 1, __popc(need)); }
+            }
+        }
+        __syncthreads();
+        // 2. the pending points into the queue, in slot order
+        int nq = 0;
+#pragma unroll
+        for (int w = 0; w < TPC * W; ++w) nq += s_wn[w];
+#pragma unroll 1
+        for (int h = 0; h < TPC; ++h) {
+            const int slot = h * ICP_THREADS + tid;
+            const bool pend = s_bpos[slot] == ICP_PENDING;
+            const unsigned need = __ballot_sync(KP_FULL, pend);
+            int base = 0;
+            for (int w = 0; w < h * W + warp; ++w) base += s_wn[w];
+            if (pend) s_queue[base + __popc(need & ((1u << lane) - 1u))] = slot;
+        }
+        __syncthreads();
+        // 3. the grid searches, one per thread in turn
+        for (int j = tid; j < nq; j += ICP_THREADS) {
+            const int o = s_queue[j];
+            if (use_vbi) { const KpVbiDev v = *p.vbi; s_bpos[o] = icp_nearest_vbi(v, s_x[o], s_y[o], s_z[o], p.r2, p.slack, s_prev[o]); }
+            else s_bpos[o] = icp_nearest(g, s_x[o], s_y[o], s_z[o], p.r2, p.slack, s_prev[o]);
+        }
+        __syncthreads();
+        // 4. per tile: the terms of the thread's own point, the tile's slot row
+#pragma unroll 1
+        for (int h = 0; h < TPC; ++h) {
+            const int tile = blockIdx.x * TPC + h, slot = h * ICP_THREADS + tid;
+            icp_tile_terms<MODE>(p, tpts, tile * ICP_THREADS + tid, s_x[slot], s_y[slot], s_z[slot], s_bpos[slot], sh, lane, warp);
+            __syncthreads();
+            if (tid < ICP_NV && (unsigned)tile < ntiles) {
+                double s = 0;
+                for (int w = 0; w < W; ++w) s += sh[w][tid];
+                p.slots[(size_t)tile * ICP_NV + tid] = s;
+            }
+            if (h + 1 < TPC) __syncthreads();          // sh is written again by the next tile
+        }
     }
-    // ---- two-level hand-over.  CTAs form groups of ICP_GROUP consecutive blocks; the last CTA of a group to
+    // ---- two-level hand-over.  Tiles form groups of ICP_GROUP consecutive slot rows; the last CTA of a group to
     // finish (group ticket) folds the group's slot rows into one group row, then takes the global ticket; the last
     // group folds the group rows.  Each fold is one round of loads (a row per warp-slot, fixed order), instead of
-    // one CTA walking ~2000 rows; the tickets see ICP_GROUP and gridDim/ICP_GROUP atomics per address instead of
+    // one CTA walking ~2000 rows; the tickets see ICP_GROUP / TPC and gridDim/ICP_GROUP atomics per address instead of
     // gridDim.  Fixed tree -> the sums do not depend on which CTA does the folding.
-    constexpr int W = ICP_THREADS / 32;
     // (the CTAs that own source points: a batched launch is sized for the capacity and the rest left at once)
-    const unsigned nact = max(1u, ((unsigned)p.ns + ICP_THREADS - 1) / ICP_THREADS);
-    const unsigned group = blockIdx.x / ICP_GROUP, ngroups = (nact + ICP_GROUP - 1) / ICP_GROUP;
-    const unsigned g0 = group * ICP_GROUP, gsize = min((unsigned)ICP_GROUP, nact - g0);
+    constexpr unsigned CG = ICP_GROUP / TPC;           // CTAs per group
+    const unsigned nact = (ntiles + TPC - 1) / TPC;
+    const unsigned group = blockIdx.x / CG, ngroups = (nact + CG - 1) / CG;
+    const unsigned gsize = min(CG, nact - group * CG);
+    const unsigned t0 = group * ICP_GROUP, grows = min((unsigned)ICP_GROUP, ntiles - t0);
     auto fold = [&](const double *rows, unsigned nrows, double *dst_sh) {
         // warp w adds rows w, w + W, ... (all its loads in flight together), then the W partial sums in order
         double sacc = 0;
@@ -487,7 +639,7 @@ __device__ __forceinline__ void icp_iter_body(const IcpParams &p)
     __syncthreads();
     if (s_ticket != gsize - 1) return;
     __threadfence();
-    fold(p.slots + (size_t)g0 * ICP_NV, gsize, tot);
+    fold(p.slots + (size_t)t0 * ICP_NV, grows, tot);
     if (tid < ICP_NV) p.gslots[(size_t)group * ICP_NV + tid] = tot[tid];
     if (tid == 0) p.gticket[group] = 0;             // re-armed for the next pass
     __threadfence();
@@ -514,9 +666,9 @@ __global__ void __launch_bounds__(ICP_THREADS, ICP_B_CTAS) k_icp_iter_b(const Ic
     // CTAs beyond the pair's source count, and every CTA of a converged pair, leave before touching anything else
     const IcpParams *me = pp + blockIdx.y;
     const int ns = *me->ns_dev;
-    if (blockIdx.x * ICP_THREADS >= (unsigned)max(ns, 1) || me->st->done) return;
+    if (blockIdx.x * (ICP_B_TILES * ICP_THREADS) >= (unsigned)max(ns, 1) || me->st->done) return;
     const IcpParams p = icp_params_batched(pp);      // thread-local copy: the loops read registers, not shared memory
-    icp_iter_body<MODE>(p);
+    icp_iter_body<MODE, true>(p);
 }
 // batched init: moving source = init * src, state reset, slack from the device-side grid
 __global__ void __launch_bounds__(256) k_icp_init_b(const IcpParams *pp)
@@ -570,6 +722,12 @@ int kp_icp_batch_create(kp_ctx *ctx, const KpIcpPairDesc *pairs, int npairs, int
                             (size_t)ngroups * ICP_NV * sizeof(double) + (size_t)ngroups * sizeof(unsigned int) + sizeof(IcpState) + 1024;
     KP_CUDA(ctx, cudaMalloc(&out->d_work, per_pair * (size_t)npairs));
     KP_CUDA(ctx, cudaMemset(out->d_work, 0, per_pair * (size_t)npairs));
+    if (getenv("KP_DEBUG_ICP")) {
+        // tally of the list-decided and the grid-searched points per pass, summed over every run; printed at destroy
+        const size_t bytes = sizeof(int32_t) * 2 * (size_t)(out->max_iter + 1) * (size_t)npairs;
+        KP_CUDA(ctx, cudaMalloc(&out->d_tally, bytes));
+        KP_CUDA(ctx, cudaMemset(out->d_tally, 0, bytes));
+    }
     std::vector<IcpParams> h((size_t)npairs);
     char *w = (char *)out->d_work;
     auto take = [&](size_t bytes) { char *r = w; w += (bytes + 255) & ~(size_t)255; return r; };
@@ -587,6 +745,8 @@ int kp_icp_batch_create(kp_ctx *ctx, const KpIcpPairDesc *pairs, int npairs, int
         p.r2 = max_corr * max_corr; p.max_corr = max_corr;
         p.max_iter = out->max_iter; p.rel_fit = rel_fitness; p.rel_rmse = rel_rmse;
         p.gdev = pairs[i].tgt_grid; p.ns_dev = pairs[i].n_src; p.src = pairs[i].src; p.vbi = pairs[i].tgt_vbi;
+        p.tlist = pairs[i].tgt_list; p.trho = pairs[i].tgt_rho;
+        p.tally = out->d_tally ? out->d_tally + (size_t)i * 2 * (out->max_iter + 1) : nullptr;
         for (int e = 0; e < 16; ++e) p.init_T[e] = pairs[i].init_T[e];
         p.res_T = pairs[i].res_T; p.res_fit = pairs[i].res_fit; p.res_rmse = pairs[i].res_rmse; p.res_iters = pairs[i].res_iters;
         h[i] = p;
@@ -598,6 +758,18 @@ int kp_icp_batch_create(kp_ctx *ctx, const KpIcpPairDesc *pairs, int npairs, int
 void kp_icp_batch_destroy(KpIcpBatch *b)
 {
     if (!b) return;
+    if (b->d_tally) {
+        const int np = b->max_iter + 1;
+        std::vector<int32_t> t((size_t)2 * np * b->npairs);
+        if (cudaMemcpy(t.data(), b->d_tally, sizeof(int32_t) * t.size(), cudaMemcpyDeviceToHost) == cudaSuccess)
+            for (int i = 0; i < b->npairs; ++i)
+                for (int k = 0; k < np; ++k) {
+                    const int32_t *r = t.data() + ((size_t)i * np + k) * 2;
+                    if (r[0] || r[1]) fprintf(stderr, "[kp icp] pair %d pass %d list %d grid %d\n", i, k, r[0], r[1]);
+                }
+        cudaFree(b->d_tally);
+        b->d_tally = nullptr;
+    }
     if (b->d_params) cudaFree(b->d_params);
     if (b->d_work) cudaFree(b->d_work);
     b->d_params = b->d_work = nullptr;
@@ -611,7 +783,7 @@ int kp_icp_batch_run(kp_ctx *ctx, const KpIcpBatch &b)
     k_icp_init_b<<<dim3((unsigned)(gi > 0 ? gi : 1), (unsigned)b.npairs), 256, 0, ctx->stream>>>(pp);
     KP_LAUNCH_CHECK(ctx);
     for (int i = 0; i <= b.max_iter; ++i) {
-        k_icp_iter_b<ICP_PLANE><<<dim3((unsigned)b.grid, (unsigned)b.npairs), ICP_THREADS, 0, ctx->stream>>>(pp);
+        k_icp_iter_b<ICP_PLANE><<<dim3((unsigned)((b.grid + ICP_B_TILES - 1) / ICP_B_TILES), (unsigned)b.npairs), ICP_THREADS, 0, ctx->stream>>>(pp);
         KP_LAUNCH_CHECK(ctx);
     }
     k_icp_results_b<<<kp_blocks(b.npairs, 64), 64, 0, ctx->stream>>>(pp, b.npairs);
