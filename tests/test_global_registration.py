@@ -188,6 +188,18 @@ def test_gpu_ransac_correspondence_matches_oracle(ctx, oracle):
         assert got["validated"] == ref["validated"] and got["best_iter"] == ref["best_iter"]
         assert abs(got["fitness"] - ref["fitness"]) <= 1.0 / len(cor) and np.abs(got["T"] - ref["T"]).max() < 1e-9
         assert np.abs(got["T"] - D).max() < 2e-2
+    # kp_umeyama on more than three rows, each checker off (edge_sim <= 0, dist_thr <= 0), and the early exit at its
+    # ends: confidence 0 stops after the first valid hypothesis, confidence 1 never stops early
+    for ransac_n, edge_sim, dist_thr, conf, iters in ((4, 0.95, None, 0.999, 50000), (8, 0.95, None, 0.999, 50000),
+                                                      (3, 0.0, None, 0.999, 20000), (4, -1.0, None, 0.999, 20000),
+                                                      (3, 0.95, 0.0, 0.999, 20000), (8, 0.95, -1.0, 0.999, 20000),
+                                                      (3, 0.95, None, 0.0, 20000), (4, 0.95, None, 1.0, 20000)):
+        a = dict(ransac_n=ransac_n, edge_sim=edge_sim, dist_thr=dist_thr, confidence=conf, max_iter=iters, seed=3)
+        ref = oracle.ransac_correspondence(src, tgt, cor, 0.02, **a)
+        got = G.ransac_correspondence(ctx, src, tgt, cor, 0.02, **a)
+        assert got["validated"] == ref["validated"] and got["best_iter"] == ref["best_iter"], a
+        assert abs(got["fitness"] - ref["fitness"]) <= 1.0 / len(cor) and np.abs(got["T"] - ref["T"]).max() < 1e-9, a
+        assert ref["validated"] > 0
     # degenerate inputs
     z = G.ransac_correspondence(ctx, src, tgt, cor[:2], 0.02, max_iter=100)
     assert z["fitness"] == 0 and np.array_equal(z["T"], np.eye(4))
