@@ -333,8 +333,22 @@ typedef struct {
      *     follows `scale`, like floor_band) and is applied with the caller's sign.  Every coefficient must be finite.
      * Create refuses any other floor_mode, and a non-finite coefficient in plane mode (KP_E_ARG). */
     int32_t floor_mode;     double floor_plane[4];
+    /* input of the pipeline:
+     *   KP_INPUT_DEPTH (0, the default): depth images + the xy-table, through kp_pipeline_run / _run_ex / _run_host.
+     *   KP_INPUT_CLOUDS (1): saved point clouds (the fused `.pcd` files a recording left), through kp_pipeline_run_clouds
+     *     only.  A cloud enters the stages from the voxel downsample on; the other entry points refuse such a pipeline and
+     *     kp_pipeline_run_clouds refuses a depth pipeline (KP_E_ARG).  Create needs S = 1, do_icp = 0 and do_crop = 0
+     *     (ICP needs the sensors, the crop the images), else KP_E_ARG; P is the row capacity of one cloud; h_xytab and
+     *     h_T may be NULL; unproject_flags and scale are ignored; every length is in the clouds' own unit.
+     * cloud_voxel (cloud input only; 0 or 1, else KP_E_ARG):
+     *   1: voxel_down_sample(voxel_size) first, as filter_outliers does.
+     *   0: the valid rows go to the SOR / ROR / floor stages as they are, in input order (floor_removal.py has no voxel
+     *      step); voxel_size then only sizes the neighbour-search grids: pass the clouds' typical point spacing.  Every
+     *      search is certified, so it changes the speed, never a result.  n_voxel = n_fused. */
+    int32_t input_mode;     int32_t cloud_voxel;
 } kp_pipeline_cfg;
 enum { KP_FLOOR_RANSAC = 0, KP_FLOOR_PLANE = 1 };
+enum { KP_INPUT_DEPTH = 0, KP_INPUT_CLOUDS = 1 };
 typedef struct {
     int64_t n_fused, n_voxel, n_sor, n_floor_inliers, n_out;
     double icp_T[5][16];    /* refined T_master<-sub_i, i = 1..S-1 */
@@ -374,6 +388,17 @@ KP_EXPORT int kp_pipeline_run_host(kp_pipeline *p, const uint16_t *h_depth, int6
 KP_EXPORT int kp_pipeline_run_ex(kp_pipeline *p, const uint16_t *depth, const uint8_t *rgb, int inputs_on_device, int64_t F,
                                  const int64_t *h_frame_ids, kp_frame_result *h_results, float *d_out_xyz,
                                  int64_t out_stride, float *d_fixed);
+/* the cloud input (cfg.input_mode = KP_INPUT_CLOUDS): F clouds as a CSR batch, cloud f = rows h_offsets[f] ..
+ * h_offsets[f + 1] of xyz float32 [n][3] (inputs_on_device != 0: a device pointer, else a host pointer whose rows are
+ * copied batch by batch); h_offsets int64 [F + 1] on the host.  A row whose x is NaN is absent: it is dropped, the others
+ * keep their order, and n_fused counts the valid rows.  The other arguments and the records are those of
+ * kp_pipeline_run_ex (the ICP fields are 0).  KP_E_ARG before anything is enqueued for decreasing offsets, a negative
+ * first offset, a cloud of more than P rows, or a pipeline built for depth.  The coordinates of a present row must be
+ * finite: a cloud with an infinite bound, or (cloud_voxel = 1) an extent the voxel keys cannot hold, gets status
+ * KP_E_RANGE and an empty result. */
+KP_EXPORT int kp_pipeline_run_clouds(kp_pipeline *p, const float *xyz, const int64_t *h_offsets, int inputs_on_device, int64_t F,
+                                     const int64_t *h_frame_ids, kp_frame_result *h_results, float *d_out_xyz,
+                                     int64_t out_stride, float *d_fixed);
 KP_EXPORT int64_t kp_pipeline_launch_count(kp_pipeline *p);
 /* frames per launch (B) and batch slots in flight (W) the pipeline was built with */
 KP_EXPORT int kp_pipeline_frames_in_flight(kp_pipeline *p, int *batch, int *slots);

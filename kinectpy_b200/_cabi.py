@@ -21,6 +21,7 @@ UNPROJECT_INT16 = 1
 UNPROJECT_DROP_ANY_ZERO = 2
 RESAMPLE_RANDOM, RESAMPLE_PREFIX = 0, 1
 FLOOR_RANSAC, FLOOR_PLANE = 0, 1
+INPUT_DEPTH, INPUT_CLOUDS = 0, 1
 
 
 class KinectPyB200Error(RuntimeError):
@@ -44,6 +45,7 @@ class PipelineCfg(C.Structure):
         ("do_crop", C.c_int32), ("crop_gate", C.c_double), ("resample_n", C.c_int32), ("resample_mode", C.c_int32),
         ("ror_nb_points", C.c_int32), ("ror_radius", C.c_double),
         ("floor_mode", C.c_int32), ("floor_plane", C.c_double * 4),
+        ("input_mode", C.c_int32), ("cloud_voxel", C.c_int32),
     ]
 
 
@@ -121,6 +123,7 @@ SIGNATURES = {
     "kp_pipeline_profile": (C.c_int, [_vp, C.c_int, C.c_int, C.POINTER(C.c_char_p), _pf64, _pi64, _pf64, C.POINTER(C.c_int)]),
     "kp_pipeline_run_host": (C.c_int, [_vp, _vp, _i64, C.POINTER(FrameResult), _vp, _i64]),
     "kp_pipeline_run_ex": (C.c_int, [_vp, _vp, _vp, C.c_int, _i64, _vp, C.POINTER(FrameResult), _vp, _i64, _vp]),
+    "kp_pipeline_run_clouds": (C.c_int, [_vp, _vp, _vp, C.c_int, _i64, _vp, C.POINTER(FrameResult), _vp, _i64, _vp]),
 }
 
 _lib = None

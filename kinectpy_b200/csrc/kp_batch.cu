@@ -55,6 +55,10 @@ struct FMask {
     const uint8_t *mask; int64_t stride; int invert;
     __device__ bool operator()(int seg, int64_t i) const { return (mask[seg * stride + i] != 0) != (invert != 0); }
 };
+struct FValid {                 // rows whose x is not NaN (kp_b_compact_rows without a mask)
+    const float *in; int64_t stride;
+    __device__ bool operator()(int seg, int64_t i) const { return !isnan(in[3 * (seg * stride + i)]); }
+};
 struct FRunHead {
     const uint32_t *keys; int64_t stride;
     __device__ bool operator()(int seg, int64_t i) const
@@ -347,6 +351,7 @@ int kp_b_compact_rows(const BLaunch &L, const BScan &S, DCnt n, const uint8_t *m
                       const float *in, float *out, int64_t row_stride, DOut total, const uint32_t *aux_in, uint32_t *aux_out)
 {
     KP_PROFB(L.ctx, "compact_rows", 0.0);
+    if (!mask) return bc_run(L, S, n, FValid{in, row_stride}, ERows{in, out, row_stride, aux_in, aux_out}, total);
     return bc_run(L, S, n, FMask{mask, mask_stride, invert}, ERows{in, out, row_stride, aux_in, aux_out}, total);
 }
 int kp_b_partition_rows(const BLaunch &L, const BScan &S, DCnt n, const uint8_t *mask, int64_t mask_stride, const float *in,

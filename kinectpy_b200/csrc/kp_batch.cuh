@@ -59,7 +59,8 @@ struct BScan {
 };
 
 // ---- compaction family (count + last-CTA scan, then scatter): no CTA ever waits for another one
-// rows of `in` whose mask byte (xor invert) is set -> packed into `out`; total[seg] = rows kept
+// rows of `in` whose mask byte (xor invert) is set -> packed into `out`; total[seg] = rows kept.  mask NULL: the rows whose
+// x is not NaN
 // aux_in / aux_out (nullable): a 4-byte payload per row (its packed voxel coordinates) that travels with the row
 int kp_b_compact_rows(const BLaunch &L, const BScan &S, DCnt n, const uint8_t *mask, int64_t mask_stride, int invert,
                       const float *in, float *out, int64_t row_stride, DOut total, const uint32_t *aux_in = nullptr,

@@ -21,6 +21,8 @@ int kp_unproject_engine(kp_ctx *ctx, const uint16_t *d_depth, const float *d_xyt
                         int flags, double scale, float *d_xyz, float *d_xyz_raw, int32_t *d_slots, int32_t *d_rows,
                         const uint8_t *d_rgb, const double *d_crop_med, double crop_gate);
 size_t kp_unproject_engine_slots(int B, int S, int64_t P);
+int kp_load_clouds_engine(kp_ctx *ctx, const float *d_xyz, const int64_t *h_off, int B, int64_t P, int64_t stride, int nan_fill,
+                          float *d_out, int32_t *d_slots, int32_t *d_rows, int32_t *d_nrows);
 int kp_crop_median_engine(kp_ctx *ctx, const uint16_t *d_depth, const uint32_t *d_vbits, int B, int S, int64_t P, uint32_t *d_hist,
                           double *d_med);
 size_t kp_crop_median_hist_elems();
@@ -99,6 +101,7 @@ __device__ void vox_setup(const float *b6, int nvalid, double voxel, KpVoxDev &v
 struct SetupParams {
     EngDyn *dyn; EngCloud *icl; const int32_t *rows;     // K1 bounds rows [B][S][2][8]
     int S; double voxel, icp_voxel; int do_icp;     // do_icp: the rows carry a second set (the ICP inputs)
+    int no_voxel;                                   // cloud input without a downsample: no voxel grid decides validity
 };
 __global__ void k_e_frame_setup(const __grid_constant__ SetupParams p, int B)
 {
@@ -122,7 +125,17 @@ __global__ void k_e_frame_setup(const __grid_constant__ SetupParams p, int B)
     }
     int32_t status = KP_OK;
     for (int c = 0; c < 6; ++c) d.b6[c] = b6[c];
-    vox_setup(b6, nvalid, p.voxel, d.vox_fused, status);
+    bool ok;
+    if (p.no_voxel) {
+        // (a tiny voxel_size only makes the neighbour grids coarser); the grids need finite bounds
+        ok = nvalid > 0;
+        for (int c = 0; c < 6; ++c) ok = ok && isfinite(b6[c]);
+        if (nvalid > 0 && !ok) status = KP_E_RANGE;
+        d.vox_fused.ok = 0;
+    } else {
+        vox_setup(b6, nvalid, p.voxel, d.vox_fused, status);
+        ok = d.vox_fused.ok;
+    }
     d.n_fused = nvalid;
     for (int s = 0; s < p.S && p.do_icp; ++s) {
         const int32_t *r = rows + (size_t)(2 * s + 1) * 8;
@@ -134,7 +147,7 @@ __global__ void k_e_frame_setup(const __grid_constant__ SetupParams p, int B)
         if (p.do_icp) vox_setup(cl.b6, r[6], p.icp_voxel, cl.vox, status);
         if (!cl.vox.ok) cl.nv = 0;
     }
-    if (!d.vox_fused.ok) d.n_fused = 0;      // empty or out of range: every later stage sees an empty cloud
+    if (!ok) d.n_fused = 0;                  // empty or out of range: every later stage sees an empty cloud
     d.status = status;
 }
 
@@ -1222,6 +1235,8 @@ struct EngSlot {
     std::vector<void *> allocs;
     // K1
     uint16_t *d_depth = nullptr;                      // staging for host depth [B][S][P]
+    float *cl_in = nullptr;                           // cloud input: staging for a batch's host rows [B * P][3]
+    int32_t *cl_rows = nullptr;                       // cloud input: rows of each cloud of the batch [B]
     uint8_t *d_rgb = nullptr;                         // crop: staging for host segmentation images [B][S][P][3]
     uint32_t *crop_hist = nullptr;                    // crop: median-pass histograms [B*S][...] (zero between calls)
     double *crop_med = nullptr;                       // crop: median of every (frame, sensor) of the last batch [B][S]
@@ -1281,6 +1296,8 @@ struct kp_pipeline {
     int64_t cap_cells = 1 << 25;
     int64_t cap_bricks = 1 << 23;
     int64_t NPr = 0, Pr = 0;          // row strides of the engine's own arrays: S*P and P rounded up to 64 (aligned vector access)
+    int64_t fstride = 0;              // row stride of the fused clouds: S*P (K1 writes them), NPr for the cloud input
+    bool clouds = false;              // cfg.input_mode == KP_INPUT_CLOUDS
     bool use_graph = true, profiling = false, use_vbi_icp = false, use_vbi_knn = false;
     bool icp_lists = true;            // ICP passes take the partner from the target's neighbour lists where they decide it (KP_ICP_LISTS)
     double rho_mult_a = 1.15, rho_mult_b = 2.0;
@@ -1744,7 +1761,12 @@ int slot_create(kp_pipeline *pl, EngSlot &s)
     PL_CUDA(pl, cudaEventCreateWithFlags(&s.ev_join, cudaEventDisableTiming));
 #define SA(ptr, count) KP_TRY(slot_alloc(pl, s, (size_t)(count), &(ptr)))
 #define SAZ(ptr, count) KP_TRY(slot_alloc(pl, s, (size_t)(count), &(ptr), true))
-    SAZ(s.d_depth, B * NP);
+    if (pl->clouds) {
+        SA(s.cl_in, B * P * 3);
+        SAZ(s.cl_rows, B);
+    } else {
+        SAZ(s.d_depth, B * NP);
+    }
     if (c.do_crop) {
         SAZ(s.d_rgb, B * NP * 3);
         SAZ(s.crop_hist, (size_t)B * S * kp_crop_median_hist_elems());
@@ -1761,7 +1783,7 @@ int slot_create(kp_pipeline *pl, EngSlot &s)
     }
     SA(s.k1_slots, kp_unproject_engine_slots(B, S, P));
     SAZ(s.k1_rows, (size_t)B * S * 2 * 8);
-    SA(s.fused, B * NP * 3);
+    SA(s.fused, B * pl->fstride * 3);
     SAZ(s.dyn, B);
     SAZ(s.icl, (size_t)B * S);
     SAZ(s.d_res, B);
@@ -1904,7 +1926,7 @@ int enqueue_core(kp_pipeline *pl, EngSlot &s, bool fork)
     const bool icp = c.do_icp && S > 1;
     kp_ctx *ctx = s.ctx;
     {
-        SetupParams sp{s.dyn, s.icl, s.k1_rows, S, c.voxel_size, c.icp_voxel, icp ? 1 : 0};
+        SetupParams sp{s.dyn, s.icl, s.k1_rows, S, c.voxel_size, c.icp_voxel, icp ? 1 : 0, pl->clouds && !c.cloud_voxel};
         k_e_frame_setup<<<kp_blocks(B, 32), 32, 0, ctx->stream>>>(sp, B);
         KP_LAUNCH_CHECK(ctx);
     }
@@ -1915,9 +1937,14 @@ int enqueue_core(kp_pipeline *pl, EngSlot &s, bool fork)
         KP_CUDA(ctx, cudaStreamWaitEvent(s.aux->stream, s.ev_fork, 0));
     }
     if (icp && fork) KP_TRY(stage_icp(pl, s, ictx));      // enqueued first so that its small kernels interleave with the main branch
-    // ---- filter_outliers: voxel + SOR
-    KP_TRY(stage_voxel(pl, ctx, B, NP, s.fused, NP, &s.dyn->vox_fused, sizeof(EngDyn), DYN_CNT(s, n_fused), s.keys, s.keys_tmp, s.vals,
-                       s.vals_tmp, NPr, s.sortw, s.scan, s.run_start, NPr + 64, s.A, NPr, DYN_OUT(s, n_voxel), s.vA));
+    // ---- filter_outliers: voxel + SOR (cloud input without a downsample: the load stage compacted the rows into A)
+    if (pl->clouds && !c.cloud_voxel) {
+        k_e_copy_cnt<<<kp_blocks(B, 64), 64, 0, ctx->stream>>>(DYN_CNT(s, n_fused), DYN_OUT(s, n_voxel), B);
+        KP_LAUNCH_CHECK(ctx);
+    } else {
+        KP_TRY(stage_voxel(pl, ctx, B, NP, s.fused, pl->fstride, &s.dyn->vox_fused, sizeof(EngDyn), DYN_CNT(s, n_fused), s.keys, s.keys_tmp,
+                           s.vals, s.vals_tmp, NPr, s.sortw, s.scan, s.run_start, NPr + 64, s.A, NPr, DYN_OUT(s, n_voxel), s.vA));
+    }
     const float *sor_out = s.A;
     const uint32_t *v_sor_out = s.vA;
     if (c.sor_k > 0) {
@@ -1979,10 +2006,45 @@ int enqueue_k1(kp_pipeline *p, EngSlot &s, const uint16_t *d_depth, const uint8_
                                s.crop_med, c.crop_gate);
 }
 
-int run_impl(kp_pipeline *p, const uint16_t *depth, const uint8_t *rgb, int depth_on_device, int64_t F, const int64_t *h_frame_ids,
-             kp_frame_result *h_results, float *out_xyz, int64_t out_stride, float *d_fixed)
+// the load stage of a cloud batch (outside the graph, where K1 runs for depth): frame b = rows off[b] .. off[b + 1] of
+// d_xyz, b < nf; the frames beyond nf get empty clouds.  Without a downsample the valid rows are compacted into A here.
+int enqueue_load(kp_pipeline *p, EngSlot &s, const float *d_xyz, const int64_t *off, int nf)
 {
-    if (!p || !h_results || F < 0 || (F > 0 && !depth)) return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_run: bad argument");
+    const kp_pipeline_cfg &c = p->cfg;
+    const int B = p->B;
+    int64_t rel[17];
+    for (int b = 0; b <= B; ++b) rel[b] = off[b < nf ? b : nf] - off[0];
+    KP_TRY(kp_load_clouds_engine(s.ctx, d_xyz, rel, B, c.P, p->fstride, c.cloud_voxel, s.fused, s.k1_slots, s.k1_rows, s.cl_rows));
+    if (c.cloud_voxel) return KP_OK;
+    BLaunch L{s.ctx, B, p->NPr, ctas_for(p, 4)};
+    return kp_b_compact_rows(L, s.scan, DCnt{s.cl_rows, 1}, nullptr, 0, 0, s.fused, s.A, p->NPr, DOut{s.sink, 1});
+}
+
+// depth (depth, rgb) or clouds (xyz, h_offsets) in, one entry each
+int run_impl(kp_pipeline *p, const uint16_t *depth, const uint8_t *rgb, const float *xyz, const int64_t *h_offsets, int depth_on_device,
+             int64_t F, const int64_t *h_frame_ids, kp_frame_result *h_results, float *out_xyz, int64_t out_stride, float *d_fixed)
+{
+    const bool clouds = h_offsets != nullptr;
+    if (!p || !h_results || F < 0 || (F > 0 && !(clouds ? (const void *)xyz : (const void *)depth)))
+        return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_run: bad argument");
+    if (clouds != p->clouds) {
+        p->err = p->clouds ? "kp_pipeline_run: this pipeline takes point clouds (kp_pipeline_run_clouds)"
+                           : "kp_pipeline_run_clouds: this pipeline takes depth images (kp_pipeline_run / _run_ex)";
+        return KP_E_ARG;
+    }
+    if (clouds) {
+        if (h_offsets[0] < 0) { p->err = "kp_pipeline_run_clouds: negative first offset"; return KP_E_ARG; }
+        for (int64_t f = 0; f < F; ++f) {
+            const int64_t n = h_offsets[f + 1] - h_offsets[f];
+            if (n < 0 || n > p->cfg.P) {
+                char buf[160];
+                snprintf(buf, sizeof buf, "kp_pipeline_run_clouds: cloud %lld has %lld rows (offsets must not decrease; at most P = %lld rows)",
+                         (long long)f, (long long)n, (long long)p->cfg.P);
+                p->err = buf;
+                return KP_E_ARG;
+            }
+        }
+    }
     if (out_xyz && out_stride <= 0) { p->err = "kp_pipeline_run: out_stride must be > 0 when an output buffer is given"; return KP_E_ARG; }
     if (F > 0 && !rgb != !p->cfg.do_crop) {
         p->err = p->cfg.do_crop ? "kp_pipeline_run: this pipeline crops: it needs the segmentation images (rgb)"
@@ -2009,20 +2071,32 @@ int run_impl(kp_pipeline *p, const uint16_t *depth, const uint8_t *rgb, int dept
         kp_ctx *ctx = s.ctx;
         const int64_t f0 = i * B;
         const int nf = (int)(F - f0 < B ? F - f0 : B);
-        const uint16_t *d_depth = depth + f0 * NP;
-        const uint8_t *d_rgb = rgb ? rgb + 3 * f0 * NP : nullptr;
-        if (!depth_on_device) {
-            PL_CUDA(p, cudaMemcpyAsync(s.d_depth, depth + f0 * NP, sizeof(uint16_t) * (size_t)nf * NP, cudaMemcpyHostToDevice, ctx->stream));
-            d_depth = s.d_depth;
-            if (rgb) {
-                PL_CUDA(p, cudaMemcpyAsync(s.d_rgb, d_rgb, 3 * (size_t)nf * NP, cudaMemcpyHostToDevice, ctx->stream));
-                d_rgb = s.d_rgb;
+        int rc;
+        if (clouds) {
+            const float *d_xyz = xyz + 3 * h_offsets[f0];
+            const int64_t rows = h_offsets[f0 + nf] - h_offsets[f0];
+            if (!depth_on_device && rows > 0) {
+                PL_CUDA(p, cudaMemcpyAsync(s.cl_in, d_xyz, 12 * (size_t)rows, cudaMemcpyHostToDevice, ctx->stream));
+                d_xyz = s.cl_in;
             }
+            rc = enqueue_load(p, s, d_xyz, h_offsets + f0, nf);
+            if (rc != KP_OK) { p->err = ctx->err; return rc; }
+        } else {
+            const uint16_t *d_depth = depth + f0 * NP;
+            const uint8_t *d_rgb = rgb ? rgb + 3 * f0 * NP : nullptr;
+            if (!depth_on_device) {
+                PL_CUDA(p, cudaMemcpyAsync(s.d_depth, depth + f0 * NP, sizeof(uint16_t) * (size_t)nf * NP, cudaMemcpyHostToDevice, ctx->stream));
+                d_depth = s.d_depth;
+                if (rgb) {
+                    PL_CUDA(p, cudaMemcpyAsync(s.d_rgb, d_rgb, 3 * (size_t)nf * NP, cudaMemcpyHostToDevice, ctx->stream));
+                    d_rgb = s.d_rgb;
+                }
+            }
+            // frames of a short last batch beyond nf: empty bounds rows -> empty clouds, every stage is a no-op for them
+            if (nf < B) PL_CUDA(p, cudaMemsetAsync(s.k1_rows, 0, sizeof(int32_t) * (size_t)B * S * 2 * 8, ctx->stream));
+            rc = enqueue_k1(p, s, d_depth, d_rgb, nf);
+            if (rc != KP_OK) { p->err = ctx->err; return rc; }
         }
-        // frames of a short last batch beyond nf: empty bounds rows -> empty clouds, every stage is a no-op for them
-        if (nf < B) PL_CUDA(p, cudaMemsetAsync(s.k1_rows, 0, sizeof(int32_t) * (size_t)B * S * 2 * 8, ctx->stream));
-        int rc = enqueue_k1(p, s, d_depth, d_rgb, nf);
-        if (rc != KP_OK) { p->err = ctx->err; return rc; }
         if (direct) {
             rc = enqueue_core(p, s, !p->profiling);
             if (rc != KP_OK) { p->err = ctx->err.empty() ? s.aux->err : ctx->err; return rc; }
@@ -2083,7 +2157,11 @@ extern "C" {
 
 int kp_pipeline_create(int device, const kp_pipeline_cfg *cfg, const float *h_xytab, const double *h_T, kp_pipeline **out)
 {
-    if (!cfg || !h_xytab || !out) return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: NULL argument");
+    if (!cfg || !out || (!h_xytab && cfg->input_mode != KP_INPUT_CLOUDS)) return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: NULL argument");
+    if (cfg->input_mode != KP_INPUT_DEPTH && cfg->input_mode != KP_INPUT_CLOUDS)
+        return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: input_mode must be KP_INPUT_DEPTH or KP_INPUT_CLOUDS (got %d)", cfg->input_mode);
+    if (cfg->input_mode == KP_INPUT_CLOUDS && (cfg->S != 1 || cfg->do_icp || cfg->do_crop || (cfg->cloud_voxel != 0 && cfg->cloud_voxel != 1)))
+        return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: the cloud input needs S = 1, do_icp = 0, do_crop = 0 and cloud_voxel 0 or 1");
     if (cfg->S < 1 || cfg->S > ENG_MAX_S || cfg->P < 1) return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: need 1..6 sensors and P >= 1");
     if (!(cfg->voxel_size > 0.0)) return kp_set_err(nullptr, KP_E_ARG, "kp_pipeline_create: voxel_size <= 0");
     if (cfg->floor_mode != KP_FLOOR_RANSAC && cfg->floor_mode != KP_FLOOR_PLANE)
@@ -2132,6 +2210,8 @@ int kp_pipeline_create(int device, const kp_pipeline_cfg *cfg, const float *h_xy
     // the lists come from the normals search on the target grid, which the voxel-brick index replaces
     p->icp_lists = !(getenv("KP_ICP_LISTS") && atoi(getenv("KP_ICP_LISTS")) == 0) && !p->use_vbi_icp;
     p->use_vbi_knn = getenv("KP_KNN_VBI") && atoi(getenv("KP_KNN_VBI")) != 0;   // measured slower than the grid level 0: off unless asked for
+    p->clouds = cfg->input_mode == KP_INPUT_CLOUDS;
+    if (p->clouds && !cfg->cloud_voxel) p->use_vbi_knn = false;      // (the index needs the packed voxel coordinates of a downsample)
     p->knn_rad = (getenv("KP_KNN_RAD") && atoi(getenv("KP_KNN_RAD")) == 2) ? 2 : 1;
     if (getenv("KP_KNN_MID")) p->knn_mid = atof(getenv("KP_KNN_MID"));
     if (getenv("KP_VBI_RHO_A")) p->rho_mult_a = atof(getenv("KP_VBI_RHO_A"));
@@ -2146,6 +2226,7 @@ int kp_pipeline_create(int device, const kp_pipeline_cfg *cfg, const float *h_xy
     p->cap_bricks = bricks;
     p->NPr = ((int64_t)NP + 63) & ~(int64_t)63;
     p->Pr = (cfg->P + 63) & ~(int64_t)63;
+    p->fstride = p->clouds ? p->NPr : (int64_t)NP;
     p->T_fuse.assign(16 * S, 0.0);
     p->T_icp.assign(16 * S, 0.0);
     for (int s = 0; s < S; ++s)
@@ -2159,8 +2240,10 @@ int kp_pipeline_create(int device, const kp_pipeline_cfg *cfg, const float *h_xy
         kp_pipeline_destroy(p);
         return kp_set_err(nullptr, rc, "kp_pipeline_create: %s", m.c_str());
     };
-    if (cudaMalloc((void **)&p->d_tab, sizeof(float) * 2 * NP) != cudaSuccess) { p->err = "table allocation failed"; return fail(KP_E_NOMEM); }
-    if (cudaMemcpy(p->d_tab, h_xytab, sizeof(float) * 2 * NP, cudaMemcpyHostToDevice) != cudaSuccess) { p->err = "table copy failed"; return fail(KP_E_CUDA); }
+    if (!p->clouds) {
+        if (cudaMalloc((void **)&p->d_tab, sizeof(float) * 2 * NP) != cudaSuccess) { p->err = "table allocation failed"; return fail(KP_E_NOMEM); }
+        if (cudaMemcpy(p->d_tab, h_xytab, sizeof(float) * 2 * NP, cudaMemcpyHostToDevice) != cudaSuccess) { p->err = "table copy failed"; return fail(KP_E_CUDA); }
+    }
     if (cfg->do_crop) {
         // the crop median counts a pixel outside the table as z = 0: which pixels those are, one bit each
         const int64_t words = (cfg->P + 31) / 32;
@@ -2181,7 +2264,8 @@ int kp_pipeline_create(int device, const kp_pipeline_cfg *cfg, const float *h_xy
     // One untimed pass over empty frames per slot: loads every kernel outside a capture and proves the launch
     // sequence on the degenerate input; then the sequence is captured as the slot's graph.
     for (auto &s : p->slots) {
-        int rc = enqueue_k1(p, s, s.d_depth, s.d_rgb, B);
+        const int64_t none[1] = {0};
+        int rc = p->clouds ? enqueue_load(p, s, s.cl_in, none, 0) : enqueue_k1(p, s, s.d_depth, s.d_rgb, B);
         if (rc == KP_OK) rc = enqueue_core(p, s, true);
         if (rc != KP_OK) { p->err = s.ctx->err.empty() ? s.aux->err : s.ctx->err; return fail(rc); }
         if (cudaStreamSynchronize(s.ctx->stream) != cudaSuccess || cudaStreamSynchronize(s.aux->stream) != cudaSuccess) {
@@ -2216,13 +2300,20 @@ const char *kp_pipeline_last_error(kp_pipeline *p) { return p ? p->err.c_str() :
 int kp_pipeline_run(kp_pipeline *p, const uint16_t *depth, int depth_on_device, int64_t F, kp_frame_result *h_results,
                     float *d_out_xyz, int64_t out_stride)
 {
-    return run_impl(p, depth, nullptr, depth_on_device, F, nullptr, h_results, d_out_xyz, out_stride, nullptr);
+    return run_impl(p, depth, nullptr, nullptr, nullptr, depth_on_device, F, nullptr, h_results, d_out_xyz, out_stride, nullptr);
 }
 
 int kp_pipeline_run_ex(kp_pipeline *p, const uint16_t *depth, const uint8_t *rgb, int inputs_on_device, int64_t F,
                        const int64_t *h_frame_ids, kp_frame_result *h_results, float *d_out_xyz, int64_t out_stride, float *d_fixed)
 {
-    return run_impl(p, depth, rgb, inputs_on_device, F, h_frame_ids, h_results, d_out_xyz, out_stride, d_fixed);
+    return run_impl(p, depth, rgb, nullptr, nullptr, inputs_on_device, F, h_frame_ids, h_results, d_out_xyz, out_stride, d_fixed);
+}
+
+int kp_pipeline_run_clouds(kp_pipeline *p, const float *xyz, const int64_t *h_offsets, int inputs_on_device, int64_t F,
+                           const int64_t *h_frame_ids, kp_frame_result *h_results, float *d_out_xyz, int64_t out_stride, float *d_fixed)
+{
+    if (p && !h_offsets) { p->err = "kp_pipeline_run_clouds: NULL offsets"; return KP_E_ARG; }
+    return run_impl(p, nullptr, nullptr, xyz, h_offsets, inputs_on_device, F, h_frame_ids, h_results, d_out_xyz, out_stride, d_fixed);
 }
 
 int kp_pipeline_run_host(kp_pipeline *p, const uint16_t *h_depth, int64_t F, kp_frame_result *h_results, float *h_out_xyz,
@@ -2238,7 +2329,7 @@ int kp_pipeline_run_host(kp_pipeline *p, const uint16_t *h_depth, int64_t F, kp_
             return KP_E_ARG;
         }
     }
-    return run_impl(p, h_depth, nullptr, 0, F, nullptr, h_results, h_out_xyz, out_stride, nullptr);
+    return run_impl(p, h_depth, nullptr, nullptr, nullptr, 0, F, nullptr, h_results, h_out_xyz, out_stride, nullptr);
 }
 
 int64_t kp_pipeline_launch_count(kp_pipeline *p)

@@ -345,6 +345,104 @@ __global__ void __launch_bounds__(256) k_bounds_fold(const int32_t *slots, int64
     }
 }
 
+// ---- cloud input of the frame engine: the load stage in place of K1
+// Frame f of the batch is rows off[f] .. off[f + 1] of `xyz` (a CSR batch of float32 [n][3] clouds).  CTA (tile, f) owns
+// rows [2048 tile, 2048 tile + 2048) of the frame, a warp 256 consecutive rows, a lane 8.  A warp's rows are 768
+// consecutive floats that start at any 4-byte offset (a CSR start is a multiple of 12 bytes, and the caller's pointer
+// need not be 16-byte aligned): the warp reads the 16-byte-aligned float4s that cover them, coalesced, through the
+// warp-private stage of up_store_rows (a float4 that is not wholly inside the warp's rows is read float by float, so
+// nothing outside the cloud is touched), then every lane takes its 8 rows from the stage.  Bounds and count of the
+// valid rows (x not NaN) go to the warp's slot in K1's format, which k_bounds_fold folds per frame; no atomics.
+constexpr int CL_MAX_B = 16;
+struct CloudLoadParams {
+    const float *xyz;
+    int64_t off[CL_MAX_B + 1];     // rows relative to xyz; a frame beyond the batch's clouds has an empty range
+    int64_t P;                     // capacity (rows) of one cloud
+    int64_t stride;                // rows between the frames' output segments (a multiple of 64)
+    int nan_fill;                  // 1: rows [n_f, P) of the segment are set to NaN (the voxel keys read all P rows)
+    float *out;                    // [B][stride][3]
+    int32_t *slots;                // [B][tiles][8 warps][8]
+    int32_t *n_rows;               // [B]: rows of each cloud, valid or not
+};
+__global__ void __launch_bounds__(UP_THREADS) k_e_load_clouds(const __grid_constant__ CloudLoadParams p)
+{
+    __shared__ float stage_s[UP_THREADS / 32][32 * 25];
+    const int f = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int64_t lo = p.off[f], n = p.off[f + 1] - lo;
+    const int64_t w0 = (int64_t)blockIdx.x * UP_TILE + (int64_t)warp * (32 * UP_PPT);       // the warp's first row
+    const int nrw = (int)max((int64_t)0, min((int64_t)(32 * UP_PPT), n - w0));              // its rows of the cloud
+    float *stage = stage_s[warp];
+    if (blockIdx.x == 0 && tid == 0) p.n_rows[f] = (int32_t)n;
+    float v[UP_PPT * 3];
+    if (nrw > 0) {
+        const float *src = p.xyz + 3 * (lo + w0);
+        const int mis = (int)((((uintptr_t)src) >> 2) & 3u);          // floats between the aligned float4 and src
+        const float4 *a4 = reinterpret_cast<const float4 *>(src - mis);
+        const int nf = 3 * nrw;
+#pragma unroll
+        for (int k = 0; k < 7; ++k) {                                   // 7 x 32 float4 cover 768 + 3 floats
+            const int q = 32 * k + lane, e0 = 4 * q - mis;              // first float of this float4, relative to src
+            if (e0 >= nf || e0 + 4 <= 0) continue;
+            float t[4];
+            if (e0 >= 0 && e0 + 4 <= nf) {
+                const float4 x = __ldg(a4 + q);
+                t[0] = x.x; t[1] = x.y; t[2] = x.z; t[3] = x.w;
+            } else {
+#pragma unroll
+                for (int c = 0; c < 4; ++c) t[c] = (e0 + c >= 0 && e0 + c < nf) ? __ldg(src + e0 + c) : 0.0f;
+            }
+#pragma unroll
+            for (int c = 0; c < 4; ++c) {
+                const int e = e0 + c;
+                if (e >= 0 && e < nf) stage[(e / 24) * 25 + e % 24] = t[c];
+            }
+        }
+        __syncwarp();
+#pragma unroll
+        for (int j = 0; j < UP_PPT * 3; ++j) v[j] = stage[lane * 25 + j];
+        __syncwarp();
+    }
+    float mn[3] = {INFINITY, INFINITY, INFINITY}, mx[3] = {-INFINITY, -INFINITY, -INFINITY};
+    int cnt = 0;
+#pragma unroll
+    for (int j = 0; j < UP_PPT; ++j) {
+        if (lane * UP_PPT + j < nrw) {
+            if (!isnan(v[3 * j])) {
+                ++cnt;
+#pragma unroll
+                for (int c = 0; c < 3; ++c) { mn[c] = fminf(mn[c], v[3 * j + c]); mx[c] = fmaxf(mx[c], v[3 * j + c]); }
+            }
+        } else {
+            v[3 * j] = v[3 * j + 1] = v[3 * j + 2] = NAN;
+        }
+    }
+    // rows out: the cloud's rows, and with nan_fill NaN up to P
+    const int nout = p.nan_fill ? (int)max((int64_t)0, min((int64_t)(32 * UP_PPT), p.P - w0)) : nrw;
+    float *dst = p.out + 3 * ((int64_t)f * p.stride + w0);
+    if (nout == 32 * UP_PPT) {
+        up_store_rows(stage, v, dst, lane);
+    } else {
+#pragma unroll
+        for (int j = 0; j < UP_PPT; ++j)
+            if (lane * UP_PPT + j < nout) {
+                float *o = dst + 3 * (lane * UP_PPT + j);
+                o[0] = v[3 * j]; o[1] = v[3 * j + 1]; o[2] = v[3 * j + 2];
+            }
+    }
+    int enc[7] = {kp_f2ord(mn[0]), kp_f2ord(mn[1]), kp_f2ord(mn[2]), kp_f2ord(mx[0]), kp_f2ord(mx[1]), kp_f2ord(mx[2]), cnt};
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        enc[c] = __reduce_min_sync(KP_FULL, enc[c]);
+        enc[3 + c] = __reduce_max_sync(KP_FULL, enc[3 + c]);
+    }
+    enc[6] = __reduce_add_sync(KP_FULL, enc[6]);
+    if (lane == 0) {
+        int4 *slot = reinterpret_cast<int4 *>(p.slots) + 2 * (((int64_t)f * gridDim.x + blockIdx.x) * (UP_THREADS / 32) + warp);
+        slot[0] = make_int4(enc[0], enc[1], enc[2], enc[3]);
+        slot[1] = make_int4(enc[4], enc[5], enc[6], 0);
+    }
+}
+
 __global__ void k_bounds_decode_batch(const int32_t *enc, int B, float *bounds, int32_t *nvalid)
 {
     int b = blockIdx.x * blockDim.x + threadIdx.x;
@@ -660,6 +758,30 @@ int kp_unproject_engine(kp_ctx *ctx, const uint16_t *d_depth, const float *d_xyt
 size_t kp_unproject_engine_slots(int B, int S, int64_t P)
 {
     return (size_t)B * S * 2 * kp_blocks(P, UP_TILE) * (UP_THREADS / 32) * 8;
+}
+
+// frame engine, cloud input: frame f of the batch = rows h_off[f] .. h_off[f + 1] of d_xyz (h_off [B + 1] on the host,
+// relative to d_xyz) -> segment f of d_out (row stride `stride`, NaN over rows [n_f, P) with nan_fill), bounds rows
+// [B][8] in K1's layout, d_nrows [B].  d_slots: kp_unproject_engine_slots(B, 1, P) int32 scratch.
+int kp_load_clouds_engine(kp_ctx *ctx, const float *d_xyz, const int64_t *h_off, int B, int64_t P, int64_t stride, int nan_fill,
+                          float *d_out, int32_t *d_slots, int32_t *d_rows, int32_t *d_nrows)
+{
+    if (B <= 0 || P <= 0) return KP_OK;
+    if (B > CL_MAX_B) return kp_set_err(ctx, KP_E_ARG, "frame engine: at most %d clouds per batch (got %d)", CL_MAX_B, B);
+    const int64_t rows = h_off[B] - h_off[0];
+    const int64_t ntiles = kp_blocks(P, UP_TILE);
+    // algorithmic bytes: the rows in, the rows (and the NaN fill) out, one 32-byte slot per warp, the row counts
+    KP_PROFB(ctx, "cloud_load", (double)rows * 12.0 + (nan_fill ? (double)B * P : (double)rows) * 12.0 +
+                                    (double)B * ntiles * (UP_THREADS / 32) * 32.0 + (double)B * 4.0);
+    CloudLoadParams p;
+    p.xyz = d_xyz;
+    for (int f = 0; f <= CL_MAX_B; ++f) p.off[f] = h_off[f < B ? f : B];
+    p.P = P; p.stride = stride; p.nan_fill = nan_fill; p.out = d_out; p.slots = d_slots; p.n_rows = d_nrows;
+    k_e_load_clouds<<<dim3((unsigned)ntiles, (unsigned)B), UP_THREADS, 0, ctx->stream>>>(p);
+    KP_LAUNCH_CHECK(ctx);
+    k_bounds_fold<<<B, 256, 0, ctx->stream>>>(d_slots, ntiles * (UP_THREADS / 32), d_rows);
+    KP_LAUNCH_CHECK(ctx);
+    return KP_OK;
 }
 
 // frame engine: crop medians d_med [B][S] of the batch's depth (d_vbits [S][(P + 31) / 32]: finite table entries;

@@ -4,7 +4,8 @@
 per-point Python loop of ``pcd_above_plane`` (``floor_removal.py:42-48``) becomes one mask kernel
 plus an ordered compaction.  ``remove_floor`` is the body of the script's loop
 (``floor_removal.py:64-73``) as a function: floor band by max-y, RANSAC plane on the band, keep the
-band's non-plane points, merge with the upper part, statistical outlier removal.
+band's non-plane points, merge with the upper part, statistical outlier removal.  ``remove_floor_batch``
+runs that body over a list of clouds in one batched frame-engine pipeline.
 """
 from __future__ import annotations
 
@@ -14,7 +15,7 @@ import os
 
 import numpy as np
 
-from . import _cabi
+from . import _cabi, geometry
 from .geometry import PointCloud
 from .io_formats import read_point_cloud, write_point_cloud
 
@@ -77,6 +78,33 @@ def remove_floor(pcd: PointCloud, band: float = 200, distance_threshold: float =
     if return_details:
         return filtered, plane_model, inliers
     return filtered
+
+
+def remove_floor_batch(pcds, band: float = 200, distance_threshold: float = 30, ransac_n: int = 30, num_iterations: int = 2000,
+                       nb_neighbors: int = 50, std_ratio: float = 0.30, seed=None, spacing: float = 10.0, n_streams: int = 16):
+    """``remove_floor`` over a list of clouds in one batched frame-engine pipeline (cloud input, no voxel step): the same
+    literals, the same results, without a host round trip per cloud.  ``spacing``: the clouds' typical point spacing in
+    their unit (millimetres for the literals above); it sizes the neighbour-search grids only, never a result.  A cloud
+    with fewer than ``ransac_n`` points is returned as it is (the engine's floor-skip rule), and a band of fewer than
+    ``ransac_n`` points has no plane (nothing is removed from it).  Returns a list of ``PointCloud``."""
+    from .pipeline import FramePipeline, PipelineConfig
+    if nb_neighbors < 1 or not std_ratio > 0:
+        raise _cabi.KinectPyB200Error(_cabi.KP_E_ARG, "nb_neighbors < 1 or std_ratio <= 0")
+    pcds = list(pcds)
+    if not pcds:
+        return []
+    cap = max(max(len(p) for p in pcds), 1)
+    cfg = PipelineConfig(input_mode=_cabi.INPUT_CLOUDS, cloud_voxel=0, n_sensors=1, pixels=cap, scale=1.0, voxel_size=float(spacing),
+                         sor_k=0, do_floor=True, floor_band=float(band), ransac_thr=float(distance_threshold),
+                         ransac_n=int(ransac_n), ransac_iters=int(num_iterations), floor_sor_k=int(nb_neighbors),
+                         floor_sor_ratio=float(std_ratio), do_icp=False, n_streams=int(n_streams),
+                         seed=int(geometry._SEED[0] if seed is None else seed) & 0xFFFFFFFFFFFFFFFF)
+    pipe = FramePipeline(cfg)
+    try:
+        outs = pipe.run_clouds(pcds, want_points=True, out_stride=cap)
+    finally:
+        pipe.close()
+    return [PointCloud(o.points) for o in outs]
 
 
 def main(pattern='E:/Extracted_data/*/*/*/master_1/filtered_and_registered_pointclouds/*.pcd'):

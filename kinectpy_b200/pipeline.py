@@ -8,6 +8,10 @@ fuse, ``filter_outliers``) followed by the ``floor_removal.py:64-73`` loop body 
 ``execute_point_to_plane_registration`` refinement of every sub sensor's extrinsic
 (``preprocessing/registration.py:65-86``).  Frames are independent, so multi-GPU use is one
 pipeline per rank over a disjoint slice of the frame indices (no collective on the frame path).
+
+With ``input_mode=INPUT_CLOUDS`` the pipeline takes saved point clouds instead (``run_clouds``): the fused ``.pcd`` files
+a recording left go through the same stages from the voxel downsample on (``cloud_voxel=0``: from the SOR on, which is
+``floor_removal.py``'s composition).
 """
 from __future__ import annotations
 
@@ -19,6 +23,7 @@ import numpy as np
 
 from . import _cabi
 from ._cabi import FrameResult, KinectPyB200Error, PipelineCfg
+from .geometry import PointCloud
 
 
 @dataclass
@@ -61,6 +66,12 @@ class PipelineConfig:
     # cloud's unit, then the floor SOR)
     floor_mode: int = _cabi.FLOOR_RANSAC
     floor_plane: tuple = (0.0, 0.0, 0.0, 0.0)
+    # INPUT_DEPTH (depth images + xy-table, ``run``) or INPUT_CLOUDS (saved clouds, ``run_clouds``: n_sensors = 1,
+    # pixels = row capacity of one cloud, do_icp and do_crop off, lengths in the clouds' unit, scale ignored)
+    input_mode: int = _cabi.INPUT_DEPTH
+    # cloud input: 1 = voxel_down_sample(voxel_size) first (filter_outliers); 0 = the rows as they are, voxel_size = the
+    # clouds' typical point spacing, which sizes the neighbour-search grids only (speed, never a result)
+    cloud_voxel: int = 1
 
     def to_c(self) -> PipelineCfg:
         c = PipelineCfg()
@@ -80,7 +91,20 @@ class PipelineConfig:
         if len(pl) != 4:
             raise ValueError("floor_plane must hold 4 coefficients (a, b, c, d)")
         c.floor_plane[:] = pl
+        c.input_mode, c.cloud_voxel = self.input_mode, int(self.cloud_voxel)
         return c
+
+
+def _cloud_rows(c) -> np.ndarray:
+    """float32 [n, 3] rows of a PointCloud or an array, a row with a non-finite coordinate set to NaN (absent)."""
+    h = np.asarray(c._p.peek_host() if isinstance(c, PointCloud) else c)
+    h = h.reshape(0, 3) if h.size == 0 else h
+    if h.ndim != 2 or h.shape[1] != 3:
+        raise ValueError(f"a cloud must have shape (n, 3), got {h.shape}")
+    bad = ~np.isfinite(h).all(axis=1)
+    a = np.array(h, dtype=np.float32)
+    a[bad] = np.nan
+    return a
 
 
 @dataclass
@@ -101,19 +125,26 @@ class FrameOutput:
 
 
 class FramePipeline:
-    def __init__(self, cfg: PipelineConfig, xy_tables: np.ndarray, T_fuse: np.ndarray, T_icp_init: Optional[np.ndarray] = None,
-                 device: int = 0):
+    def __init__(self, cfg: PipelineConfig, xy_tables: Optional[np.ndarray] = None, T_fuse: Optional[np.ndarray] = None,
+                 T_icp_init: Optional[np.ndarray] = None, device: int = 0):
+        """``xy_tables`` and ``T_fuse`` are required for depth input; a cloud pipeline (``input_mode=INPUT_CLOUDS``) takes
+        neither."""
         self.lib = _cabi.load_library()
         self.cfg = cfg
         self.device = device
         S, P = cfg.n_sensors, cfg.pixels
-        tab = np.ascontiguousarray(xy_tables, dtype=np.float32).reshape(S, P, 2)
-        Tf = np.ascontiguousarray(T_fuse, dtype=np.float64).reshape(S, 16)
-        Ti = Tf if T_icp_init is None else np.ascontiguousarray(T_icp_init, dtype=np.float64).reshape(S, 16)
-        both = np.ascontiguousarray(np.stack([Tf, Ti]))
+        tab = both = None
+        if cfg.input_mode != _cabi.INPUT_CLOUDS or xy_tables is not None or T_fuse is not None:
+            if xy_tables is None or T_fuse is None:
+                raise ValueError("a depth pipeline needs xy_tables and T_fuse")
+            tab = np.ascontiguousarray(xy_tables, dtype=np.float32).reshape(S, P, 2)
+            Tf = np.ascontiguousarray(T_fuse, dtype=np.float64).reshape(S, 16)
+            Ti = Tf if T_icp_init is None else np.ascontiguousarray(T_icp_init, dtype=np.float64).reshape(S, 16)
+            both = np.ascontiguousarray(np.stack([Tf, Ti]))
         h = C.c_void_p()
         c = cfg.to_c()
-        rc = self.lib.kp_pipeline_create(device, C.byref(c), tab.ctypes.data, both.ctypes.data, C.byref(h))
+        rc = self.lib.kp_pipeline_create(device, C.byref(c), tab.ctypes.data if tab is not None else None,
+                                         both.ctypes.data if both is not None else None, C.byref(h))
         if rc != 0:
             raise KinectPyB200Error(rc, (self.lib.kp_last_error(None) or b"").decode())
         self.handle = h
@@ -164,11 +195,18 @@ class FramePipeline:
             if rgb is not None:
                 rgb = np.ascontiguousarray(rgb, dtype=np.uint8).reshape(-1, S, P, 3)
             rptr = rgb.ctypes.data if rgb is not None else None
+        res, out, stride, fixed, ids = self._buffers(F, want_points, out_stride, want_fixed, frame_ids)
+        rc = self.lib.kp_pipeline_run_ex(self.handle, ptr, rptr, 1 if on_dev else 0, F, ids.ctypes.data if ids is not None else None,
+                                         res, out.ptr if out is not None else None, stride, fixed.ptr if fixed is not None else None)
+        return self._outputs(rc, res, F, out, fixed, check)
+
+    def _buffers(self, F, want_points, out_stride, want_fixed, frame_ids):
+        """Result records, the optional device buffers of the final clouds and fixed-N slots, the frame ids."""
         res = (FrameResult * F)()
         out = None
         stride = 0
         if want_points:
-            stride = int(out_stride or S * P)
+            stride = int(out_stride or self.cfg.n_sensors * self.cfg.pixels)
             out = self._ctx.empty((F, stride, 3), np.float32)
             self._ctx.sync()
         fixed = None
@@ -180,8 +218,10 @@ class FramePipeline:
             ids = np.ascontiguousarray(frame_ids, dtype=np.int64).reshape(-1)
             if ids.size != F:
                 raise ValueError("frame_ids must hold one id per frame")
-        rc = self.lib.kp_pipeline_run_ex(self.handle, ptr, rptr, 1 if on_dev else 0, F, ids.ctypes.data if ids is not None else None,
-                                         res, out.ptr if out is not None else None, stride, fixed.ptr if fixed is not None else None)
+        return res, out, stride, fixed, ids
+
+    def _outputs(self, rc, res, F, out, fixed, check):
+        S = self.cfg.n_sensors
         if rc != 0 and (check or all(res[f].status == 0 for f in range(F))):      # (a call-level error has no frame status)
             self._raise(rc)
         outs: List[FrameOutput] = []
@@ -202,6 +242,32 @@ class FramePipeline:
             outs.append(fo)
         self._last_raw = res
         return outs
+
+    def run_clouds(self, clouds, want_points: bool = False, out_stride: Optional[int] = None, want_fixed: bool = False,
+                   frame_ids=None, check: bool = True):
+        """Cloud input (``input_mode=INPUT_CLOUDS``).  ``clouds``: a list of ``PointCloud`` or ``(n, 3)`` arrays (host: the
+        rows are copied to the device batch by batch), or a pair ``(DeviceArray of float32 [rows, 3], offsets)`` with
+        cloud f = rows ``offsets[f] .. offsets[f + 1]``.  A host row with a non-finite coordinate is absent, as on
+        ``PointCloud``'s upload (a NaN row to the engine).  The other arguments and the outputs are those of ``run``."""
+        on_dev = isinstance(clouds, tuple) and len(clouds) == 2 and isinstance(clouds[0], _cabi.DeviceArray)
+        if on_dev:
+            dev, off = clouds
+            off = np.ascontiguousarray(off, dtype=np.int64).reshape(-1)
+            ptr = dev.ptr
+        else:
+            arrs = [_cloud_rows(c) for c in clouds]
+            off = np.zeros(len(arrs) + 1, np.int64)
+            off[1:] = np.cumsum([a.shape[0] for a in arrs])
+            flat = np.ascontiguousarray(np.concatenate(arrs, 0) if arrs else np.zeros((0, 3), np.float32), dtype=np.float32)
+            ptr = flat.ctypes.data
+        F = off.size - 1
+        if F < 0:
+            raise ValueError("offsets must hold F + 1 entries")
+        res, out, stride, fixed, ids = self._buffers(F, want_points, out_stride, want_fixed, frame_ids)
+        rc = self.lib.kp_pipeline_run_clouds(self.handle, ptr, off.ctypes.data, 1 if on_dev else 0, F,
+                                             ids.ctypes.data if ids is not None else None, res,
+                                             out.ptr if out is not None else None, stride, fixed.ptr if fixed is not None else None)
+        return self._outputs(rc, res, F, out, fixed, check)
 
     def run_raw(self, depth_ptr: int, on_device: bool, n_frames: int, d_out_ptr=None, out_stride: int = 0):
         """Timing form: no numpy conversion of the results (returns the ctypes result array).  ``d_out_ptr``:
